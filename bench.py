@@ -2,7 +2,7 @@
 """bench.py — marker x trait LOD tests/sec on the BXD-shape bulkscan (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--workload alt-grid|null-grid|null-exact|scaled-null-exact|perms]
+                    [--workload alt-grid|null-grid|null-exact|scaled-null-exact|perms] [--dump-outputs DIR]
 
 One "step" = one full scan call through the C-ABI (rotation by U' -> per-trait null statistics / Brent
 fit -> marker operand -> fused DMMA scan with the LOD epilogue) on synthetic data (SURVEY 8d):
@@ -25,6 +25,11 @@ The kinship eigendecomposition is setup (one-off, timed separately and reported 
 N > 1 (torchrun, one rank per GPU): traits (bulkscan) or permutations (scan) are sharded across ranks
 (strong scaling: the problem is fixed), G/U are replicated, there is no data-path collective; NCCL is
 used for the barrier and the max-over-ranks time.
+
+--dump-outputs DIR (one GPU) writes the results of the last timed step as DIR/<name>.npy (float64), named and
+oriented as the Python API returns them (markers x traits / permutations); an output of more than DUMP_ENTRIES
+entries is cut to a fixed, seeded sample of its traits (permutations) and markers.  The inputs are seeded too, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +44,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for sub in ("bulklmm.jl_b200", "oracle"):
     sys.path.insert(0, os.path.join(ROOT, sub))
+sys.dont_write_bytecode = True  # the source tree may be read-only: nothing is cached there
 
 import numpy as np  # noqa: E402
 
@@ -61,6 +67,7 @@ WORKLOADS = {
     "perms": dict(n=79, p=7321, m=10001, c=1, method="perms", opts=dict(prior_variance=0.0), fmult=1,
                   cfg="BASELINE.json configs[3]", outputs="lod, L_perms (p x nperms f64), per-permutation max", cpu_m=10000),
 }
+DUMP_ENTRIES = 1 << 21  # 16 MB of float64; no workload has more than two outputs this large, so a dump is <= 64 MB
 
 
 def fp64_peak():
@@ -240,8 +247,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer e2e leg")
     ap.add_argument("--no-other", action="store_true", help="skip the short runs of the other configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results (sampled above DUMP_ENTRIES entries) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; it does not apply to --impl reference")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs needs one GPU: at N > 1 each rank holds only its shard of the results")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -327,6 +340,14 @@ def main():
             self.pr = eng.make_problem(n, p, 1 if self.perms else ml, c, *[t.data_ptr() for t in self.d])
             self.flops = 2.0 * n * p * (ml + (1 if self.perms else 0)) * w["fmult"]
             self.out_bytes = 8.0 * sum(int(np.prod(s)) for s in self.out_shapes[:2])
+
+        def outputs(self):
+            """(name, device tensor) of each result a caller of the path receives, named as in blmm_b200's results;
+            matrices are traits (permutations) x markers here, the transpose of the caller's layout"""
+            if self.perms:
+                Lp, mx, lod, s = self.dout
+                return [("L_perms", Lp), ("max_lod", mx), ("lod", lod), ("sigma2_e", s[:1]), ("h2_null", s[1:])]
+            return [("L", self.dout[0]), ("h2_panel" if self.alt else "h2_null_list", self.dout[1])]
 
         @staticmethod
         def call(E, perms, pr, opts, outs, perm_ptr, nperms):
@@ -451,6 +472,21 @@ def main():
             out[nm] = nb / best / 1e9
         return out
 
+    def dump_outputs(job, outdir):
+        """job's results as outdir/<name>.npy in the caller's orientation (markers x traits); a matrix of more than
+        DUMP_ENTRIES entries is cut to the same seeded, sorted sample of its rows and columns on every run"""
+        os.makedirs(outdir, exist_ok=True)
+        for name, t in job.outputs():
+            if t.dim() == 2 and t.numel() > DUMP_ENTRIES:
+                r, c = t.shape
+                kc = min(c, DUMP_ENTRIES // min(r, 256))
+                kr = min(r, DUMP_ENTRIES // kc)
+                rng = np.random.default_rng(0)
+                rows = torch.from_numpy(np.sort(rng.choice(r, kr, replace=False))).to(dev)
+                cols = torch.from_numpy(np.sort(rng.choice(c, kc, replace=False))).to(dev)
+                t = t.index_select(0, rows).index_select(1, cols)
+            np.save(os.path.join(outdir, name + ".npy"), np.ascontiguousarray(t.cpu().numpy().T))
+
     def run_e2e(job, steps):
         """rank 0 drives all `world` GPUs through one context; the other ranks wait on the CPU barrier"""
         out = None
@@ -483,6 +519,8 @@ def main():
     r = job.timed(args.steps, args.warmup)
     clocks = sampler.stop(*r["wall"]) if rank == 0 else None
     value = job.tests_total * args.steps / (r["total_ms"] * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(job, args.dump_outputs)
 
     # ---- roofline of the dominant kernel (the fused scan), measured live with CUDA events inside the library
     peak, peak_src = fp64_peak()
