@@ -97,10 +97,65 @@ void matrix_to_host(blmm_ctx* ctx, cudaStream_t stream, double* dst, int64_t ld,
   }
 }
 
-// Large pageable results go through the ring; small ones are not worth the hand-over.
-bool via_ring(const double* dst, int64_t p, int64_t cols) {
-  return (double)p * (double)cols * 8.0 >= 8e6 && !host_ptr_is_pinned(dst);
+void copy_out(blmm_ctx* ctx, double* dst, const double* src_dev, size_t count, int mem_space) {
+  if (!dst || dst == src_dev) return;
+  CUDA_TRY(cudaMemcpyAsync(dst, src_dev, count * sizeof(double),
+                           mem_space == BLMM_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost,
+                           ctx->stream));
 }
+
+// Where the results of a scan call are computed and how they reach the caller.  Device mode: the kernels write into the
+// caller's arrays, or into workspace for an output the caller passed NULL for that the kernels write anyway.  Host
+// mode: they write into workspace, and deliver() queues the copies into the caller's arrays in the order the outputs
+// were bound, then collects the device flags and waits for the drain threads.
+class Results {
+ public:
+  Results(blmm_ctx* ctx, int mem_space) : dev(mem_space == BLMM_MEM_DEVICE), ctx_(ctx) {}
+  const bool dev;
+  // `count` results
+  double* vec(double* user, Slot s, size_t count) { return bind(user, s, Copy{user, nullptr, (int64_t)count, 1, 0}); }
+  // a p x cols result: leading dimension ld in the caller's array, p in workspace
+  double* panel(double* user, Slot s, int64_t p, int64_t cols, int64_t ld) {
+    return bind(user, s, Copy{user, nullptr, p, cols, ld});
+  }
+  // `count` results the kernels always write into workspace (device mode: copied device-to-device right away)
+  void copy(double* user, const double* src, size_t count) {
+    if (dev)
+      copy_out(ctx_, user, src, count, BLMM_MEM_DEVICE);
+    else if (user)
+      add(Copy{user, src, (int64_t)count, 1, 0});
+  }
+  void deliver() {
+    if (dev) return;
+    for (int i = 0; i < n_; ++i) {
+      const Copy& c = q_[i];
+      if (c.ld == 0)
+        copy_out(ctx_, c.dst, c.src, (size_t)c.rows, BLMM_MEM_HOST);
+      else  // large pageable results go through the ring; small ones are not worth the hand-over
+        matrix_to_host(ctx_, ctx_->stream, c.dst, c.ld, c.src, c.rows, c.cols,
+                       (double)c.rows * (double)c.cols * 8.0 < 8e6 || host_ptr_is_pinned(c.dst));
+    }
+    finish_and_check(ctx_);
+    hostpipe_wait(ctx_->pipe);
+  }
+
+ private:
+  struct Copy { double* dst; const double* src; int64_t rows, cols, ld; };  // ld == 0: a vector
+  double* bind(double* user, Slot s, Copy c) {
+    if (dev && user) return user;
+    double* d = ws<double>(ctx_, s, (size_t)c.rows * c.cols);
+    c.src = d;
+    if (!dev && user) add(c);
+    return d;
+  }
+  void add(const Copy& c) {
+    if (n_ == 5) throw Fail{BLMM_E_INVALID, "internal: more results than Results holds"};
+    q_[n_++] = c;
+  }
+  blmm_ctx* ctx_;
+  Copy q_[5];  // a call has at most five outputs
+  int n_ = 0;
+};
 
 void check_problem(const blmm_problem* pr, bool need_markers, bool need_decomp = true) {
   if (!pr) throw Fail{BLMM_E_INVALID, "problem is NULL"};
@@ -116,32 +171,37 @@ void check_problem(const blmm_problem* pr, bool need_markers, bool need_decomp =
     throw Fail{BLMM_E_INVALID, "problem too large"};
 }
 
+// leading dimension of the caller's p-row result matrices
+int64_t out_ld(const blmm_opts* o, int64_t p) {
+  const int64_t ld = o->ld_out ? o->ld_out : p;
+  if (ld < p) throw Fail{BLMM_E_INVALID, "ld_out < p"};
+  return ld;
+}
+
+void check_optim_interval(const blmm_opts* o) {
+  if (o->optim_interval < 1) throw Fail{BLMM_E_INVALID, "optim_interval must be >= 1"};
+}
+
 LikParams lik_of(const blmm_opts* o) { return LikParams{o->prior_variance, o->prior_sample_size, o->reml ? 1 : 0}; }
 
-// Rotated inputs of one call (device, padded column-major).
+// Inputs of one call on the device (rotated ones padded, column-major).
 struct Rotated {
   int n, n_pad, nq, c;
-  int64_t m, p;
+  int64_t m;
   const double* lambda;
-  const double* dU;  // the rotation matrix on the device (observation weights folded in)
-  const double* dC;  // the unrotated covariates on the device
-  double *Y0, *C0, *G0;
+  const double* dU;  // the rotation matrix (observation weights folded in)
+  const double* dC;  // the unrotated covariates
+  double *C0, *Y0 = nullptr, *G0 = nullptr;  // U'C, U'Y, U'G: rotate_covariates, rotate_traits, rotate_markers_aside
 };
 
-struct Rotated;
-void rotate_markers(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space, cudaStream_t stream);
-void rotate_markers_aside(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space, cudaStream_t after);
-void rotate_traits(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space);
-
-Rotated rotate_inputs(blmm_ctx* ctx, const blmm_problem* pr, int mem_space, bool with_markers,
-                      bool with_traits = true, bool covariates_on_second_stream = false, bool rotate_cov = true) {
+// Stages U, lambda and the covariates; rotates nothing.
+Rotated stage_inputs(blmm_ctx* ctx, const blmm_problem* pr, int mem_space) {
   Rotated R;
   R.n = (int)pr->n;
   R.nq = num_kchunks(pr->n);
   R.n_pad = R.nq * KC;
   R.c = (int)pr->c;
   R.m = pr->m;
-  R.p = with_markers ? pr->p : 0;
   const size_t n = (size_t)pr->n;
   const double* dU = stage_in(ctx, S_U_IN, pr->U, n * n, mem_space);
   if (pr->obs_weights) {
@@ -153,23 +213,13 @@ Rotated rotate_inputs(blmm_ctx* ctx, const blmm_problem* pr, int mem_space, bool
   }
   R.dU = dU;
   R.lambda = stage_in(ctx, S_LAM, pr->lambda, n, mem_space);
-  const double* dC = stage_in(ctx, S_C_IN, pr->Covar, n * R.c, mem_space);
-  R.dC = dC;
+  R.dC = stage_in(ctx, S_C_IN, pr->Covar, n * R.c, mem_space);
   R.C0 = ws<double>(ctx, S_C0, (size_t)R.n_pad * R.c);
-  cudaStream_t cov_stream = ctx->stream;
-  if (covariates_on_second_stream) {
-    // grid scans: the covariate rotation and everything that hangs off it on the marker side run on the second
-    // stream from here on, while the main stream goes straight to the trait rotation
-    CUDA_TRY(cudaEventRecord(ctx->fork_ev, ctx->stream));
-    CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->fork_ev, 0));
-    cov_stream = ctx->copy_stream;
-  }
-  if (rotate_cov) ctx->launches += launch_rotate(dU, dC, pr->n, R.C0, R.n_pad, R.n_pad, R.n, R.c, cov_stream);
-  R.Y0 = nullptr;
-  if (with_traits) rotate_traits(ctx, pr, R, mem_space);
-  R.G0 = nullptr;
-  if (with_markers) rotate_markers_aside(ctx, pr, R, mem_space, ctx->stream);
   return R;
+}
+
+void rotate_covariates(blmm_ctx* ctx, const Rotated& R, cudaStream_t stream) {
+  ctx->launches += launch_rotate(R.dU, R.dC, R.n, R.C0, R.n_pad, R.n_pad, R.n, R.c, stream);
 }
 
 void rotate_traits(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space) {
@@ -179,42 +229,25 @@ void rotate_traits(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_sp
   ctx->launches += launch_rotate(R.dU, dY, pr->n, R.Y0, R.n_pad, R.n_pad, R.n, R.m, ctx->stream);
 }
 
-void rotate_markers(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space, cudaStream_t stream) {
-  const size_t n = (size_t)pr->n;
-  const double* dG = stage_in(ctx, S_G_IN, pr->G, n * (size_t)pr->p, mem_space, stream);
-  R.G0 = ws<double>(ctx, S_G0, (size_t)R.n_pad * pr->p);
-  ctx->launches += launch_rotate(R.dU, dG, pr->n, R.G0, R.n_pad, R.n_pad, R.n, pr->p, stream);
+// Reallocating a workspace slot frees the old buffer, and cudaFree synchronises the device: the marker slots are sized
+// before a call's first fork, so that no allocation serialises the streams mid-overlap.
+void reserve_marker_ws(blmm_ctx* ctx, const blmm_problem* pr, int mem_space) {
+  ws<double>(ctx, S_G_IN, mem_space == BLMM_MEM_HOST ? (size_t)pr->n * pr->p : 1);
+  ws<double>(ctx, S_G0, (size_t)num_kchunks(pr->n) * KC * pr->p);
 }
 
-// Staging and rotating the markers depends on nothing but G and U: it runs on the third stream, beside whatever the
-// other two are doing (trait rotation / statistics / Brent fit; covariates and weight constants); `consumer` is made
-// to wait for it by wait_markers() right before the first kernel that reads G0.
-void rotate_markers_aside(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space, cudaStream_t after) {
-  ws<double>(ctx, S_G_IN, mem_space == BLMM_MEM_HOST ? (size_t)pr->n * pr->p : 1);  // (re)allocations first: cudaFree
-  ws<double>(ctx, S_G0, (size_t)R.n_pad * pr->p);                                    // synchronises the device
-  CUDA_TRY(cudaEventRecord(ctx->aux_fork_ev, after));  // dU (and a previous call's readers of G0) are ordered before
+// Staging and rotating the markers depends on nothing but G and U: it runs on the third stream, forked from the main
+// stream, beside whatever the other two are doing (trait rotation / statistics / Brent fit; covariates and weight
+// constants); the consumer is made to wait for it by wait_markers() right before the first kernel that reads G0.
+void rotate_markers_aside(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space) {
+  CUDA_TRY(cudaEventRecord(ctx->aux_fork_ev, ctx->stream));  // dU (and a previous call's readers of G0) are ordered before
   CUDA_TRY(cudaStreamWaitEvent(ctx->aux_stream, ctx->aux_fork_ev, 0));
-  rotate_markers(ctx, pr, R, mem_space, ctx->aux_stream);
+  const double* dG = stage_in(ctx, S_G_IN, pr->G, (size_t)pr->n * (size_t)pr->p, mem_space, ctx->aux_stream);
+  R.G0 = ws<double>(ctx, S_G0, (size_t)R.n_pad * pr->p);
+  ctx->launches += launch_rotate(R.dU, dG, pr->n, R.G0, R.n_pad, R.n_pad, R.n, pr->p, ctx->aux_stream);
   CUDA_TRY(cudaEventRecord(ctx->aux_done_ev, ctx->aux_stream));
 }
 void wait_markers(blmm_ctx* ctx, cudaStream_t consumer) { CUDA_TRY(cudaStreamWaitEvent(consumer, ctx->aux_done_ev, 0)); }
-
-// The marker side of a grid scan (G -> U'G -> weight-folded marker operand) depends only on G, U and the
-// per-h2 weight constants, the trait side only on Y: the two chains are latency-bound on their own, so the
-// marker chain runs on the second stream while the main stream does the traits.  Returns after queueing;
-// the caller makes the main stream wait on ctx->join_ev before the scan.
-void fork_marker_side(blmm_ctx* ctx, const blmm_problem* pr, Rotated& R, int mem_space, int nk, WeightConsts wc,
-                      bool fold_sw, double* Mop, int64_t p_pad, bool already_forked = false) {
-  if (!already_forked) {
-    CUDA_TRY(cudaEventRecord(ctx->fork_ev, ctx->stream));
-    CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->fork_ev, 0));
-  }
-  R.p = pr->p;
-  wait_markers(ctx, ctx->copy_stream);  // queued by the caller before the covariate chain (rotate_markers_aside)
-  ctx->launches += launch_marker_operand(R.G0, R.p, p_pad, R.n, R.n_pad, R.c, nk, wc, fold_sw, Mop, ctx->d_flags,
-                                         ctx->copy_stream);
-  CUDA_TRY(cudaEventRecord(ctx->join_ev, ctx->copy_stream));
-}
 
 WeightConsts weight_ws(blmm_ctx* ctx, int nk, int n_pad, int c) {
   WeightConsts wc;
@@ -238,22 +271,13 @@ const double* upload_grid(blmm_ctx* ctx, const blmm_opts* o) {
   return d;
 }
 
-void copy_out(blmm_ctx* ctx, double* dst, const double* src_dev, size_t count, int mem_space) {
-  if (!dst || dst == src_dev) return;
-  CUDA_TRY(cudaMemcpyAsync(dst, src_dev, count * sizeof(double),
-                           mem_space == BLMM_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost,
-                           ctx->stream));
-}
-
-// output_pvals: -log10 p of every LOD, computed on the device before anything is copied back
-double* pvals_after_scan(blmm_ctx* ctx, const blmm_opts* o, const double* dL, int64_t p, int64_t m, int64_t ldL) {
-  if (o->chisq_df <= 0) return nullptr;
+// output_pvals: -log10 p of every LOD into dP, computed on the device before anything is copied back
+void pvals_after_scan(blmm_ctx* ctx, const blmm_opts* o, const double* dL, double* dP, int64_t p, int64_t m,
+                      int64_t ldL) {
+  if (o->chisq_df <= 0) return;
   if (o->chisq_df > 1000) throw Fail{BLMM_E_INVALID, "chisq_df must be in 1..1000"};
   if (!o->log10p_out) throw Fail{BLMM_E_INVALID, "chisq_df > 0 but log10p_out is NULL"};
-  const bool dev = o->mem_space == BLMM_MEM_DEVICE;
-  double* dP = dev ? o->log10p_out : ws<double>(ctx, S_PVAL, (size_t)p * m);
   ctx->launches += launch_lod2log10p(dL, p, m, ldL, ldL, o->chisq_df, dP, ctx->sm_count, ctx->stream);
-  return dP;
 }
 
 // zeroed device counter for the stream kernels' dynamic unit scheduler
@@ -261,6 +285,17 @@ unsigned long long* fresh_unit_counter(blmm_ctx* ctx) {
   unsigned long long* c = ws<unsigned long long>(ctx, S_UNITCTR, 1);
   CUDA_TRY(cudaMemsetAsync(c, 0, sizeof(unsigned long long), ctx->stream));
   return c;
+}
+
+// The scan launch(es) of a call between the two profiling events blmm_last_scan_ms reads.
+template <typename F>
+void timed_scan(blmm_ctx* ctx, F&& launch) {
+  if (ctx->profiling) CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
+  launch();
+  if (ctx->profiling) {
+    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
+    ctx->scan_timed = true;
+  }
 }
 
 void run_scan(blmm_ctx* ctx, ScanParams P) {
@@ -276,7 +311,7 @@ void run_scan(blmm_ctx* ctx, ScanParams P) {
     int maxw = 0, maxp = 0;
     cudaDeviceGetAttribute(&maxw, cudaDevAttrMaxAccessPolicyWindowSize, ctx->device);
     cudaDeviceGetAttribute(&maxp, cudaDevAttrMaxPersistingL2CacheSize, ctx->device);
-    const size_t bytes = (size_t)(P.e ? P.nk : (P.tile_k0 ? P.ngrid : 1)) * P.nq * P.p_pad * KC * 8;  // every slab a tile may use
+    const size_t bytes = (size_t)P.nk * P.nq * P.p_pad * KC * 8;  // every slab a tile may use
     if (!ctx->l2_limit_set) {  // per device: a multi-GPU process holds one context per GPU
       cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, std::min<size_t>((size_t)maxp, (size_t)64 << 20));
       ctx->l2_limit_set = true;
@@ -293,27 +328,24 @@ void run_scan(blmm_ctx* ctx, ScanParams P) {
     window = cudaStreamSetAttribute(ctx->stream, cudaStreamAttributeAccessPolicyWindow, &av) == cudaSuccess;
     cudaGetLastError();
   }
-  if (ctx->profiling) CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
-  if (P.nq <= scan_max_nq(P.nk)) {
-    const int launched = launch_scan(P, ctx->sm_count, ctx->stream);
-    if (!launched) throw Fail{BLMM_E_INVALID, "scan kernel: unsupported parameter combination"};
-    ctx->launches += launched;
-  } else {
-    // n too large for the shared-memory-resident trait tile: same arithmetic, K streamed
-    static_assert(SCAN_TT == 128 && SCAN_MT == 64, "packing shared with the streamed GRID kernel");
-    StreamParams Q{};
-    Q.Mop = P.Mop; Q.Xop = P.Top; Q.e = P.e; Q.et = P.et; Q.tile_k0 = P.tile_k0; Q.n_tiles_dev = P.n_tiles_dev;
-    Q.col_map = P.col_map; Q.grid = P.grid; Q.ngrid = P.ngrid; Q.L = P.L; Q.L0 = P.L0;
-    Q.H2 = P.H2; Q.colmax = P.colmax; Q.ldL = P.ldL; Q.nq = P.nq; Q.p = P.p; Q.p_pad = P.p_pad; Q.m = P.m;
-    Q.xcol_pad = P.tcol_pad; Q.tcol_pad = P.tcol_pad; Q.n_tt = P.n_tiles_t; Q.nk = P.nk;
-    Q.argmax_mode = P.argmax_mode; Q.half_n = P.half_n;
-    Q.unit_counter = fresh_unit_counter(ctx);  // n > 100: operands beyond L2 are the normal case here
-    ctx->launches += launch_scan_stream_grid(Q, ctx->sm_count, ctx->stream);
-  }
-  if (ctx->profiling) {
-    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
-    ctx->scan_timed = true;
-  }
+  timed_scan(ctx, [&] {
+    if (P.nq <= scan_max_nq(P.nk)) {
+      const int launched = launch_scan(P, ctx->sm_count, ctx->stream);
+      if (!launched) throw Fail{BLMM_E_INVALID, "scan kernel: unsupported parameter combination"};
+      ctx->launches += launched;
+    } else {
+      // n too large for the shared-memory-resident trait tile: same arithmetic, K streamed
+      static_assert(SCAN_TT == 128 && SCAN_MT == 64, "packing shared with the streamed GRID kernel");
+      StreamParams Q{};
+      Q.Mop = P.Mop; Q.Xop = P.Top; Q.e = P.e; Q.et = P.et; Q.tile_k0 = P.tile_k0; Q.n_tiles_dev = P.n_tiles_dev;
+      Q.col_map = P.col_map; Q.grid = P.grid; Q.ngrid = P.ngrid; Q.L = P.L; Q.L0 = P.L0;
+      Q.H2 = P.H2; Q.colmax = P.colmax; Q.ldL = P.ldL; Q.nq = P.nq; Q.p = P.p; Q.p_pad = P.p_pad; Q.m = P.m;
+      Q.xcol_pad = P.tcol_pad; Q.tcol_pad = P.tcol_pad; Q.n_tt = P.n_tiles_t; Q.nk = P.nk;
+      Q.argmax_mode = P.argmax_mode; Q.half_n = P.half_n;
+      Q.unit_counter = fresh_unit_counter(ctx);  // n > 100: operands beyond L2 are the normal case here
+      ctx->launches += launch_scan_stream_grid(Q, ctx->sm_count, ctx->stream);
+    }
+  });
   if (window) {
     cudaStreamAttrValue av;
     memset(&av, 0, sizeof av);
@@ -327,6 +359,98 @@ double trace_now() {
   return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
+// Chunk boundaries in trait tiles, tbeg[0..nchunk].  The link idles until the first chunk exists, so the first two
+// chunks are small (1/4 and 1/2 of an even share, at least one tile) and the rest share what is left evenly.
+void chunk_tiles(int n_tiles, int nchunk, int* tbeg) {
+  const int even = n_tiles / nchunk;
+  const int first = std::max(1, even / 4), second = std::max(1, even / 2);
+  tbeg[0] = 0;
+  tbeg[1] = std::min(n_tiles, first);
+  tbeg[2] = std::min(n_tiles, first + second);
+  const int rest = n_tiles - tbeg[2];
+  for (int ch = 3; ch <= nchunk; ++ch) tbeg[ch] = tbeg[2] + (int)((int64_t)rest * (ch - 2) / (nchunk - 2));
+}
+
+// Host-buffer alt-grid: the p x m panels (2 x 2 GB at BXD size) leave over PCIe, which takes ~4x the scan itself.  The
+// trait tiles are scanned in chunks, and each chunk's columns are copied back on the second stream while the next
+// chunks are scanned.  The h2 panel holds one of <= 255 grid values per entry, so it crosses PCIe as one-byte grid
+// indices (1/8 of the bytes) through the pinned ring and is expanded to grid[index] in the caller's Float64 array by
+// the drain threads; L goes straight into a pinned destination, or through the same ring into a pageable one
+// (blmm_hostpipe.cu).  dL / dH: the p x m workspace panels (dH NULL without an h2 panel).
+void alt_grid_to_host_chunked(blmm_ctx* ctx, const ScanParams& P, const blmm_opts* o, double* L_out, double* h2_out,
+                              double* dL, double* dH, int64_t ld, double t_enter) {
+  const int64_t p = P.p, m = P.m;
+  const int n_tiles = P.n_tiles_t;
+  // PCIe is the bottleneck, so what matters is how soon the first copy starts: more, smaller chunks for big panels
+  const int nchunk = n_tiles >= 64 ? MAX_CHUNK : 8;
+  // The index encoding is worth it when the panel is large (PCIe time saved > host expansion time): >= 1e8
+  // entries by default.  BLMM_B200_H2_TRANSFER = index | f64 overrides; BLMM_B200_HOST_THREADS sets the drain
+  // thread count (default min(16, cores - 1), divided between the GPUs of a multi-GPU context).
+  const char* h2_mode = getenv("BLMM_B200_H2_TRANSFER");
+  const bool want_idx = h2_mode ? (h2_mode[0] == 'i') : (ctx->idx_hint >= 0 ? ctx->idx_hint == 1 : (double)p * (double)m >= 1e8);
+  const bool idx_panel = dH && want_idx && P.nq <= scan_max_nq(P.nk);
+  uint8_t* dI = idx_panel ? ws<uint8_t>(ctx, S_H2IDX, (size_t)p * m) : nullptr;
+  if (idx_panel && ctx->h_idx_cap < (size_t)p * m) {
+    // the whole index panel has its own pinned staging (1 byte per entry), so that queueing its copies never
+    // waits for a ring slot: every copy of the call is in the stream before the first one has finished
+    if (ctx->h_idx) CUDA_TRY(cudaFreeHost(ctx->h_idx));
+    ctx->h_idx = nullptr;
+    ctx->h_idx_cap = 0;
+    CUDA_TRY(cudaMallocHost(&ctx->h_idx, (size_t)p * m));
+    ctx->h_idx_cap = (size_t)p * m;
+  }
+  const bool L_pinned = host_ptr_is_pinned(L_out);
+  const bool H_pinned = h2_out && host_ptr_is_pinned(h2_out);
+  HostPipe* pipe = (idx_panel || !L_pinned || (dH && !H_pinned)) ? host_pipe(ctx) : nullptr;
+  // only index expansion to do (every Float64 copy is a direct DMA): a few drain threads, not all of them
+  hostpipe_set_active(pipe, (L_pinned && (idx_panel || !dH || H_pinned)) ? 6 : 1 << 30);
+  int tbeg[MAX_CHUNK + 1];
+  chunk_tiles(n_tiles, nchunk, tbeg);
+  int64_t cbeg[MAX_CHUNK + 1];
+  for (int ch = 0; ch <= nchunk; ++ch) cbeg[ch] = std::min<int64_t>((int64_t)tbeg[ch] * SCAN_TT, m);
+  // every chunk's scan is queued first: the copy loop below may block on ring slots
+  for (int ch = 0; ch < nchunk; ++ch) {
+    const int t0 = tbeg[ch], t1 = tbeg[ch + 1];
+    if (t1 == t0) continue;
+    const int64_t c0 = cbeg[ch];
+    ScanParams Pc = P;
+    Pc.Top = P.Top + (int64_t)t0 * SCAN_TT * KC;
+    Pc.e = P.e + (int64_t)t0 * SCAN_TT;
+    Pc.et = P.et + (int64_t)t0 * SCAN_TT;
+    Pc.L = dL + c0 * p;
+    Pc.H2 = (dH && !idx_panel) ? dH + c0 * p : nullptr;
+    Pc.H2idx = idx_panel ? dI + c0 * p : nullptr;
+    Pc.m = m - c0;
+    Pc.n_tiles_t = t1 - t0;
+    run_scan(ctx, Pc);
+    CUDA_TRY(cudaEventRecord(ctx->chunk_ev[ch], ctx->stream));
+  }
+  for (int ch = 0; ch < nchunk; ++ch) {
+    const int64_t c0 = cbeg[ch], c1 = cbeg[ch + 1];
+    if (c1 == c0) continue;
+    CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->chunk_ev[ch], 0));
+    // indices first: their expansion then overlaps the (8x larger) copy of the chunk's LOD columns
+    if (idx_panel) {
+      CUDA_TRY(cudaMemcpyAsync(ctx->h_idx + c0 * p, dI + c0 * p, (size_t)(c1 - c0) * p, cudaMemcpyDeviceToHost,
+                               ctx->copy_stream));
+      CUDA_TRY(cudaEventRecord(ctx->idx_ev[ch], ctx->copy_stream));
+      hostpipe_push_staged(pipe, ctx->idx_ev[ch], h2_out + c0 * ld, ld, ctx->h_idx + c0 * p, p, c1 - c0, o->h2_grid);
+    }
+    matrix_to_host(ctx, ctx->copy_stream, L_out + c0 * ld, ld, dL + c0 * p, p, c1 - c0, L_pinned);
+    if (dH && !idx_panel) matrix_to_host(ctx, ctx->copy_stream, h2_out + c0 * ld, ld, dH + c0 * p, p, c1 - c0, H_pinned);
+  }
+  const double t_queued = trace_now();
+  finish_and_check(ctx);
+  const double t_scanned = trace_now();
+  CUDA_TRY(cudaStreamSynchronize(ctx->copy_stream));
+  const double t_copied = trace_now();
+  hostpipe_wait(pipe);
+  if (getenv("BLMM_B200_TRACE"))
+    fprintf(stderr, "[blmm trace] dev %d alt-grid host call: queued %.2f ms, scans done %.2f, copies done %.2f, drained %.2f\n",
+            ctx->device, (t_queued - t_enter) * 1e3, (t_scanned - t_enter) * 1e3, (t_copied - t_enter) * 1e3,
+            (trace_now() - t_enter) * 1e3);
+}
+
 int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* L_out, double* h2_out) {
   const double t_enter = trace_now();
   check_problem(pr, true);
@@ -335,21 +459,30 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   const int ms = o->mem_space;
   const int nk = o->ngrid;
   const int64_t p = pr->p, m = pr->m;
-  const int64_t ld = o->ld_out ? o->ld_out : p;
-  if (ld < p) throw Fail{BLMM_E_INVALID, "ld_out < p"};
+  const int64_t ld = out_ld(o, p);
   if (m == 0) return BLMM_OK;
   const double* d_grid = upload_grid(ctx, o);
-  // rotation matrix, covariates and weight constants first (both sides need them), then the marker side forks
+  Results out(ctx, ms);
+  double* dL = out.panel(L_out, S_L, p, m, ld);
+  double* dP = o->chisq_df > 0 ? out.panel(o->log10p_out, S_PVAL, p, m, ld) : nullptr;
+  // alt-grid: the p x m h2 panel; null-grid: h2_null_list, written by the trait statistics
+  double* dH = (alt && h2_out) ? out.panel(h2_out, S_H2P, p, m, ld) : nullptr;
+  double* h2v = (!alt && h2_out) ? out.vec(h2_out, S_H2V, m) : nullptr;
+  const int64_t ldL = out.dev ? ld : p;
   const int64_t p_pad = round_up(p, SCAN_MT);
-  ws<double>(ctx, S_G_IN, ms == BLMM_MEM_HOST ? (size_t)pr->n * p : 1);  // (re)allocations before the fork: cudaFree
-  ws<double>(ctx, S_G0, (size_t)num_kchunks(pr->n) * KC * p);            // would otherwise synchronise mid-overlap
+  reserve_marker_ws(ctx, pr, ms);
   double* Mop = ws<double>(ctx, S_MOP, (size_t)nk * num_kchunks(pr->n) * KC * p_pad);
   WeightConsts wc = weight_ws(ctx, nk, num_kchunks(pr->n) * KC, (int)pr->c);
-  // second stream: covariate rotation -> weight constants -> marker rotation -> marker operand;
-  // main stream: trait rotation, then (after the weight constants) the trait statistics
+  Rotated R = stage_inputs(ctx, pr, ms);
+  // The marker side of a grid scan (G -> U'G -> weight-folded marker operand) depends only on G, U and the per-h2
+  // weight constants, the trait side only on Y: the two chains are latency-bound on their own, so the covariate
+  // rotation, the weight constants and the marker operand run on the second stream (U'G on the third) while the main
+  // stream does the trait rotation and then (after the weight constants) the trait statistics.
+  CUDA_TRY(cudaEventRecord(ctx->fork_ev, ctx->stream));
+  CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->fork_ev, 0));
   const bool rot_in_wc = pr->n <= 128;  // small n: the covariate rotation is folded into the weight-constant blocks
-  Rotated R = rotate_inputs(ctx, pr, ms, false, false, true, !rot_in_wc);
-  rotate_markers_aside(ctx, pr, R, ms, ctx->stream);  // third stream: G -> U'G beside the covariate chain
+  if (!rot_in_wc) rotate_covariates(ctx, R, ctx->copy_stream);
+  rotate_markers_aside(ctx, pr, R, ms);
   if (rot_in_wc)
     ctx->launches += launch_weight_consts_rot(d_grid, nk, R.lambda, R.dU, R.dC, R.n, R.n_pad, R.c, wc, R.C0,
                                               ctx->d_flags, ctx->copy_stream);
@@ -357,7 +490,10 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
     ctx->launches += launch_weight_consts(d_grid, nk, R.lambda, R.C0, R.n, R.n_pad, R.c, wc, ctx->d_flags,
                                           ctx->copy_stream);
   CUDA_TRY(cudaEventRecord(ctx->wc_ev, ctx->copy_stream));
-  fork_marker_side(ctx, pr, R, ms, nk, wc, true, Mop, p_pad, true);
+  wait_markers(ctx, ctx->copy_stream);
+  ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, nk, wc, true, Mop, ctx->d_flags,
+                                         ctx->copy_stream);
+  CUDA_TRY(cudaEventRecord(ctx->join_ev, ctx->copy_stream));
   rotate_traits(ctx, pr, R, ms);
   CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ctx->wc_ev, 0));
 
@@ -370,9 +506,6 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   int* bin_count = bins, *bin_start = bins + 256, *bin_cursor = bins + 512, *n_tiles = bins + 768;
   CUDA_TRY(cudaMemsetAsync(bins, 0, (3 * 256 + 8) * sizeof(int), ctx->stream));
 
-  // null-grid: h2_null_list is written straight into the caller's array in device mode
-  double* h2v = nullptr;
-  if (!alt && h2_out) h2v = (ms == BLMM_MEM_DEVICE) ? h2_out : ws<double>(ctx, S_H2V, m);
   // alt-grid: the statistics kernel also writes the packed trait operand and the per-k scalars when it can
   TraitFuse fuse{nullptr, nullptr, nullptr, 0, false};
   if (alt) {
@@ -395,27 +528,20 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   P.m = m;
   P.half_n = (double)R.n / 2.0;
   P.argmax_mode = (o->h2_panel_mode == BLMM_H2PANEL_ARGMAX) ? 1 : 0;
-  double* dL = (ms == BLMM_MEM_DEVICE) ? L_out : ws<double>(ctx, S_L, (size_t)p * m);
   P.L = dL;
-  P.ldL = (ms == BLMM_MEM_DEVICE) ? ld : p;
-  double* dH = nullptr;
+  P.ldL = ldL;
   if (alt) {
-    const int64_t tcol_pad = fuse.tcol_pad;
-    double *e = fuse.e, *et = fuse.et, *Top = fuse.Top;
     if (!fuse.done) {
-      ctx->launches += launch_alt_scalars(ell, rss, ellmax, m, tcol_pad, nk, R.n, e, et, ctx->stream);
-      ctx->launches += launch_pack_traits(Yr, nullptr, m, tcol_pad, R.n_pad, nullptr, Top, ctx->stream);
+      ctx->launches += launch_alt_scalars(ell, rss, ellmax, m, fuse.tcol_pad, nk, R.n, fuse.e, fuse.et, ctx->stream);
+      ctx->launches += launch_pack_traits(Yr, nullptr, m, fuse.tcol_pad, R.n_pad, nullptr, fuse.Top, ctx->stream);
     }
-    P.Top = Top;
-    P.e = e;
-    P.et = et;
-    P.tcol_pad = tcol_pad;
-    P.n_tiles_t = (int)(tcol_pad / SCAN_TT);
+    P.Top = fuse.Top;
+    P.e = fuse.e;
+    P.et = fuse.et;
+    P.tcol_pad = fuse.tcol_pad;
+    P.n_tiles_t = (int)(fuse.tcol_pad / SCAN_TT);
     P.nk = nk;
-    if (h2_out) {
-      dH = (ms == BLMM_MEM_DEVICE) ? h2_out : ws<double>(ctx, S_H2P, (size_t)p * m);
-      P.H2 = dH;
-    }
+    P.H2 = dH;
   } else {
     const int64_t tcol_pad = round_up(m, SCAN_TT) + (int64_t)nk * SCAN_TT;
     int* tile_k0 = ws<int>(ctx, S_TILEK0, tcol_pad / SCAN_TT);
@@ -439,105 +565,13 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
     P.nk = 1;
   }
   CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ctx->join_ev, 0));  // marker operand ready
-  if (ms == BLMM_MEM_HOST && alt && P.n_tiles_t >= 16 && o->chisq_df <= 0) {
-    // Host-buffer alt-grid: the p x m panels (2 x 2 GB at BXD size) leave over PCIe, which takes ~4x the scan
-    // itself.  The trait tiles are scanned in chunks, and each chunk's columns are copied back on the second stream
-    // while the next chunks are scanned.  The h2 panel holds one of <= 255 grid values per entry, so it crosses
-    // PCIe as one-byte grid indices (1/8 of the bytes) through the pinned ring and is expanded to grid[index] in
-    // the caller's Float64 array by the drain threads; L goes straight into a pinned destination, or through the
-    // same ring into a pageable one (blmm_hostpipe.cu).
-    const int n_tiles = P.n_tiles_t;
-    // PCIe is the bottleneck, so what matters is how soon the first copy starts: more, smaller chunks for big panels
-    const int nchunk = n_tiles >= 64 ? MAX_CHUNK : 8;
-    // The index encoding is worth it when the panel is large (PCIe time saved > host expansion time): >= 1e8
-    // entries by default.  BLMM_B200_H2_TRANSFER = index | f64 overrides; BLMM_B200_HOST_THREADS sets the drain
-    // thread count (default min(16, cores - 1), divided between the GPUs of a multi-GPU context).
-    const char* h2_mode = getenv("BLMM_B200_H2_TRANSFER");
-    const bool want_idx = h2_mode ? (h2_mode[0] == 'i') : (ctx->idx_hint >= 0 ? ctx->idx_hint == 1 : (double)p * (double)m >= 1e8);
-    const bool idx_panel = dH && want_idx && P.nq <= scan_max_nq(P.nk);
-    uint8_t* dI = idx_panel ? ws<uint8_t>(ctx, S_H2IDX, (size_t)p * m) : nullptr;
-    if (idx_panel && ctx->h_idx_cap < (size_t)p * m) {
-      // the whole index panel has its own pinned staging (1 byte per entry), so that queueing its copies never
-      // waits for a ring slot: every copy of the call is in the stream before the first one has finished
-      if (ctx->h_idx) CUDA_TRY(cudaFreeHost(ctx->h_idx));
-      ctx->h_idx = nullptr;
-      ctx->h_idx_cap = 0;
-      CUDA_TRY(cudaMallocHost(&ctx->h_idx, (size_t)p * m));
-      ctx->h_idx_cap = (size_t)p * m;
-    }
-    const bool L_pinned = host_ptr_is_pinned(L_out);
-    const bool H_pinned = h2_out && host_ptr_is_pinned(h2_out);
-    HostPipe* pipe = (idx_panel || !L_pinned || (dH && !H_pinned)) ? host_pipe(ctx) : nullptr;
-    // only index expansion to do (every Float64 copy is a direct DMA): a few drain threads, not all of them
-    hostpipe_set_active(pipe, (L_pinned && (idx_panel || !dH || H_pinned)) ? 6 : 1 << 30);
-    // Chunk boundaries in trait tiles.  The link idles until the first chunk exists, so the first two chunks are small
-    // (1/4 and 1/2 of an even share, at least one tile) and the rest share what is left evenly.
-    int tbeg[MAX_CHUNK + 1];
-    {
-      const int even = n_tiles / nchunk;
-      const int first = std::max(1, even / 4), second = std::max(1, even / 2);
-      tbeg[0] = 0;
-      tbeg[1] = std::min(n_tiles, first);
-      tbeg[2] = std::min(n_tiles, first + second);
-      const int rest = n_tiles - tbeg[2];
-      for (int ch = 3; ch <= nchunk; ++ch) tbeg[ch] = tbeg[2] + (int)((int64_t)rest * (ch - 2) / (nchunk - 2));
-    }
-    int64_t cbeg[MAX_CHUNK + 1];
-    for (int ch = 0; ch <= nchunk; ++ch) cbeg[ch] = std::min<int64_t>((int64_t)tbeg[ch] * SCAN_TT, m);
-    // every chunk's scan is queued first: the copy loop below may block on ring slots
-    for (int ch = 0; ch < nchunk; ++ch) {
-      const int t0 = tbeg[ch], t1 = tbeg[ch + 1];
-      if (t1 == t0) continue;
-      const int64_t c0 = cbeg[ch];
-      ScanParams Pc = P;
-      Pc.Top = P.Top + (int64_t)t0 * SCAN_TT * KC;
-      Pc.e = P.e + (int64_t)t0 * SCAN_TT;
-      Pc.et = P.et + (int64_t)t0 * SCAN_TT;
-      Pc.L = dL + c0 * p;
-      Pc.H2 = (dH && !idx_panel) ? dH + c0 * p : nullptr;
-      Pc.H2idx = idx_panel ? dI + c0 * p : nullptr;
-      Pc.m = m - c0;
-      Pc.n_tiles_t = t1 - t0;
-      run_scan(ctx, Pc);
-      CUDA_TRY(cudaEventRecord(ctx->chunk_ev[ch], ctx->stream));
-    }
-    for (int ch = 0; ch < nchunk; ++ch) {
-      const int64_t c0 = cbeg[ch], c1 = cbeg[ch + 1];
-      if (c1 == c0) continue;
-      CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->chunk_ev[ch], 0));
-      // indices first: their expansion then overlaps the (8x larger) copy of the chunk's LOD columns
-      if (idx_panel) {
-        CUDA_TRY(cudaMemcpyAsync(ctx->h_idx + c0 * p, dI + c0 * p, (size_t)(c1 - c0) * p, cudaMemcpyDeviceToHost,
-                                 ctx->copy_stream));
-        CUDA_TRY(cudaEventRecord(ctx->idx_ev[ch], ctx->copy_stream));
-        hostpipe_push_staged(pipe, ctx->idx_ev[ch], h2_out + c0 * ld, ld, ctx->h_idx + c0 * p, p, c1 - c0, o->h2_grid);
-      }
-      matrix_to_host(ctx, ctx->copy_stream, L_out + c0 * ld, ld, dL + c0 * p, p, c1 - c0, L_pinned);
-      if (dH && !idx_panel) matrix_to_host(ctx, ctx->copy_stream, h2_out + c0 * ld, ld, dH + c0 * p, p, c1 - c0, H_pinned);
-    }
-    const double t_queued = trace_now();
-    finish_and_check(ctx);
-    const double t_scanned = trace_now();
-    CUDA_TRY(cudaStreamSynchronize(ctx->copy_stream));
-    const double t_copied = trace_now();
-    hostpipe_wait(pipe);
-    if (getenv("BLMM_B200_TRACE"))
-      fprintf(stderr, "[blmm trace] dev %d alt-grid host call: queued %.2f ms, scans done %.2f, copies done %.2f, drained %.2f\n",
-              ctx->device, (t_queued - t_enter) * 1e3, (t_scanned - t_enter) * 1e3, (t_copied - t_enter) * 1e3,
-              (trace_now() - t_enter) * 1e3);
+  if (!out.dev && alt && P.n_tiles_t >= 16 && o->chisq_df <= 0) {
+    alt_grid_to_host_chunked(ctx, P, o, L_out, h2_out, dL, dH, ld, t_enter);  // delivers L and the h2 panel itself
     return BLMM_OK;
   }
   run_scan(ctx, P);
-  double* dP = pvals_after_scan(ctx, o, dL, p, m, P.ldL);
-
-  if (ms == BLMM_MEM_HOST) {
-    matrix_to_host(ctx, ctx->stream, L_out, ld, dL, p, m, !via_ring(L_out, p, m));
-    if (dP) matrix_to_host(ctx, ctx->stream, o->log10p_out, ld, dP, p, m, !via_ring(o->log10p_out, p, m));
-    if (dH) matrix_to_host(ctx, ctx->stream, h2_out, ld, dH, p, m, !via_ring(h2_out, p, m));
-    if (h2v) copy_out(ctx, h2_out, h2v, m, ms);
-    finish_and_check(ctx);
-    hostpipe_wait(ctx->pipe);
-  }
+  pvals_after_scan(ctx, o, dL, dP, p, m, ldL);
+  out.deliver();
   return BLMM_OK;
 }
 
@@ -548,22 +582,23 @@ int grid_loglik(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, doubl
   const int64_t m = pr->m;
   if (m == 0) return BLMM_OK;
   const double* d_grid = upload_grid(ctx, o);
-  Rotated R = rotate_inputs(ctx, pr, ms, false);
+  Results out(ctx, ms);
+  double* ell = out.vec(ell_out, S_ELL, (size_t)nk * m);
+  Rotated R = stage_inputs(ctx, pr, ms);
+  rotate_covariates(ctx, R, ctx->stream);
+  rotate_traits(ctx, pr, R, ms);
   WeightConsts wc = weight_ws(ctx, nk, R.n_pad, R.c);
   ctx->launches += launch_weight_consts(d_grid, nk, R.lambda, R.C0, R.n, R.n_pad, R.c, wc, ctx->d_flags, ctx->stream);
   double* Yr = ws<double>(ctx, S_YR, (size_t)R.n_pad * m);
-  double* ell = (ms == BLMM_MEM_DEVICE) ? ell_out : ws<double>(ctx, S_ELL, (size_t)nk * m);
   double* rss = ws<double>(ctx, S_RSS, (size_t)nk * m);
   int* best = ws<int>(ctx, S_BEST, m);
   double* ellmax = ws<double>(ctx, S_ELLMAX, m);
   ctx->launches += launch_trait_stats(R.Y0, m, R.n, R.n_pad, R.c, nk, wc, lik_of(o), d_grid, Yr, ell, rss, best,
                                       ellmax, nullptr, nullptr, ctx->d_flags, ctx->stream);
-  if (ms == BLMM_MEM_HOST) {
-    copy_out(ctx, ell_out, ell, (size_t)nk * m, ms);
-    // a zero-norm trait is only an error for the scans (colDivide!), not for wls_multivar
-    CUDA_TRY(cudaMemsetAsync(ctx->d_flags + FLAG_ZERO_NORM, 0, sizeof(int), ctx->stream));
-    finish_and_check(ctx);
-  }
+  // a zero-norm trait is only an error for the scans (colDivide!), not for wls_multivar (a device-mode call leaves
+  // the flag for the next blmm_sync)
+  if (!out.dev) CUDA_TRY(cudaMemsetAsync(ctx->d_flags + FLAG_ZERO_NORM, 0, sizeof(int), ctx->stream));
+  out.deliver();
   return BLMM_OK;
 }
 
@@ -587,21 +622,18 @@ int fit_h2(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* h2
   const int ms = o->mem_space;
   const int64_t m = pr->m;
   if (m == 0) return BLMM_OK;
-  if (o->optim_interval < 1) throw Fail{BLMM_E_INVALID, "optim_interval must be >= 1"};
-  Rotated R = rotate_inputs(ctx, pr, ms, false);
+  check_optim_interval(o);
+  Results out(ctx, ms);
+  double* h2 = out.vec(h2_out, S_H2V, m);
+  double* s2 = out.vec(sigma2_out, S_SIG2, m);
+  double* el = out.vec(ell_out, S_ELLV, m);
+  Rotated R = stage_inputs(ctx, pr, ms);
+  rotate_covariates(ctx, R, ctx->stream);
+  rotate_traits(ctx, pr, R, ms);
   double* Yr = residualised_traits(ctx, R, o);
-  const bool dev = ms == BLMM_MEM_DEVICE;
-  double* h2 = (dev && h2_out) ? h2_out : ws<double>(ctx, S_H2V, m);
-  double* s2 = (dev && sigma2_out) ? sigma2_out : ws<double>(ctx, S_SIG2, m);
-  double* el = (dev && ell_out) ? ell_out : ws<double>(ctx, S_ELLV, m);
   ctx->launches += launch_fit_h2(Yr, m, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2, el,
                                  ctx->d_flags, ctx->stream);
-  if (!dev) {
-    copy_out(ctx, h2_out, h2, m, ms);
-    copy_out(ctx, sigma2_out, s2, m, ms);
-    copy_out(ctx, ell_out, el, m, ms);
-    finish_and_check(ctx);
-  }
+  out.deliver();
   return BLMM_OK;
 }
 
@@ -611,17 +643,22 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
                    double* sigma2_out) {
   check_problem(pr, true);
   if (!L_out) throw Fail{BLMM_E_INVALID, "L_out is NULL"};
-  if (o->optim_interval < 1) throw Fail{BLMM_E_INVALID, "optim_interval must be >= 1"};
+  check_optim_interval(o);
   const int ms = o->mem_space;
-  const bool dev = ms == BLMM_MEM_DEVICE;
   const int64_t p = pr->p, m = pr->m;
-  const int64_t ld = o->ld_out ? o->ld_out : p;
-  if (ld < p) throw Fail{BLMM_E_INVALID, "ld_out < p"};
+  const int64_t ld = out_ld(o, p);
   if (m == 0) return BLMM_OK;
-  Rotated R = rotate_inputs(ctx, pr, ms, true);
+  Results out(ctx, ms);
+  double* dL = out.panel(L_out, S_L, p, m, ld);
+  double* dP = o->chisq_df > 0 ? out.panel(o->log10p_out, S_PVAL, p, m, ld) : nullptr;
+  double* h2 = out.vec(h2_out, S_H2V, m);
+  double* s2 = out.vec(sigma2_out, S_SIG2, m);
+  reserve_marker_ws(ctx, pr, ms);
+  Rotated R = stage_inputs(ctx, pr, ms);
+  rotate_covariates(ctx, R, ctx->stream);
+  rotate_traits(ctx, pr, R, ms);
+  rotate_markers_aside(ctx, pr, R, ms);
   double* Yr = residualised_traits(ctx, R, o);  // also leaves the w = 1 constants in weight slot 0
-  double* h2 = (dev && h2_out) ? h2_out : ws<double>(ctx, S_H2V, m);
-  double* s2 = (dev && sigma2_out) ? sigma2_out : ws<double>(ctx, S_SIG2, m);
   ctx->launches += launch_fit_h2(Yr, m, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2,
                                  nullptr, ctx->d_flags, ctx->stream);
   // markers residualised (unweighted) on the covariates and normalised: r^2 is invariant to both
@@ -643,9 +680,8 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   P.Mop = Mop;
   P.Xop = Xop;
   P.dyinv = dyinv;
-  double* dL = dev ? L_out : ws<double>(ctx, S_L, (size_t)p * m);
   P.L = dL;
-  P.ldL = dev ? ld : p;
+  P.ldL = out.dev ? ld : p;
   P.nq = R.nq;
   P.p = (int)p;
   P.p_pad = (int)p_pad;
@@ -660,22 +696,10 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   bool dynamic = operand_bytes > 100e6;
   if (const char* d = getenv("BLMM_STREAM_DYNAMIC")) dynamic = d[0] == '1';  // test hook: force either scheduler
   P.unit_counter = dynamic ? fresh_unit_counter(ctx) : nullptr;
-  if (ctx->profiling) CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
-  ctx->launches += launch_scan_exact(P, R.c, ctx->sm_count, ctx->stream);
-  if (ctx->profiling) {
-    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
-    ctx->scan_timed = true;
-  }
+  timed_scan(ctx, [&] { ctx->launches += launch_scan_exact(P, R.c, ctx->sm_count, ctx->stream); });
   CUDA_TRY(cudaGetLastError());
-  double* dP = pvals_after_scan(ctx, o, dL, p, m, P.ldL);
-  if (!dev) {
-    matrix_to_host(ctx, ctx->stream, L_out, ld, dL, p, m, !via_ring(L_out, p, m));
-    if (dP) matrix_to_host(ctx, ctx->stream, o->log10p_out, ld, dP, p, m, !via_ring(o->log10p_out, p, m));
-    copy_out(ctx, h2_out, h2, m, ms);
-    copy_out(ctx, sigma2_out, s2, m, ms);
-    finish_and_check(ctx);
-    hostpipe_wait(ctx->pipe);
-  }
+  pvals_after_scan(ctx, o, dL, dP, p, m, P.ldL);
+  out.deliver();
   return BLMM_OK;
 }
 
@@ -685,34 +709,30 @@ int scan_alt(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* 
   if (pr && pr->m != 1) throw Fail{BLMM_E_ONE_TRAIT, "Can only handle one trait."};
   check_problem(pr, true);
   if (!lod_out) throw Fail{BLMM_E_INVALID, "lod_out is NULL"};
-  if (o->optim_interval < 1) throw Fail{BLMM_E_INVALID, "optim_interval must be >= 1"};
+  check_optim_interval(o);
   if (pr->c + 1 > MAXC) throw Fail{BLMM_E_INVALID, "scan_alt supports at most " + std::to_string(MAXC - 1) + " covariates"};
-  const int ms = o->mem_space;
-  const bool dev = ms == BLMM_MEM_DEVICE;
   const int64_t p = pr->p;
-  Rotated R = rotate_inputs(ctx, pr, ms, true);
+  Results out(ctx, o->mem_space);
+  double* dlod = out.vec(lod_out, S_L, p);
+  double* dh2 = h2_each_out ? out.vec(h2_each_out, S_H2P, p) : nullptr;
+  reserve_marker_ws(ctx, pr, o->mem_space);
+  Rotated R = stage_inputs(ctx, pr, o->mem_space);
+  rotate_covariates(ctx, R, ctx->stream);
+  rotate_traits(ctx, pr, R, o->mem_space);
+  rotate_markers_aside(ctx, pr, R, o->mem_space);
   double* Yr = residualised_traits(ctx, R, o);
   double* misc = ws<double>(ctx, S_MISC, 8);  // [0] h2_null, [1] sigma2, [2] ell_null
   ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, misc, misc + 1,
                                  nullptr, ctx->d_flags, ctx->stream);
-  double* dlod = dev ? lod_out : ws<double>(ctx, S_L, p);
-  double* dh2 = h2_each_out ? (dev ? h2_each_out : ws<double>(ctx, S_H2P, p)) : nullptr;
   wait_markers(ctx, ctx->stream);  // U'G was computed on the third stream meanwhile
   const int launched = launch_scan_alt(Yr, R.G0, p, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval,
                                        misc, misc + 2, dlod, dh2, ctx->stream);
   if (!launched) throw Fail{BLMM_E_INVALID, "unsupported covariate count"};
   ctx->launches += launched;
   CUDA_TRY(cudaGetLastError());
-  if (dev) {
-    if (h2_out) CUDA_TRY(cudaMemcpyAsync(h2_out, misc, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-    if (sigma2_out) CUDA_TRY(cudaMemcpyAsync(sigma2_out, misc + 1, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-  } else {
-    copy_out(ctx, lod_out, dlod, p, ms);
-    if (h2_each_out) copy_out(ctx, h2_each_out, dh2, p, ms);
-    if (h2_out) copy_out(ctx, h2_out, misc, 1, ms);
-    if (sigma2_out) copy_out(ctx, sigma2_out, misc + 1, 1, ms);
-    finish_and_check(ctx);
-  }
+  out.copy(h2_out, misc, 1);
+  out.copy(sigma2_out, misc + 1, 1);
+  out.deliver();
   return BLMM_OK;
 }
 
@@ -722,35 +742,40 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
   check_problem(pr, true);
   if (nperms < 0 || (nperms > 0 && !perm_idx)) throw Fail{BLMM_E_INVALID, "perm_idx is NULL"};
   if (!lod_out) throw Fail{BLMM_E_INVALID, "lod_out is NULL"};
-  if (o->optim_interval < 1) throw Fail{BLMM_E_INVALID, "optim_interval must be >= 1"};
+  check_optim_interval(o);
   const int ms = o->mem_space;
-  const bool dev = ms == BLMM_MEM_DEVICE;
   const int64_t p = pr->p;
-  const int64_t ld = o->ld_out ? o->ld_out : p;
-  if (ld < p) throw Fail{BLMM_E_INVALID, "ld_out < p"};
-  // Small n: rotation of y and the covariates, residualisation, Brent, weight constants and the null residual are ONE
-  // launch (null_fit_chain_kernel); otherwise the same steps as separate kernels.
-  const bool fused = pr->n <= 128 && !getenv("BLMM_B200_NO_CHAIN");  // test hook: force the separate kernels
-  Rotated R = rotate_inputs(ctx, pr, ms, true, !fused, false, !fused);
-  double* h2 = (dev && h2_out) ? h2_out : ws<double>(ctx, S_H2V, 1);
-  double* s2 = (dev && sigma2_out) ? sigma2_out : ws<double>(ctx, S_SIG2, 1);
+  const int64_t ld = out_ld(o, p);
+  Results out(ctx, ms);
+  double* d_lod = out.vec(lod_out, S_L, p);
+  // (the h2-panel slot is free in a permutation scan)
+  double* d_Lp = (Lperms_out && nperms > 0) ? out.panel(Lperms_out, S_H2P, p, nperms, ld) : nullptr;
+  double* d_max = (maxlod_out && nperms > 0) ? out.vec(maxlod_out, S_COLMAX, nperms) : nullptr;
+  double* h2 = out.vec(h2_out, S_H2V, 1);
+  double* s2 = out.vec(sigma2_out, S_SIG2, 1);
+  reserve_marker_ws(ctx, pr, ms);
+  Rotated R = stage_inputs(ctx, pr, ms);
   WeightConsts wc = weight_ws(ctx, 1, R.n_pad, R.c);
   double* z = ws<double>(ctx, S_Z, R.n_pad + 8);
   double* zrss = z + R.n_pad;
+  // Small n: rotation of y and the covariates, residualisation, Brent, weight constants and the null residual are ONE
+  // launch (null_fit_chain_kernel), with the markers rotated beside it; otherwise the same steps as separate kernels,
+  // the markers forked after the trait rotation.
+  const bool fused = pr->n <= 128 && !getenv("BLMM_B200_NO_CHAIN");  // test hook: force the separate kernels
   bool chained = false;
   if (fused) {
+    rotate_markers_aside(ctx, pr, R, ms);
     const double* dY = stage_in(ctx, S_Y_IN, pr->Y, (size_t)pr->n, ms);
     double* Yr1 = ws<double>(ctx, S_YR, (size_t)R.n_pad);
     const int launched = launch_null_fit_chain(R.dU, dY, R.dC, R.lambda, R.n, R.n_pad, R.c, lik_of(o), o->optim_interval,
                                                R.C0, Yr1, wc, h2, s2, z, zrss, ctx->d_flags, ctx->stream);
     ctx->launches += launched;
-    chained = launched > 0;
-    if (!chained) {  // does not apply (shared memory): rotate here and fall through to the separate kernels
-      ctx->launches += launch_rotate(R.dU, R.dC, pr->n, R.C0, R.n_pad, R.n_pad, R.n, R.c, ctx->stream);
-      rotate_traits(ctx, pr, R, ms);
-    }
+    chained = launched > 0;  // 0: does not apply (shared memory)
   }
   if (!chained) {
+    rotate_covariates(ctx, R, ctx->stream);
+    rotate_traits(ctx, pr, R, ms);
+    if (!fused) rotate_markers_aside(ctx, pr, R, ms);
     double* Yr = residualised_traits(ctx, R, o);
     ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2,
                                    nullptr, ctx->d_flags, ctx->stream);
@@ -765,16 +790,11 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
 
   const int64_t ncol = nperms + 1;
   const int64_t tcol_pad = round_up(ncol, SCAN_TT);
-  const int32_t* d_perm = nullptr;
-  if (nperms > 0) {
-    if (dev) {
-      d_perm = perm_idx;
-    } else {
-      int32_t* dp = ws<int32_t>(ctx, S_PERM, (size_t)R.n * nperms);
-      CUDA_TRY(cudaMemcpyAsync(dp, perm_idx, (size_t)R.n * nperms * sizeof(int32_t), cudaMemcpyHostToDevice,
-                               ctx->stream));
-      d_perm = dp;
-    }
+  const int32_t* d_perm = nperms > 0 ? perm_idx : nullptr;
+  if (nperms > 0 && !out.dev) {
+    int32_t* dp = ws<int32_t>(ctx, S_PERM, (size_t)R.n * nperms);
+    CUDA_TRY(cudaMemcpyAsync(dp, perm_idx, (size_t)R.n * nperms * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    d_perm = dp;
   }
   double* Top = ws<double>(ctx, S_TOP, (size_t)R.n_pad * tcol_pad);
   double* et1 = ws<double>(ctx, S_ET, tcol_pad);
@@ -793,28 +813,15 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
   P.n_tiles_t = (int)(tcol_pad / SCAN_TT);
   P.nk = 1;
   P.half_n = (double)R.n / 2.0;
-  double* d_lod = dev ? lod_out : ws<double>(ctx, S_L, (size_t)p * (Lperms_out ? ncol : 1));
   P.L0 = d_lod;
-  double* d_Lp = nullptr;
-  if (Lperms_out && nperms > 0) d_Lp = dev ? Lperms_out : d_lod + p;
   P.L = d_Lp;
-  P.ldL = dev ? ld : p;
-  double* d_max = nullptr;
-  if (maxlod_out && nperms > 0) {
-    d_max = dev ? maxlod_out : ws<double>(ctx, S_COLMAX, nperms);
+  P.ldL = out.dev ? ld : p;
+  if (d_max) {
     CUDA_TRY(cudaMemsetAsync(d_max, 0, nperms * sizeof(double), ctx->stream));
     P.colmax = d_max;
   }
   run_scan(ctx, P);
-  if (!dev) {
-    copy_out(ctx, lod_out, d_lod, p, ms);
-    if (d_Lp) matrix_to_host(ctx, ctx->stream, Lperms_out, ld, d_Lp, p, nperms, !via_ring(Lperms_out, p, nperms));
-    if (d_max) copy_out(ctx, maxlod_out, d_max, nperms, ms);
-    copy_out(ctx, h2_out, h2, 1, ms);
-    copy_out(ctx, sigma2_out, s2, 1, ms);
-    finish_and_check(ctx);
-    hostpipe_wait(ctx->pipe);
-  }
+  out.deliver();
   return BLMM_OK;
 }
 
@@ -825,10 +832,8 @@ int kinship(blmm_ctx* ctx, int64_t n, int64_t p, const double* G, double* K_out,
   double* dK = (ms == BLMM_MEM_DEVICE) ? K_out : ws<double>(ctx, S_KIN, (size_t)n * n);
   ctx->launches += launch_kinship(dG, (int)n, p, dK, part, ctx->stream);
   CUDA_TRY(cudaGetLastError());
-  if (ms == BLMM_MEM_HOST) {
-    copy_out(ctx, K_out, dK, (size_t)n * n, ms);
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  }
+  copy_out(ctx, K_out, dK, (size_t)n * n, ms);
+  if (ms == BLMM_MEM_HOST) CUDA_TRY(cudaStreamSynchronize(ctx->stream));
   return BLMM_OK;
 }
 
@@ -893,10 +898,8 @@ int decompose(blmm_ctx* ctx, int64_t n, const double* K, int scheme, double* U_o
                                                                              scheme == BLMM_DECOMP_SVD, dU, dl);
   ctx->launches += 1;
   CUDA_TRY(cudaGetLastError());
-  if (ms == BLMM_MEM_HOST) {
-    copy_out(ctx, U_out, dU, nn, ms);
-    copy_out(ctx, lambda_out, dl, n, ms);
-  }
+  copy_out(ctx, U_out, dU, nn, ms);
+  copy_out(ctx, lambda_out, dl, n, ms);
   CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // `order` is a host temporary
   return BLMM_OK;
 }
@@ -981,10 +984,8 @@ int weight_kinship(blmm_ctx* ctx, int64_t n, const double* K, const double* w, d
   double* out = (ms == BLMM_MEM_DEVICE) ? K_out : ws<double>(ctx, S_EIGV, (size_t)n * n + n + 8);
   ctx->launches += launch_weight_kinship(dK, dw, (int)n, out, ctx->stream);
   CUDA_TRY(cudaGetLastError());
-  if (ms == BLMM_MEM_HOST) {
-    copy_out(ctx, K_out, out, (size_t)n * n, ms);
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  }
+  copy_out(ctx, K_out, out, (size_t)n * n, ms);
+  if (ms == BLMM_MEM_HOST) CUDA_TRY(cudaStreamSynchronize(ctx->stream));
   return BLMM_OK;
 }
 
@@ -1017,6 +1018,15 @@ int guarded(blmm_ctx* ctx, F&& f) {
     ctx->err = "unknown failure";
     return BLMM_E_INVALID;
   }
+}
+
+// the scan entry points: guarded() with the options checked first
+template <typename F>
+int guarded(blmm_ctx* ctx, const blmm_opts* opts, F&& f) {
+  return guarded(ctx, [&] {
+    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
+    return f();
+  });
 }
 
 }  // namespace
@@ -1193,8 +1203,7 @@ int blmm_rotate(blmm_ctx* ctx, const blmm_problem* prob, double* Y0_out, double*
 
 int blmm_bulkscan(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* L_out, double* h2_out) {
   if (ctx && ctx->multi) return multi_bulkscan(ctx, prob, opts, L_out, h2_out);
-  return guarded(ctx, [&] {
-    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
+  return guarded(ctx, opts, [&] {
     switch (opts->method) {
       case BLMM_METHOD_NULL_GRID:
       case BLMM_METHOD_ALT_GRID:
@@ -1209,19 +1218,13 @@ int blmm_bulkscan(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts
 
 int blmm_grid_loglik(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* ell_out) {
   if (ctx && ctx->multi) return multi_grid_loglik(ctx, prob, opts, ell_out);
-  return guarded(ctx, [&] {
-    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
-    return grid_loglik(ctx, prob, opts, ell_out);
-  });
+  return guarded(ctx, opts, [&] { return grid_loglik(ctx, prob, opts, ell_out); });
 }
 
 int blmm_fit_h2(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* h2_out, double* sigma2_out,
                 double* ell_out) {
   if (ctx && ctx->multi) return multi_fit_h2(ctx, prob, opts, h2_out, sigma2_out, ell_out);
-  return guarded(ctx, [&] {
-    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
-    return fit_h2(ctx, prob, opts, h2_out, sigma2_out, ell_out);
-  });
+  return guarded(ctx, opts, [&] { return fit_h2(ctx, prob, opts, h2_out, sigma2_out, ell_out); });
 }
 
 int blmm_scan_perms(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, const int32_t* perm_idx,
@@ -1229,8 +1232,7 @@ int blmm_scan_perms(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* op
                     double* h2_out) {
   if (ctx && ctx->multi)
     return multi_scan_perms(ctx, prob, opts, perm_idx, nperms, lod_out, Lperms_out, maxlod_out, sigma2_out, h2_out);
-  return guarded(ctx, [&] {
-    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
+  return guarded(ctx, opts, [&] {
     return scan_perms(ctx, prob, opts, perm_idx, nperms, lod_out, Lperms_out, maxlod_out, sigma2_out, h2_out);
   });
 }
@@ -1238,16 +1240,12 @@ int blmm_scan_perms(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* op
 int blmm_scan_null(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* lod_out,
                    double* sigma2_out, double* h2_out) {
   if (ctx && ctx->multi) return multi_scan_null(ctx, prob, opts, lod_out, sigma2_out, h2_out);
-  return guarded(ctx, [&] {
-    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
-    return bulkscan_exact(ctx, prob, opts, lod_out, h2_out, sigma2_out);
-  });
+  return guarded(ctx, opts, [&] { return bulkscan_exact(ctx, prob, opts, lod_out, h2_out, sigma2_out); });
 }
 
 int blmm_scan_alt(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* lod_out,
                   double* h2_each_marker_out, double* sigma2_out, double* h2_out) {
-  FORWARD_ERR(ctx, guarded(_p, [&] {
-    if (!opts) throw Fail{BLMM_E_INVALID, "opts is NULL"};
+  FORWARD_ERR(ctx, guarded(_p, opts, [&] {
     return scan_alt(_p, prob, opts, lod_out, h2_each_marker_out, sigma2_out, h2_out);
   }));
 }
