@@ -55,6 +55,8 @@ SIGNATURES = {
                                  C.POINTER(C.c_int), C.c_int]),
     "blmm_rotate": (C.c_int, [C.c_void_p, C.POINTER(Problem), C.c_void_p, C.c_void_p, C.c_int]),
     "blmm_bulkscan": (C.c_int, [C.c_void_p, C.POINTER(Problem), C.POINTER(Opts), C.c_void_p, C.c_void_p]),
+    "blmm_bulkscan_peaks": (C.c_int, [C.c_void_p, C.POINTER(Problem), C.POINTER(Opts), C.c_void_p, C.c_void_p,
+                                      C.c_void_p]),
     "blmm_grid_loglik": (C.c_int, [C.c_void_p, C.POINTER(Problem), C.POINTER(Opts), C.c_void_p]),
     "blmm_fit_h2": (C.c_int, [C.c_void_p, C.POINTER(Problem), C.POINTER(Opts), C.c_void_p, C.c_void_p,
                               C.c_void_p]),

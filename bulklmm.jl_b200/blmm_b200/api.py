@@ -217,6 +217,12 @@ class Engine:
         self._check(self.lib.blmm_bulkscan(self.h, C.byref(pr), C.byref(opts), C.c_void_p(L_ptr),
                                            C.c_void_p(h2_ptr) if h2_ptr else None))
 
+    def bulkscan_peaks_raw(self, pr, opts, lod_ptr: int, marker_ptr: Optional[int], h2_ptr: Optional[int]):
+        """blmm_bulkscan_peaks with raw pointers (m doubles, m int64 markers, m doubles)."""
+        vp = lambda a: C.c_void_p(a) if a else None
+        self._check(self.lib.blmm_bulkscan_peaks(self.h, C.byref(pr), C.byref(opts), vp(lod_ptr), vp(marker_ptr),
+                                                 vp(h2_ptr)))
+
     def scan_perms_raw(self, pr, opts, perm_ptr: int, nperms: int, lod_ptr: int, Lperms_ptr: Optional[int],
                        max_ptr: Optional[int], s2_ptr: Optional[int], h2_ptr: Optional[int]):
         vp = lambda a: C.c_void_p(a) if a else None
@@ -245,6 +251,24 @@ class Engine:
             H = np.empty(m) if want_h2 else None
         self._check(self.lib.blmm_bulkscan(self.h, C.byref(pr), C.byref(o), _ptr(Lout), _ptr(H)))
         return (Lout, H, P) if chisq_df else (Lout, H)
+
+    def bulkscan_peaks_host(self, Y, G, Covar, U, lam, method, h2_grid, reml, prior_variance, prior_sample_size,
+                            optim_interval=1, h2_panel_mode=L.H2PANEL_REFERENCE, weights=None, chisq_df=0):
+        """Per-trait peaks of the bulk scan: (lod, marker (0-based int64), h2) or, with chisq_df > 0,
+        (lod, marker, h2, log10p), each of length m; no p x m matrix is formed."""
+        Y, G, Covar, U = _f(Y), _f(G), _f(Covar), _f(U)
+        lam = np.ascontiguousarray(lam, dtype=np.float64)
+        weights = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
+        m = Y.shape[1]
+        pr = self._host_problem(Y, G, Covar, U, lam, weights)
+        P = np.empty(m) if chisq_df else None
+        o, keep = self.make_opts(method=method, reml=reml, prior_variance=prior_variance,
+                                 prior_sample_size=prior_sample_size, h2_grid=h2_grid,
+                                 optim_interval=optim_interval, h2_panel_mode=h2_panel_mode, chisq_df=chisq_df,
+                                 log10p_out=None if P is None else P.ctypes.data)
+        lod, marker, H = np.empty(m), np.empty(m, dtype=np.int64), np.empty(m)
+        self._check(self.lib.blmm_bulkscan_peaks(self.h, C.byref(pr), C.byref(o), _ptr(lod), _ptr(marker), _ptr(H)))
+        return (lod, marker, H, P) if chisq_df else (lod, marker, H)
 
     def grid_loglik(self, Y, Covar, U, lam, h2_grid, reml=False, prior_variance=1.0, prior_sample_size=0.0):
         Y, Covar, U = _f(Y), _f(Covar), _f(U)
@@ -410,6 +434,34 @@ def bulkscan(Y, G, K, Covar=None, method: str = "null-grid", h2_grid=None, nb: i
     if output_pvals:
         out.log10Pvals_mat = res[2]  # fused on the device before the copy-back (blmm_opts.chisq_df)
         out.Chisq_df = chisq_df
+    return out
+
+
+def bulkscan_peaks(Y, G, K, Covar=None, method: str = "null-grid", h2_grid=None, nb: int = 1, nt_blas: int = 1,
+                   addIntercept: bool = True, weights=None, prior_variance: float = 1.0,
+                   prior_sample_size: float = 0.0, reml: bool = False, optim_interval: int = 1,
+                   decomp_scheme: str = "eigen", output_pvals: bool = False, chisq_df: int = 1,
+                   h2_panel_mode: str = "reference", decomposition=None, engine: Optional[Engine] = None):
+    """The per-trait peaks of `bulkscan` with the same keywords, without forming the p x m LOD matrix:
+    `lod[j]` = L[marker[j], j] at the first maximum of column j (NaN ranks highest, as Julia's findmax), `marker`
+    0-based, `h2[j]` = h2_panel[marker[j], j] (alt-grid) or h2_null_list[j]; `log10Pvals` with output_pvals."""
+    eng = engine or default_engine()
+    if method not in _METHODS:
+        raise BlmmError(L.E_INVALID, "unknown method: choose null-exact, null-grid or alt-grid")
+    if h2_grid is None:
+        h2_grid = np.arange(10) / 10.0
+    Y, G, C0, K, weights = _prep(Y, G, Covar, K, weights, addIntercept, eng)
+    if decomposition is None:
+        U, lam, _ = eng.decompose(K, decomp_scheme)
+    else:
+        U, lam = decomposition
+    mode = L.H2PANEL_ARGMAX if h2_panel_mode == "argmax" else L.H2PANEL_REFERENCE
+    res = eng.bulkscan_peaks_host(Y, G, C0, U, lam, _METHODS[method], h2_grid, reml, prior_variance,
+                                  prior_sample_size, optim_interval=optim_interval, h2_panel_mode=mode,
+                                  weights=weights, chisq_df=chisq_df if output_pvals else 0)
+    out = SimpleNamespace(lod=res[0], marker=res[1], h2=res[2])
+    if output_pvals:
+        out.log10Pvals = res[3]
     return out
 
 

@@ -341,7 +341,7 @@ void run_scan(blmm_ctx* ctx, ScanParams P) {
       Q.col_map = P.col_map; Q.grid = P.grid; Q.ngrid = P.ngrid; Q.L = P.L; Q.L0 = P.L0;
       Q.H2 = P.H2; Q.colmax = P.colmax; Q.ldL = P.ldL; Q.nq = P.nq; Q.p = P.p; Q.p_pad = P.p_pad; Q.m = P.m;
       Q.xcol_pad = P.tcol_pad; Q.tcol_pad = P.tcol_pad; Q.n_tt = P.n_tiles_t; Q.nk = P.nk;
-      Q.argmax_mode = P.argmax_mode; Q.half_n = P.half_n;
+      Q.argmax_mode = P.argmax_mode; Q.half_n = P.half_n; Q.peaks = P.peaks;
       Q.unit_counter = fresh_unit_counter(ctx);  // n > 100: operands beyond L2 are the normal case here
       ctx->launches += launch_scan_stream_grid(Q, ctx->sm_count, ctx->stream);
     }
@@ -451,27 +451,50 @@ void alt_grid_to_host_chunked(blmm_ctx* ctx, const ScanParams& P, const blmm_opt
             (trace_now() - t_enter) * 1e3);
 }
 
-int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* L_out, double* h2_out) {
+// The output side of a bulk scan when it is not the p x m panels: the per-trait peaks of blmm_bulkscan_peaks.
+struct PeakOut {
+  double* lod;
+  int64_t* marker;  // may be NULL
+  double* h2;       // may be NULL
+};
+
+// Per-trait peaks occupy the vector results of a call; Results moves 8-byte elements, the int64 markers included.
+int64_t* marker_vec(Results& out, int64_t* user, int64_t m) {
+  return reinterpret_cast<int64_t*>(out.vec(reinterpret_cast<double*>(user), S_PKMARK, m));
+}
+
+// pk == nullptr: L_out / h2_out receive the p x m panels.  pk != nullptr: the same scan keeps one record per trait and
+// 32-marker block (PeakRec) instead, and launch_peak_reduce leaves the m peaks in pk.
+int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* L_out, double* h2_out,
+                  const PeakOut* pk = nullptr) {
   const double t_enter = trace_now();
   check_problem(pr, true);
-  if (!L_out) throw Fail{BLMM_E_INVALID, "L_out is NULL"};
+  if (pk && !pk->lod) throw Fail{BLMM_E_INVALID, "peak_lod_out is NULL"};
+  if (!pk && !L_out) throw Fail{BLMM_E_INVALID, "L_out is NULL"};
   const bool alt = o->method == BLMM_METHOD_ALT_GRID;
   const int ms = o->mem_space;
   const int nk = o->ngrid;
   const int64_t p = pr->p, m = pr->m;
-  const int64_t ld = out_ld(o, p);
+  const int64_t ld = pk ? p : out_ld(o, p);
   if (m == 0) return BLMM_OK;
   const double* d_grid = upload_grid(ctx, o);
   Results out(ctx, ms);
-  double* dL = out.panel(L_out, S_L, p, m, ld);
-  double* dP = o->chisq_df > 0 ? out.panel(o->log10p_out, S_PVAL, p, m, ld) : nullptr;
+  if (pk) h2_out = pk->h2;
+  // peaks: dL, dP and dH are m-vectors of the values at the peak
+  double* dL = pk ? out.vec(pk->lod, S_L, m) : out.panel(L_out, S_L, p, m, ld);
+  double* dP = o->chisq_df <= 0 ? nullptr
+               : pk             ? out.vec(o->log10p_out, S_PVAL, m)
+                                : out.panel(o->log10p_out, S_PVAL, p, m, ld);
   // alt-grid: the p x m h2 panel; null-grid: h2_null_list, written by the trait statistics
-  double* dH = (alt && h2_out) ? out.panel(h2_out, S_H2P, p, m, ld) : nullptr;
+  double* dH = (alt && h2_out) ? (pk ? out.vec(h2_out, S_H2P, m) : out.panel(h2_out, S_H2P, p, m, ld)) : nullptr;
   double* h2v = (!alt && h2_out) ? out.vec(h2_out, S_H2V, m) : nullptr;
+  int64_t* dM = pk ? marker_vec(out, pk->marker, m) : nullptr;
   const int64_t ldL = out.dev ? ld : p;
   const int64_t p_pad = round_up(p, SCAN_MT);
+  const int64_t n_mb = p_pad / (SCAN_MT / 2);  // the 32-marker blocks of both grid kernels
   reserve_marker_ws(ctx, pr, ms);
   double* Mop = ws<double>(ctx, S_MOP, (size_t)nk * num_kchunks(pr->n) * KC * p_pad);
+  PeakRec* parts = pk ? ws<PeakRec>(ctx, S_PEAKS, (size_t)n_mb * m) : nullptr;
   WeightConsts wc = weight_ws(ctx, nk, num_kchunks(pr->n) * KC, (int)pr->c);
   Rotated R = stage_inputs(ctx, pr, ms);
   // The marker side of a grid scan (G -> U'G -> weight-folded marker operand) depends only on G, U and the per-h2
@@ -528,8 +551,9 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   P.m = m;
   P.half_n = (double)R.n / 2.0;
   P.argmax_mode = (o->h2_panel_mode == BLMM_H2PANEL_ARGMAX) ? 1 : 0;
-  P.L = dL;
+  P.L = pk ? nullptr : dL;
   P.ldL = ldL;
+  P.peaks = parts;
   if (alt) {
     if (!fuse.done) {
       ctx->launches += launch_alt_scalars(ell, rss, ellmax, m, fuse.tcol_pad, nk, R.n, fuse.e, fuse.et, ctx->stream);
@@ -541,7 +565,7 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
     P.tcol_pad = fuse.tcol_pad;
     P.n_tiles_t = (int)(fuse.tcol_pad / SCAN_TT);
     P.nk = nk;
-    P.H2 = dH;
+    P.H2 = pk ? nullptr : dH;
   } else {
     const int64_t tcol_pad = round_up(m, SCAN_TT) + (int64_t)nk * SCAN_TT;
     int* tile_k0 = ws<int>(ctx, S_TILEK0, tcol_pad / SCAN_TT);
@@ -565,12 +589,17 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
     P.nk = 1;
   }
   CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ctx->join_ev, 0));  // marker operand ready
-  if (!out.dev && alt && P.n_tiles_t >= 16 && o->chisq_df <= 0) {
+  if (!pk && !out.dev && alt && P.n_tiles_t >= 16 && o->chisq_df <= 0) {
     alt_grid_to_host_chunked(ctx, P, o, L_out, h2_out, dL, dH, ld, t_enter);  // delivers L and the h2 panel itself
     return BLMM_OK;
   }
   run_scan(ctx, P);
-  pvals_after_scan(ctx, o, dL, dP, p, m, ldL);
+  if (pk) {
+    ctx->launches += launch_peak_reduce(parts, n_mb, m, (int)p, alt ? d_grid : nullptr, dL, dM, dH, ctx->stream);
+    pvals_after_scan(ctx, o, dL, dP, m, 1, m);
+  } else {
+    pvals_after_scan(ctx, o, dL, dP, p, m, ldL);
+  }
   out.deliver();
   return BLMM_OK;
 }
@@ -639,20 +668,26 @@ int fit_h2(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* h2
 
 // bulkscan_null (src/bulkscan.jl:212-314): per-trait Brent h2, then univar_liteqtl with the trait's own
 // weights as c+2 operand columns (blmm_scan_stream.cu, EXACT mode).  sigma2_out is optional (scan_null).
+// pk: per-trait peaks instead of the p x m panels, as in bulkscan_grid.
 int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* L_out, double* h2_out,
-                   double* sigma2_out) {
+                   double* sigma2_out, const PeakOut* pk = nullptr) {
   check_problem(pr, true);
-  if (!L_out) throw Fail{BLMM_E_INVALID, "L_out is NULL"};
+  if (pk && !pk->lod) throw Fail{BLMM_E_INVALID, "peak_lod_out is NULL"};
+  if (!pk && !L_out) throw Fail{BLMM_E_INVALID, "L_out is NULL"};
   check_optim_interval(o);
   const int ms = o->mem_space;
   const int64_t p = pr->p, m = pr->m;
-  const int64_t ld = out_ld(o, p);
+  const int64_t ld = pk ? p : out_ld(o, p);
   if (m == 0) return BLMM_OK;
   Results out(ctx, ms);
-  double* dL = out.panel(L_out, S_L, p, m, ld);
-  double* dP = o->chisq_df > 0 ? out.panel(o->log10p_out, S_PVAL, p, m, ld) : nullptr;
+  if (pk) h2_out = pk->h2;
+  double* dL = pk ? out.vec(pk->lod, S_L, m) : out.panel(L_out, S_L, p, m, ld);
+  double* dP = o->chisq_df <= 0 ? nullptr
+               : pk             ? out.vec(o->log10p_out, S_PVAL, m)
+                                : out.panel(o->log10p_out, S_PVAL, p, m, ld);
   double* h2 = out.vec(h2_out, S_H2V, m);
   double* s2 = out.vec(sigma2_out, S_SIG2, m);
+  int64_t* dM = pk ? marker_vec(out, pk->marker, m) : nullptr;
   reserve_marker_ws(ctx, pr, ms);
   Rotated R = stage_inputs(ctx, pr, ms);
   rotate_covariates(ctx, R, ctx->stream);
@@ -680,8 +715,10 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   P.Mop = Mop;
   P.Xop = Xop;
   P.dyinv = dyinv;
-  P.L = dL;
+  P.L = pk ? nullptr : dL;
   P.ldL = out.dev ? ld : p;
+  const int64_t n_mb = p_pad / (mt / 2);
+  P.peaks = pk ? ws<PeakRec>(ctx, S_PEAKS, (size_t)n_mb * m) : nullptr;
   P.nq = R.nq;
   P.p = (int)p;
   P.p_pad = (int)p_pad;
@@ -698,7 +735,12 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   P.unit_counter = dynamic ? fresh_unit_counter(ctx) : nullptr;
   timed_scan(ctx, [&] { ctx->launches += launch_scan_exact(P, R.c, ctx->sm_count, ctx->stream); });
   CUDA_TRY(cudaGetLastError());
-  pvals_after_scan(ctx, o, dL, dP, p, m, P.ldL);
+  if (pk) {
+    ctx->launches += launch_peak_reduce(P.peaks, n_mb, m, (int)p, nullptr, dL, dM, nullptr, ctx->stream);
+    pvals_after_scan(ctx, o, dL, dP, m, 1, m);
+  } else {
+    pvals_after_scan(ctx, o, dL, dP, p, m, P.ldL);
+  }
   out.deliver();
   return BLMM_OK;
 }
@@ -1210,6 +1252,23 @@ int blmm_bulkscan(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts
         return bulkscan_grid(ctx, prob, opts, L_out, h2_out);
       case BLMM_METHOD_NULL_EXACT:
         return bulkscan_exact(ctx, prob, opts, L_out, h2_out, nullptr);
+      default:
+        throw Fail{BLMM_E_INVALID, "unknown method"};
+    }
+  });
+}
+
+int blmm_bulkscan_peaks(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* peak_lod_out,
+                        int64_t* peak_marker_out, double* h2_out) {
+  if (ctx && ctx->multi) return multi_bulkscan_peaks(ctx, prob, opts, peak_lod_out, peak_marker_out, h2_out);
+  return guarded(ctx, opts, [&] {
+    const PeakOut pk{peak_lod_out, peak_marker_out, h2_out};
+    switch (opts->method) {
+      case BLMM_METHOD_NULL_GRID:
+      case BLMM_METHOD_ALT_GRID:
+        return bulkscan_grid(ctx, prob, opts, nullptr, nullptr, &pk);
+      case BLMM_METHOD_NULL_EXACT:
+        return bulkscan_exact(ctx, prob, opts, nullptr, nullptr, nullptr, &pk);
       default:
         throw Fail{BLMM_E_INVALID, "unknown method"};
     }

@@ -183,6 +183,44 @@ __device__ __forceinline__ double fix_lod(double v, double res) {
 }
 
 
+// ---------------------------------------------------------------------------------------------
+// Per-trait peaks (findmax of an LOD column over the markers) reduced in the scan epilogues.
+// ---------------------------------------------------------------------------------------------
+// The first maximum of one output column within one warp's block of markers.
+struct __align__(16) PeakRec {
+  double lod;  // the LOD itself, bit for bit (NaN payload included)
+  int marker;  // 0-based marker index; >= p when the block holds only padding rows
+  int gidx;    // alt-grid: index of that marker's h2 in the grid; otherwise 0
+};
+
+// Julia's findmax order as an integer: every NaN above +Inf (so the first NaN wins), -0.0 below +0.0, numeric order
+// otherwise.  Padding rows (row >= p) get the smallest key and never win.
+__device__ __forceinline__ long long peak_key(double v, int row, int p) {
+  const long long b = __double_as_longlong(v);
+  long long k = b >= 0 ? b : (b ^ 0x7fffffffffffffffLL);
+  k = ((b & 0x7fffffffffffffffLL) > 0x7ff0000000000000LL) ? 0x7fffffffffffffffLL : k;
+  return row < p ? k : (-0x7fffffffffffffffLL - 1);
+}
+
+// (lod, row, gidx) := the candidate (l2, r2, g2) when it ranks higher: a larger key, or the same key at a smaller row
+__device__ __forceinline__ void peak_take(double& lod, int& row, int& gidx, double l2, int r2, int g2, int p) {
+  const long long k1 = peak_key(lod, row, p), k2 = peak_key(l2, r2, p);
+  const bool take = k2 > k1 || (k2 == k1 && r2 < row);
+  lod = take ? l2 : lod;
+  row = take ? r2 : row;
+  gidx = take ? g2 : gidx;
+}
+
+// The same over the lanes lane ^ o, o = o0, 2 o0, ..., 16 (o0 = 4: the 8 marker rows g of a DMMA fragment column)
+__device__ __forceinline__ void peak_over_lanes(double& lod, int& row, int& gidx, int p, int o0) {
+  for (int o = o0; o < 32; o <<= 1) {
+    const double l2 = __shfl_xor_sync(0xffffffffu, lod, o);
+    const int r2 = __shfl_xor_sync(0xffffffffu, row, o);
+    const int g2 = __shfl_xor_sync(0xffffffffu, gidx, o);
+    peak_take(lod, row, gidx, l2, r2, g2, p);
+  }
+}
+
 // 1 / a to full double precision without the division sequence: the hardware's ~20-bit reciprocal estimate and two
 // Newton steps (4 FP64 operations; the result may differ from the correctly rounded quotient in the last bit).
 __device__ __forceinline__ double fast_rcp(double a) {

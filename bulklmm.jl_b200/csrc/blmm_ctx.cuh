@@ -19,7 +19,7 @@ enum Slot {
   S_Y_IN, S_G_IN, S_C_IN, S_U_IN, S_LAM, S_GRID, S_Y0, S_C0, S_G0, S_YR, S_W, S_SW, S_Q, S_SLW, S_LDS,
   S_ELL, S_RSS, S_BEST, S_ELLMAX, S_MOP, S_TOP, S_E, S_ET, S_BINS, S_TILEK0, S_COLMAP, S_L, S_H2P, S_H2V,
   S_SIG2, S_ELLV, S_Z, S_PERM, S_COLMAX, S_KPART, S_KIN, S_SOLVER, S_EIGV, S_MISC, S_XOP, S_DYINV, S_PVAL,
-  S_OBSW, S_UW, S_SORT, S_SORTTMP, S_PROBS, S_H2IDX, S_UNITCTR,
+  S_OBSW, S_UW, S_SORT, S_SORTTMP, S_PROBS, S_H2IDX, S_UNITCTR, S_PEAKS, S_PKMARK,
   S_COUNT
 };
 
@@ -143,5 +143,7 @@ int multi_fit_h2(blmm_ctx* parent, const blmm_problem* prob, const blmm_opts* op
 int multi_scan_null(blmm_ctx* parent, const blmm_problem* prob, const blmm_opts* opts, double* lod_out,
                     double* sigma2_out, double* h2_out);
 int multi_grid_loglik(blmm_ctx* parent, const blmm_problem* prob, const blmm_opts* opts, double* ell_out);
+int multi_bulkscan_peaks(blmm_ctx* parent, const blmm_problem* prob, const blmm_opts* opts, double* peak_lod_out,
+                         int64_t* peak_marker_out, double* h2_out);
 
 }  // namespace blmm

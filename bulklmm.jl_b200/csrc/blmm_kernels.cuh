@@ -168,6 +168,8 @@ struct ScanParams {
   int nk;                  // k-list length of every trait tile
   int argmax_mode;         // 0 = tmax! counter semantics, 1 = arg-max index
   double half_n;           // n / 2
+  PeakRec* peaks;          // non-null: per-trait peaks instead of L / H2 / H2idx / colmax: record col * (p_pad / 32) + mb
+                           // for output column col and the 32-marker block mb (launch_peak_reduce finishes them)
 };
 
 constexpr int SCAN_TT = 128;  // traits per CTA tile
@@ -206,6 +208,7 @@ struct StreamParams {
   int nk;                  // GRID: k-list length
   int argmax_mode;
   double half_n;
+  PeakRec* peaks;          // as ScanParams::peaks, with blocks of 8 * MA markers (half the marker tile)
 };
 int stream_exact_marker_tile(int c);  // marker tile of the EXACT kernel for c covariates
 int stream_grid_marker_tile();
@@ -220,6 +223,10 @@ int launch_scan_stream_grid(const StreamParams& P, int sm_count, cudaStream_t st
 // ---- post-processing (blmm_post.cu) -------------------------------------------------------------
 int launch_lod2log10p(const double* lod, int64_t rows, int64_t cols, int64_t ld_in, int64_t ld_out, int df,
                       double* out, int sm_count, cudaStream_t stream);
+// Per-trait peaks from the scan's partials part[j * n_mb + mb]: peak_lod[j] / peak_marker[j] = the first maximum of
+// column j in findmax order (peak_key), h2[j] = grid[gidx] when both grid and h2 are given.  One warp per column.
+int launch_peak_reduce(const PeakRec* part, int64_t n_mb, int64_t m, int p, const double* grid, double* peak_lod,
+                       int64_t* peak_marker, double* h2, cudaStream_t stream);
 size_t thresholds_workspace_bytes(int64_t n);
 int launch_thresholds(const double* maxlod, int64_t n, const double* probs_dev, int nprob, double* sorted,
                       void* tmp, size_t tmp_bytes, double* out, cudaStream_t stream);

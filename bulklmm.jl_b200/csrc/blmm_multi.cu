@@ -661,6 +661,27 @@ int multi_scan_null(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o
   return finish(parent, rc, fr);
 }
 
+int multi_bulkscan_peaks(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o, double* peak_lod_out,
+                         int64_t* peak_marker_out, double* h2_out) {
+  MultiState* M = parent->multi;
+  if (int e = host_only(parent, pr, o)) return e;
+  if (!peak_lod_out) return fail(parent, BLMM_E_INVALID, "peak_lod_out is NULL");
+  int fr = -1;
+  const int rc = run_all(M, [&](int r) -> int {
+    int64_t j0, j1;
+    shard_cols(pr->m, M->ndev, r, SCAN_TT, &j0, &j1);
+    if (j1 == j0) return BLMM_OK;
+    blmm_problem sp = *pr;
+    sp.Y = pr->Y + j0 * pr->n;
+    sp.m = j1 - j0;
+    blmm_opts so = *o;
+    if (o->log10p_out) so.log10p_out = o->log10p_out + j0;
+    return blmm_bulkscan_peaks(M->sub[r], &sp, &so, peak_lod_out + j0, peak_marker_out ? peak_marker_out + j0 : nullptr,
+                               h2_out ? h2_out + j0 : nullptr);
+  }, &fr);
+  return finish(parent, rc, fr);
+}
+
 int multi_grid_loglik(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o, double* ell_out) {
   MultiState* M = parent->multi;
   if (int e = host_only(parent, pr, o)) return e;

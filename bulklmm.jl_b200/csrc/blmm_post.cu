@@ -96,7 +96,37 @@ __global__ void weight_kinship_kernel(const double* __restrict__ K, const double
   out[idx] = w[a] * K[idx] * w[b];
 }
 
+// One warp per output column j: the first maximum over the column's partials (peak_key order, ties to the smaller
+// marker: a total order, so the result does not depend on which lane saw which record).
+__global__ void peak_reduce_kernel(const PeakRec* __restrict__ part, int64_t n_mb, int64_t m, int p,
+                                   const double* __restrict__ grid, double* __restrict__ peak_lod,
+                                   int64_t* __restrict__ peak_marker, double* __restrict__ h2) {
+  const int64_t j = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (j >= m) return;
+  const PeakRec* r = part + j * n_mb;
+  double lod = 0.0;
+  int row = 0x7fffffff, gi = 0;
+  for (int64_t i = lane; i < n_mb; i += 32) {
+    const PeakRec c = r[i];
+    peak_take(lod, row, gi, c.lod, c.marker, c.gidx, p);
+  }
+  peak_over_lanes(lod, row, gi, p, 1);
+  if (lane == 0) {
+    peak_lod[j] = lod;
+    if (peak_marker) peak_marker[j] = row;
+    if (grid && h2) h2[j] = grid[gi];
+  }
+}
+
 }  // namespace
+
+int launch_peak_reduce(const PeakRec* part, int64_t n_mb, int64_t m, int p, const double* grid, double* peak_lod,
+                       int64_t* peak_marker, double* h2, cudaStream_t stream) {
+  if (m <= 0) return 0;
+  peak_reduce_kernel<<<(unsigned)((m + 7) / 8), 256, 0, stream>>>(part, n_mb, m, p, grid, peak_lod, peak_marker, h2);
+  return 1;
+}
 
 int launch_lod2log10p(const double* lod, int64_t rows, int64_t cols, int64_t ld_in, int64_t ld_out, int df,
                       double* out, int sm_count, cudaStream_t stream) {

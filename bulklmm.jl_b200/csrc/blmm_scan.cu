@@ -86,7 +86,8 @@ __device__ __forceinline__ void dmma884_zero(double& c0, double& c1, double a, d
 
 // HAS_E = false: one-element k-lists with e = 1 (null-grid bins, permutations) — no running minimum,
 // no counter, no h2 panel.  COLMAX: also reduce the per-column maximum (permutation thresholds).
-template <int NQ, bool ARGMAX, bool HAS_E, bool COLMAX>
+// PEAK: store nothing per marker; every warp reduces its 32 markers of each column to one PeakRec instead.
+template <int NQ, bool ARGMAX, bool HAS_E, bool COLMAX, bool PEAK>
 __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const SmemPlan plan = plan_smem(NQ);
@@ -391,6 +392,38 @@ __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
     // stores of the unit (LOD in the accumulator registers), outside the turn
     const int kbase = (HAS_E && ARGMAX && P.tile_k0) ? P.tile_k0[tt] : 0;
     const int row0 = mt * MT + wm * 32 + g;
+    if (PEAK) {
+      // per-trait peaks: the first maximum of each column over the warp's 32 markers, over a in registers and then
+      // over g across the lanes, compared on integer keys (this runs outside the turn, like the stores it replaces)
+      const int* cmap = colmap_s + ((ntop - 1) & 1) * TT;
+#pragma unroll
+      for (int b = 0; b < BT; ++b)
+#pragma unroll
+        for (int cc = 0; cc < 2; ++cc) {
+          double lod = acc[0][b][cc];
+          int row = row0, gi = 0;
+#pragma unroll
+          for (int a = 0; a < 4; ++a) {
+            const int o = (a * BT + b) * 2 + cc;
+            const int ga = HAS_E ? kbase + (int)((cnt[(o >> 2) * VM] >> ((o & 3) * 8)) & 0xFFu) : 0;
+            if (a == 0)
+              gi = ga;
+            else
+              peak_take(lod, row, gi, acc[a][b][cc], row0 + a * 8, ga, P.p);
+          }
+          peak_over_lanes(lod, row, gi, P.p, 4);
+          const int posl = wt * (8 * BT) + b * 8 + 2 * t + cc;
+          const int64_t pos = (int64_t)tt * TT + posl;
+          const int64_t col = P.col_map ? (int64_t)cmap[posl] : (pos < P.m ? pos : -1);
+          if (g == 0 && col >= 0) P.peaks[col * (P.p_pad / 32) + mt * 2 + wm] = PeakRec{lod, row, gi};
+        }
+      if (++mt == n_mt) {
+        mt = 0;
+        ++tt;
+      }
+      TCK(4)
+      continue;
+    }
     const bool full_rows = (mt + 1) * MT <= P.p;  // every marker row of the tile exists
     const int* cmap = colmap_s + ((ntop - 1) & 1) * TT;
 #pragma unroll
@@ -481,16 +514,24 @@ __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
 #endif
 }
 
-template <int NQ, bool ARGMAX, bool HAS_E, bool COLMAX>
+template <int NQ, bool ARGMAX, bool HAS_E, bool COLMAX, bool PEAK = false>
 void launch_one(const ScanParams& P, int sm_count, cudaStream_t stream) {
   const SmemPlan plan = plan_smem(NQ);
-  cudaFuncSetAttribute(scan_kernel<NQ, ARGMAX, HAS_E, COLMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
-  scan_kernel<NQ, ARGMAX, HAS_E, COLMAX><<<sm_count, NTHREADS, plan.bytes, stream>>>(P);
+  cudaFuncSetAttribute(scan_kernel<NQ, ARGMAX, HAS_E, COLMAX, PEAK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       SMEM_LIMIT);
+  scan_kernel<NQ, ARGMAX, HAS_E, COLMAX, PEAK><<<sm_count, NTHREADS, plan.bytes, stream>>>(P);
 }
 
 template <int NQ>
 void launch_nq(const ScanParams& P, int sm_count, cudaStream_t stream) {
-  if (P.e) {
+  if (P.peaks) {
+    if (!P.e)
+      launch_one<NQ, false, false, false, true>(P, sm_count, stream);
+    else if (P.argmax_mode)
+      launch_one<NQ, true, true, false, true>(P, sm_count, stream);
+    else
+      launch_one<NQ, false, true, false, true>(P, sm_count, stream);
+  } else if (P.e) {
     if (P.argmax_mode)
       launch_one<NQ, true, true, false>(P, sm_count, stream);
     else
@@ -523,6 +564,8 @@ extern "C" __attribute__((visibility("default"))) int blmm_debug_scan_trace(long
 int launch_scan(const ScanParams& P, int sm_count, cudaStream_t stream) {
   // combinations the kernel variants do not cover
   if ((!P.e && (P.nk != 1 || !P.et_folded)) || (P.e && P.colmax)) return 0;
+  // peaks replace every per-marker output
+  if (P.peaks && (P.colmax || P.L || P.L0 || P.H2 || P.H2idx)) return 0;
   // the kernel indexes its (unit, k) iterations with 32-bit integers
   if ((int64_t)P.n_tiles_t * (P.p_pad / MT) * (int64_t)(P.nk > 0 ? P.nk : 1) >= 2147483647LL) return 0;
   switch (P.nq) {

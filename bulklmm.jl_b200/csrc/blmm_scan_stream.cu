@@ -53,7 +53,8 @@ __host__ __device__ inline StreamPlan stream_plan(int NB, int MA) {
   return s;
 }
 
-template <int NB, int MA, int MODE, bool ARGMAX>
+// PEAK: store nothing per marker; every warp reduces its 8 * MA markers of each column to one PeakRec instead.
+template <int NB, int MA, int MODE, bool ARGMAX, bool PEAK>
 __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const StreamParams P) {
   constexpr int MT = 2 * 8 * MA;        // markers per CTA tile
   constexpr int TCOLS = ST_TG * 8 * NB;  // operand columns per CTA tile
@@ -298,6 +299,34 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
     const int k0 = (MODE == MODE_GRID && P.tile_k0) ? P.tile_k0[tt] : 0;
     const int kbase = ARGMAX ? k0 : 0;
     const int i_base = mt * MT + wm * 8 * MA + g;
+    if (PEAK) {
+      // per-trait peaks: the first maximum of each column over the warp's 8 * MA markers (over a in registers, then
+      // over g across the lanes); units write disjoint records, so the dynamic scheduler needs no ordering
+#pragma unroll
+      for (int b = 0; b < NBO; ++b)
+#pragma unroll
+        for (int cc = 0; cc < 2; ++cc) {
+          double pl = lod[0][b][cc];
+          int row = i_base, gi = 0;
+#pragma unroll
+          for (int a = 0; a < MA; ++a) {
+            int ga = 0;
+            if (MODE == MODE_GRID) {
+              const int o = (a * NB + b) * 2 + cc;
+              ga = kbase + (int)((cnt[o >> 2] >> ((o & 3) * 8)) & 0xFFu);
+            }
+            if (a == 0)
+              gi = ga;
+            else
+              peak_take(pl, row, gi, lod[a][b][cc], i_base + a * 8, ga, P.p);
+          }
+          peak_over_lanes(pl, row, gi, P.p, 4);
+          const int64_t pos = (int64_t)tt * (ST_TG * 8 * NBO) + wt * (8 * NBO) + b * 8 + 2 * t + cc;
+          const int64_t col = P.col_map ? (int64_t)P.col_map[pos] : (pos < P.m ? pos : -1);
+          if (g == 0 && col >= 0) P.peaks[col * (P.p_pad / (8 * MA)) + mt * 2 + wm] = PeakRec{pl, row, gi};
+        }
+      continue;
+    }
 #pragma unroll
     for (int b = 0; b < NBO; ++b)
 #pragma unroll
@@ -471,16 +500,26 @@ __global__ void __launch_bounds__(256) exact_columns_kernel(const double* __rest
   }
 }
 
-template <int NB, int MA, int MODE>
-void launch_stream_one(const StreamParams& P, int sm_count, cudaStream_t stream) {
+template <int NB, int MA, int MODE, bool PEAK>
+void launch_stream_peak(const StreamParams& P, int sm_count, cudaStream_t stream) {
   const StreamPlan plan = stream_plan(NB, MA);
   if (MODE == MODE_GRID && P.argmax_mode) {
-    cudaFuncSetAttribute(scan_stream_kernel<NB, MA, MODE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
-    scan_stream_kernel<NB, MA, MODE, true><<<sm_count, 32 * ST_WARPS, plan.bytes, stream>>>(P);
+    cudaFuncSetAttribute(scan_stream_kernel<NB, MA, MODE, true, PEAK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         SMEM_LIMIT);
+    scan_stream_kernel<NB, MA, MODE, true, PEAK><<<sm_count, 32 * ST_WARPS, plan.bytes, stream>>>(P);
   } else {
-    cudaFuncSetAttribute(scan_stream_kernel<NB, MA, MODE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
-    scan_stream_kernel<NB, MA, MODE, false><<<sm_count, 32 * ST_WARPS, plan.bytes, stream>>>(P);
+    cudaFuncSetAttribute(scan_stream_kernel<NB, MA, MODE, false, PEAK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         SMEM_LIMIT);
+    scan_stream_kernel<NB, MA, MODE, false, PEAK><<<sm_count, 32 * ST_WARPS, plan.bytes, stream>>>(P);
   }
+}
+
+template <int NB, int MA, int MODE>
+void launch_stream_one(const StreamParams& P, int sm_count, cudaStream_t stream) {
+  if (P.peaks)
+    launch_stream_peak<NB, MA, MODE, true>(P, sm_count, stream);
+  else
+    launch_stream_peak<NB, MA, MODE, false>(P, sm_count, stream);
 }
 
 }  // namespace

@@ -18,7 +18,7 @@ module BulkLMMB200
 
 using LinearAlgebra, Random, Statistics
 
-export bulkscan, bulkscan_null, bulkscan_null_grid, bulkscan_alt_grid, scan, calcKinship, transform_rotation, Context,
+export bulkscan, bulkscan_peaks, bulkscan_null, bulkscan_null_grid, bulkscan_alt_grid, scan, calcKinship, transform_rotation, Context,
        get_thresholds, thresholds_from_max, lod2log10p, readBXDpheno, readBXDgeno, readGenoProb_ExcludeComplements
 
 const libblmm = get(ENV, "BLMM_B200_LIB", "libblmm_b200.so")
@@ -240,6 +240,38 @@ function bulkscan(Y::Array{Float64, 2}, G::Array{Float64, 2}, Covar::Array{Float
 end
 bulkscan(Y::Array{Float64, 2}, G::Array{Float64, 2}, K::Array{Float64, 2}; kw...) =
     bulkscan(Y, G, ones(size(Y, 1), 1), K; addIntercept = false, kw...)
+
+# Per-trait peaks of `bulkscan` (same keywords) without the p x m matrices (blmm_bulkscan_peaks): for every trait j,
+# lod[j] = L[marker[j], j] at findmax(L[:, j]) (marker 1-based), h2[j] = h2_panel[marker[j], j] (alt-grid) or
+# h2_null_list[j]; log10Pvals with output_pvals.
+function bulkscan_peaks(Y::Array{Float64, 2}, G::Array{Float64, 2}, Covar::Array{Float64, 2}, K::Array{Float64, 2};
+                        method::String = "null-grid", h2_grid::Array{Float64, 1} = collect(0.0:0.1:0.9),
+                        nb::Int64 = Threads.nthreads(), nt_blas::Int64 = 1,
+                        weights::Union{Missing, Array{Float64, 1}} = missing, addIntercept::Bool = true,
+                        prior_variance::Float64 = 1.0, prior_sample_size::Float64 = 0.0, reml::Bool = false,
+                        optim_interval::Int64 = 1, decomp_scheme::String = "eigen", output_pvals::Bool = false,
+                        chisq_df::Int64 = 1, ndev::Int64 = 1)
+    codes = Dict("null-grid" => METHOD_NULL_GRID, "alt-grid" => METHOD_ALT_GRID, "null-exact" => METHOD_NULL_EXACT)
+    haskey(codes, method) || throw(error("unknown method"))
+    ctx = context_for(ndev)
+    Ys, Gs, Cs, Ks, w = prep(Y, G, Covar, K, weights, addIntercept; ctx = ctx)
+    (n, m) = size(Ys); p = size(Gs, 2)
+    U, lambda = decompose(Ks; decomp_scheme = decomp_scheme, ctx = ctx)
+    grid = method == "null-exact" ? Float64[0.0] : h2_grid
+    lod, marker, h2 = Array{Float64, 1}(undef, m), Array{Int64, 1}(undef, m), Array{Float64, 1}(undef, m)
+    P = output_pvals ? Array{Float64, 1}(undef, m) : Array{Float64, 1}(undef, 0)
+    prob = BlmmProblem(n, p, m, size(Cs, 2), pointer(Ys), pointer(Gs), pointer(Cs), pointer(U), pointer(lambda), wptr(w))
+    opts = BlmmOpts(codes[method], reml, prior_variance, prior_sample_size, pointer(grid), length(grid), optim_interval,
+                    H2PANEL_REFERENCE, BLMM_MEM_HOST, 0, output_pvals ? Int32(chisq_df) : Int32(0), Int32(0),
+                    output_pvals ? pointer(P) : Ptr{Float64}(C_NULL))
+    GC.@preserve Ys Gs Cs U lambda w grid lod marker h2 P check(ctx, ccall((:blmm_bulkscan_peaks, libblmm), Cint,
+        (Ptr{Cvoid}, Ref{BlmmProblem}, Ref{BlmmOpts}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}), ctx.handle, prob, opts,
+        lod, marker, h2))
+    marker .+= 1
+    return output_pvals ? (lod = lod, marker = marker, h2 = h2, log10Pvals = P) : (lod = lod, marker = marker, h2 = h2)
+end
+bulkscan_peaks(Y::Array{Float64, 2}, G::Array{Float64, 2}, K::Array{Float64, 2}; kw...) =
+    bulkscan_peaks(Y, G, ones(size(Y, 1), 1), K; addIntercept = false, kw...)
 
 # ---- scan with permutations (src/scan.jl:485-557) ------------------------------------------------------
 # The shuffles are drawn HERE with the reference's own RNG and seed (src/transform_helpers.jl:94-102,

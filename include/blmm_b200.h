@@ -116,7 +116,7 @@ BLMM_API int blmm_abi_version(void);
 BLMM_API int blmm_create(blmm_ctx** out, int device);
 /* One context over `ndev` distinct GPUs of this box (ndev == 1 is blmm_create).  Replaces the `nb` keyword's trait
  * blocks (Threads.@threads, src/bulkscan.jl:263-309) by one host thread + GPU per block:
- *   blmm_bulkscan, blmm_scan_null, blmm_fit_h2, blmm_grid_loglik   shard the m traits,
+ *   blmm_bulkscan, blmm_bulkscan_peaks, blmm_scan_null, blmm_fit_h2, blmm_grid_loglik   shard the m traits,
  *   blmm_scan_perms                                                shards the permutation columns,
  * into contiguous column blocks (cut at the kernel's 128-column tile); G, Covar, U, lambda are replicated.
  *   BLMM_MEM_HOST  : every GPU reads its block of the caller's arrays and writes its slab of the caller's
@@ -173,6 +173,18 @@ BLMM_API int blmm_rotate(blmm_ctx* ctx, const blmm_problem* prob, double* Y0_out
  *           p x m h2_panel (alt-grid; may be NULL to skip the second output).                   */
 BLMM_API int blmm_bulkscan(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts, double* L_out,
                   double* h2_out);
+
+/* Per-trait LOD peaks of bulkscan(Y,G,Covar,K; method=...) without the p x m outputs.  For every trait j:
+ *   peak_lod_out[j]    = L[i*, j]  with i* = findmax(L[:, j]) (first index on ties; NaN ranks above every number)
+ *   peak_marker_out[j] = i* (0-based)
+ *   h2_out[j]          = alt-grid: h2_panel[i*, j] (per opts->h2_panel_mode); null-grid / null-exact: h2_null_list[j]
+ * L and h2_panel are the values blmm_bulkscan returns for the same arguments, bit for bit.
+ * opts->chisq_df > 0: opts->log10p_out receives m values, -log10 p of peak_lod_out.  ld_out is ignored.
+ * peak_marker_out and h2_out may be NULL.  On a multi-GPU context: host buffers only, traits sharded.
+ * The scan keeps one 16-byte record per trait and block of 16 or 32 markers on the device instead of the p x m
+ * matrices, so problems whose L would not fit in device memory can be scanned.                        */
+BLMM_API int blmm_bulkscan_peaks(blmm_ctx* ctx, const blmm_problem* prob, const blmm_opts* opts,
+                                 double* peak_lod_out, int64_t* peak_marker_out, double* h2_out);
 
 /* The |grid| x m matrix of null log-likelihoods `ell_results`, src/bulkscan_helpers.jl:267-269
  * (wls_multivar(...).Ell per grid point, src/wls.jl:103-176).  ell_out: ngrid x m, column-major. */
