@@ -307,7 +307,7 @@ void run_scan(blmm_ctx* ctx, ScanParams P) {
   bool window = false;
   // (k-loop scans only: a one-k scan reads each marker slab once per trait tile of its bin and measured 1-3 % slower
   // with 64 MB of L2 set aside)
-  if (l2_mode > 0 && P.e && P.nq <= scan_max_nq(P.nk)) {
+  if (l2_mode > 0 && P.e && P.nq <= SCAN_MAX_NQ) {
     int maxw = 0, maxp = 0;
     cudaDeviceGetAttribute(&maxw, cudaDevAttrMaxAccessPolicyWindowSize, ctx->device);
     cudaDeviceGetAttribute(&maxp, cudaDevAttrMaxPersistingL2CacheSize, ctx->device);
@@ -329,22 +329,16 @@ void run_scan(blmm_ctx* ctx, ScanParams P) {
     cudaGetLastError();
   }
   timed_scan(ctx, [&] {
-    if (P.nq <= scan_max_nq(P.nk)) {
-      const int launched = launch_scan(P, ctx->sm_count, ctx->stream);
-      if (!launched) throw Fail{BLMM_E_INVALID, "scan kernel: unsupported parameter combination"};
-      ctx->launches += launched;
+    int launched;
+    if (P.nq <= SCAN_MAX_NQ) {
+      launched = launch_scan(P, ctx->sm_count, ctx->stream);
     } else {
       // n too large for the shared-memory-resident trait tile: same arithmetic, K streamed
-      static_assert(SCAN_TT == 128 && SCAN_MT == 64, "packing shared with the streamed GRID kernel");
-      StreamParams Q{};
-      Q.Mop = P.Mop; Q.Xop = P.Top; Q.e = P.e; Q.et = P.et; Q.tile_k0 = P.tile_k0; Q.n_tiles_dev = P.n_tiles_dev;
-      Q.col_map = P.col_map; Q.grid = P.grid; Q.ngrid = P.ngrid; Q.L = P.L; Q.L0 = P.L0;
-      Q.H2 = P.H2; Q.colmax = P.colmax; Q.ldL = P.ldL; Q.nq = P.nq; Q.p = P.p; Q.p_pad = P.p_pad; Q.m = P.m;
-      Q.xcol_pad = P.tcol_pad; Q.tcol_pad = P.tcol_pad; Q.n_tt = P.n_tiles_t; Q.nk = P.nk;
-      Q.argmax_mode = P.argmax_mode; Q.half_n = P.half_n; Q.peaks = P.peaks;
-      Q.unit_counter = fresh_unit_counter(ctx);  // n > 100: operands beyond L2 are the normal case here
-      ctx->launches += launch_scan_stream_grid(Q, ctx->sm_count, ctx->stream);
+      P.unit_counter = fresh_unit_counter(ctx);  // n > 100: operands beyond L2 are the normal case here
+      launched = launch_scan_stream_grid(P, ctx->sm_count, ctx->stream);
     }
+    if (!launched) throw Fail{BLMM_E_INVALID, "scan kernel: unsupported parameter combination"};
+    ctx->launches += launched;
   });
   if (window) {
     cudaStreamAttrValue av;
@@ -388,7 +382,7 @@ void alt_grid_to_host_chunked(blmm_ctx* ctx, const ScanParams& P, const blmm_opt
   // thread count (default min(16, cores - 1), divided between the GPUs of a multi-GPU context).
   const char* h2_mode = getenv("BLMM_B200_H2_TRANSFER");
   const bool want_idx = h2_mode ? (h2_mode[0] == 'i') : (ctx->idx_hint >= 0 ? ctx->idx_hint == 1 : (double)p * (double)m >= 1e8);
-  const bool idx_panel = dH && want_idx && P.nq <= scan_max_nq(P.nk);
+  const bool idx_panel = dH && want_idx && P.nq <= SCAN_MAX_NQ;
   uint8_t* dI = idx_panel ? ws<uint8_t>(ctx, S_H2IDX, (size_t)p * m) : nullptr;
   if (idx_panel && ctx->h_idx_cap < (size_t)p * m) {
     // the whole index panel has its own pinned staging (1 byte per entry), so that queueing its copies never
@@ -491,7 +485,7 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   int64_t* dM = pk ? marker_vec(out, pk->marker, m) : nullptr;
   const int64_t ldL = out.dev ? ld : p;
   const int64_t p_pad = round_up(p, SCAN_MT);
-  const int64_t n_mb = p_pad / (SCAN_MT / 2);  // the 32-marker blocks of both grid kernels
+  const int64_t n_mb = peak_blocks((int)p_pad, SCAN_MT / 2);  // the 32-marker blocks of both grid kernels
   reserve_marker_ws(ctx, pr, ms);
   double* Mop = ws<double>(ctx, S_MOP, (size_t)nk * num_kchunks(pr->n) * KC * p_pad);
   PeakRec* parts = pk ? ws<PeakRec>(ctx, S_PEAKS, (size_t)n_mb * m) : nullptr;
@@ -576,7 +570,7 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
     double* Top = ws<double>(ctx, S_TOP, (size_t)R.n_pad * tcol_pad);
     // shared-memory-resident kernel: 1/rss is folded into the packed trait columns (one FP64 operation less
     // per output); the K-streamed fallback for n > 100 keeps it as the per-column scalar et
-    const bool fold = R.nq <= scan_max_nq(1);
+    const bool fold = R.nq <= SCAN_MAX_NQ;
     ctx->launches += launch_pack_traits(Yr, col_map, m, tcol_pad, R.n_pad, fold ? et : nullptr, Top, ctx->stream);
     P.et_folded = fold ? 1 : 0;
     P.Top = Top;
@@ -711,20 +705,20 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   double* dyinv = ws<double>(ctx, S_DYINV, slots);
   ctx->launches += launch_exact_columns(Yr, h2, R.lambda, R.C0, m, slots, R.n, R.n_pad, R.c, Xop, xcol_pad, dyinv,
                                         ctx->d_flags, ctx->stream);
-  StreamParams P{};
+  ScanParams P{};
   P.Mop = Mop;
-  P.Xop = Xop;
+  P.Top = Xop;
   P.dyinv = dyinv;
   P.L = pk ? nullptr : dL;
   P.ldL = out.dev ? ld : p;
-  const int64_t n_mb = p_pad / (mt / 2);
+  const int64_t n_mb = peak_blocks((int)p_pad, mt / 2);
   P.peaks = pk ? ws<PeakRec>(ctx, S_PEAKS, (size_t)n_mb * m) : nullptr;
   P.nq = R.nq;
   P.p = (int)p;
   P.p_pad = (int)p_pad;
   P.m = m;
-  P.xcol_pad = xcol_pad;
-  P.n_tt = (int)n_tt;
+  P.tcol_pad = xcol_pad;
+  P.n_tiles_t = (int)n_tt;
   P.nk = 1;
   P.half_n = (double)R.n / 2.0;
   if (const char* b = getenv("BLMM_STREAM_BAND")) P.band = atoi(b);  // development knob (L2 rasterisation study)
@@ -733,7 +727,11 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   bool dynamic = operand_bytes > 100e6;
   if (const char* d = getenv("BLMM_STREAM_DYNAMIC")) dynamic = d[0] == '1';  // test hook: force either scheduler
   P.unit_counter = dynamic ? fresh_unit_counter(ctx) : nullptr;
-  timed_scan(ctx, [&] { ctx->launches += launch_scan_exact(P, R.c, ctx->sm_count, ctx->stream); });
+  timed_scan(ctx, [&] {
+    const int launched = launch_scan_exact(P, R.c, ctx->sm_count, ctx->stream);
+    if (!launched) throw Fail{BLMM_E_INVALID, "scan kernel: unsupported parameter combination"};
+    ctx->launches += launched;
+  });
   CUDA_TRY(cudaGetLastError());
   if (pk) {
     ctx->launches += launch_peak_reduce(P.peaks, n_mb, m, (int)p, nullptr, dL, dM, nullptr, ctx->stream);
@@ -846,7 +844,7 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
   P.Top = Top;
   P.Mop = Mop;
   P.et = et1;
-  P.et_folded = (R.nq <= scan_max_nq(1)) ? 1 : 0;  // columns are normalised: v = 1 - d^2
+  P.et_folded = (R.nq <= SCAN_MAX_NQ) ? 1 : 0;  // columns are normalised: v = 1 - d^2
   P.nq = R.nq;
   P.p = (int)p;
   P.p_pad = (int)p_pad;

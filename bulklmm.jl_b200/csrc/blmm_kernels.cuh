@@ -130,7 +130,7 @@ int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_p
                     const double* lambda, LikParams lik, int optim_interval, const double* h2_null, double* ell_null,
                     double* lod, double* h2_each, cudaStream_t stream);
 
-// ---- the fused scan (blmm_scan.cu) ------------------------------------------------------------
+// ---- the scans (blmm_scan.cu, blmm_scan_stream.cu) -----------------------------------------------
 // For every (marker i, packed trait column s):
 //     d_k = sum_l Mop[k][i][l] * Top[s][l]
 //     v_k = e[k][s] - d_k^2 * et[k][s]                      k in the trait tile's k-list
@@ -139,13 +139,15 @@ int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_p
 // = bulkscan_alt_grid (src/bulkscan.jl:445-526, tmax! src/bulkscan_helpers.jl:330-350) in its
 // single-logarithm form; with a one-element k-list and e = 1 it is weighted_liteqtl + r2lod
 // (src/bulkscan_helpers.jl:175-201, 22-24) for null-grid bins and permutations.
+// launch_scan keeps the trait tile in shared memory (nq <= SCAN_MAX_NQ), launch_scan_stream_grid streams K; both, and
+// launch_scan_exact (bulkscan_null, EXACT mode), return 0 and launch nothing for fields their kernel does not implement.
 struct ScanParams {
-  const double* Top;       // trait operand   [nq][tcol_pad][KC]
-  const double* Mop;       // marker operand  [nk_total][nq][p_pad][KC]
+  const double* Top;       // trait operand   [nq][tcol_pad][KC]; EXACT: c+2 column kinds per trait (launch_exact_columns)
+  const double* Mop;       // marker operand  [nk_total][nq][p_pad][KC]  (EXACT: one slab, w = 1)
   const double* e;         // [nk][tcol_pad] or nullptr (=> 1)
-  const double* et;        // [nk][tcol_pad], required
+  const double* et;        // [nk][tcol_pad], required (not read in EXACT mode)
   int et_folded;           // e == nullptr only: et is already folded into the trait operand (columns scaled by
-                           // sqrt(et)), v = 1 - d^2; the K-streamed fallback kernel does not support it
+                           // sqrt(et)), v = 1 - d^2; resident kernel only
   const int* tile_k0;      // per trait tile: first k (index into Mop); nullptr => 0
   const int* n_tiles_dev;  // device scalar: number of trait tiles in use; nullptr => n_tiles_t
   const int* col_map;      // [tcol_pad] packed column -> output column (-1 = padding); nullptr => identity
@@ -156,69 +158,43 @@ struct ScanParams {
                            // column s-1 of L / colmax (scan_perms_lite's lod vs L_perms split, src/scan.jl:545-546)
   double* H2;              // p x m h2 panel, ld = ldL (nullptr => not stored)
   uint8_t* H2idx;          // p x m panel of grid INDICES (h2 = grid[index]), ld = p, one byte each (nullptr => not
-                           // stored): what host-buffer calls bring back over PCIe instead of 8-byte values
+                           // stored): what host-buffer calls bring back over PCIe instead of 8-byte values; resident
+                           // kernel only
   double* colmax;          // [m] max over markers per output column (nullptr => off); caller zero-fills
   int64_t ldL;
   int nq;                  // K-chunks (ceil(n / KC))
   int p;                   // markers
   int p_pad;               // padded marker count (multiple of the marker tile)
   int64_t m;               // output columns
-  int64_t tcol_pad;        // padded packed-trait count (multiple of the trait tile)
-  int n_tiles_t;           // trait tiles (upper bound when n_tiles_dev is given)
+  int64_t tcol_pad;        // padded packed-trait count (multiple of the trait tile); EXACT: operand columns of Top
+  int n_tiles_t;           // trait tiles (upper bound when n_tiles_dev is given); EXACT: tiles of 64 traits
   int nk;                  // k-list length of every trait tile
   int argmax_mode;         // 0 = tmax! counter semantics, 1 = arg-max index
   double half_n;           // n / 2
-  PeakRec* peaks;          // non-null: per-trait peaks instead of L / H2 / H2idx / colmax: record col * (p_pad / 32) + mb
-                           // for output column col and the 32-marker block mb (launch_peak_reduce finishes them)
+  PeakRec* peaks;          // non-null: per-trait peaks instead of L / H2 / H2idx / colmax, one record per output column
+                           // and warp marker block (peak_blocks; launch_peak_reduce finishes them)
+  // K-streamed kernels only
+  const double* dyinv;     // EXACT: [n_tiles_t * 64] 1 / (y_j' z_j)
+  int band;                // trait tiles per rasterisation band (0 = default)
+  unsigned long long* unit_counter;  // device scalar, zero at launch: dynamic unit scheduler (nullptr => round-robin)
 };
+
+// Per-trait peak records (ScanParams::peaks): one per output column and block of `block_rows` markers (the marker rows
+// of one warp, half a marker tile).  The record of column col and block mb is col * peak_blocks(p_pad, block_rows) + mb.
+__host__ __device__ inline int peak_blocks(int p_pad, int block_rows) { return p_pad / block_rows; }
 
 constexpr int SCAN_TT = 128;  // traits per CTA tile
 constexpr int SCAN_MT = 64;   // markers per CTA tile
-// Largest number of K-chunks the shared-memory-resident kernel supports for a k-list of nk.
-int scan_max_nq(int nk);
+constexpr int SCAN_MAX_NQ = 5;  // largest number of K-chunks for which launch_scan keeps the trait tile resident
 int launch_scan(const ScanParams& P, int sm_count, cudaStream_t stream);
+int launch_scan_stream_grid(const ScanParams& P, int sm_count, cudaStream_t stream);
 
-// ---- the K-streamed scans (blmm_scan_stream.cu) -------------------------------------------------
-// Any n.  EXACT mode: per-trait weights (bulkscan_null); GRID mode: ScanParams' arithmetic.
-struct StreamParams {
-  const double* Mop;       // marker operand [nk_total][nq][p_pad][KC]  (EXACT: one slab, w = 1)
-  const double* Xop;       // trait operand  [nq][xcol_pad][KC]; EXACT: (c+2) column kinds per trait
-  const double* dyinv;     // EXACT: [n_tt*64] 1 / (y_j' z_j)
-  const double* e;         // GRID: [nk][tcol_pad] or nullptr (=> 1)
-  const double* et;        // GRID: [nk][tcol_pad]
-  const int* tile_k0;      // GRID: per trait tile first k, or nullptr
-  const int* n_tiles_dev;  // device scalar: trait tiles in use, or nullptr => n_tt
-  const int* col_map;      // packed column -> output column (-1 = padding); nullptr => identity
-  const double* grid;      // h2 grid (device), GRID mode h2 panel
-  int ngrid;
-  double* L;
-  double* L0;
-  double* H2;
-  double* colmax;
-  int64_t ldL;
-  int nq;
-  int p;
-  int p_pad;               // multiple of the marker tile
-  int64_t m;               // output columns
-  int64_t xcol_pad;        // operand columns of Xop
-  int64_t tcol_pad;        // GRID: padded packed-trait count (= xcol_pad)
-  int band;                // trait tiles per rasterisation band (0 = default)
-  unsigned long long* unit_counter;  // device scalar, zero at launch: dynamic unit scheduler (set by the launchers' caller)
-  int n_tt;                // trait tiles (EXACT: 64 traits each; GRID: stream_grid_trait_tile())
-  int nk;                  // GRID: k-list length
-  int argmax_mode;
-  double half_n;
-  PeakRec* peaks;          // as ScanParams::peaks, with blocks of 8 * MA markers (half the marker tile)
-};
 int stream_exact_marker_tile(int c);  // marker tile of the EXACT kernel for c covariates
-int stream_grid_marker_tile();
-int stream_grid_trait_tile();
 // z_j, q_j1..q_jc, w_j columns and 1/dy_j of every trait at its own h2 (slots = n_tt*64 >= m)
 int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* C0, int64_t m,
                          int64_t slots, int n, int n_pad, int c, double* Xop, int64_t xcol_pad, double* dyinv,
                          int* flags, cudaStream_t stream);
-int launch_scan_exact(const StreamParams& P, int c, int sm_count, cudaStream_t stream);
-int launch_scan_stream_grid(const StreamParams& P, int sm_count, cudaStream_t stream);
+int launch_scan_exact(const ScanParams& P, int c, int sm_count, cudaStream_t stream);
 
 // ---- post-processing (blmm_post.cu) -------------------------------------------------------------
 int launch_lod2log10p(const double* lod, int64_t rows, int64_t cols, int64_t ld_in, int64_t ld_out, int df,

@@ -23,7 +23,7 @@
 #include <math.h>
 #include <stdlib.h>
 
-#include "blmm_kernels.cuh"
+#include "blmm_scan_epilogue.cuh"
 
 namespace blmm {
 
@@ -35,7 +35,6 @@ constexpr int BT = 2;        // 8-trait atoms per warp: 16 warps of 32 markers x
 constexpr int WT_WARPS = TT / (8 * BT);
 constexpr int NWARPS = 2 * WT_WARPS;
 constexpr int NTHREADS = 32 * NWARPS;
-constexpr int SMEM_LIMIT = 227 * 1024;
 constexpr int GRID_MAX = 256;
 
 static_assert(NWARPS == 16 && NTHREADS == 512, "ping-pong barrier counts assume 16 warps");
@@ -70,7 +69,7 @@ __host__ __device__ inline SmemPlan plan_smem(int nq) {
   s.stage_doubles = (size_t)nq * MT * KC + 2 * TT;
   s.nstage = 3;
   s.bytes = (s.top_doubles + 3 * s.stage_doubles) * 8 + FIXED_SMEM;
-  if (s.bytes > SMEM_LIMIT) {
+  if (s.bytes > SCAN_SMEM_LIMIT) {
     s.nstage = 2;
     s.bytes = (s.top_doubles + 2 * s.stage_doubles) * 8 + FIXED_SMEM;
   }
@@ -210,10 +209,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
     TCK(5)
     const bool last_of_tt = (u + 1 == u1) || (mt + 1 == n_mt);
 
-    constexpr int VM = HAS_E ? 1 : 0;  // index multiplier: the one-k variants keep no running minimum
     double acc[4][BT][2];
-    double vmin[HAS_E ? 4 : 1][BT][2];
-    uint32_t cnt[HAS_E ? 2 * BT : 1];
+    double vmin[4][BT][2];  // (the one-k variants keep no running minimum: unused there)
+    uint32_t cnt[2 * BT];
     if (HAS_E) {
 #pragma unroll
       for (int i = 0; i < 2 * BT; ++i) cnt[i] = 0u;
@@ -301,56 +299,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
               acc[a][b][cc] = fma(-d, d, 1.0);
             }
       }
-      // tmax! bookkeeping of this k: integer pipe only (strict `<` as `max .< to_compare`, on the bit
-      // patterns: equivalent for the non-negative v that occur; a negative v (r^2 > 1 by rounding)
-      // orders below every positive one, as it should)
+      // tmax! bookkeeping of this k (integer pipe only)
       auto update_min = [&]() {
-        if (HAS_E) {
-          const bool first = (kk == 0);
-#pragma unroll
-          for (int a = 0; a < 4; ++a)
-#pragma unroll
-            for (int b = 0; b < BT; ++b)
-#pragma unroll
-              for (int cc = 0; cc < 2; ++cc) {
-                const double v = acc[a][b][cc];
-                const bool better = __double_as_longlong(v) < __double_as_longlong(vmin[a * VM][b][cc]);
-                const bool upd = first || better;
-                vmin[a * VM][b][cc] = upd ? v : vmin[a * VM][b][cc];
-                const int o = (a * BT + b) * 2 + cc;
-                const int sh = (o & 3) * 8;
-                if (ARGMAX) {
-                  if (upd) cnt[(o >> 2) * VM] = (cnt[(o >> 2) * VM] & ~(0xFFu << sh)) | ((uint32_t)kk << sh);
-                } else {
-                  if (better && !first) cnt[(o >> 2) * VM] += (1u << sh);
-                }
-              }
-        }
+        if (HAS_E) running_min_step<ARGMAX>(acc, vmin, cnt, kk);
       };
       const bool last_k = (kk == nk - 1);
       if (last_k) {
         // last k of the unit: one logarithm per output; the LOD replaces the accumulator
         update_min();
-        const double c_ln = -P.half_n * 0.43429448190325182765;
-        const double c_e = -P.half_n * 0.30102999566398119521;
-        bool special = false;
         double lod[4][BT][2];
-#pragma unroll
-        for (int a = 0; a < 4; ++a)
-#pragma unroll
-          for (int b = 0; b < BT; ++b)
-#pragma unroll
-            for (int cc = 0; cc < 2; ++cc)
-              lod[a][b][cc] = fast_lod(HAS_E ? vmin[a * VM][b][cc] : acc[a][b][cc], logtab, c_ln, c_e, special);
-        if (__any_sync(0xffffffffu, special)) {
-#pragma unroll
-          for (int a = 0; a < 4; ++a)
-#pragma unroll
-            for (int b = 0; b < BT; ++b)
-#pragma unroll
-              for (int cc = 0; cc < 2; ++cc)
-                lod[a][b][cc] = fix_lod(HAS_E ? vmin[a * VM][b][cc] : acc[a][b][cc], lod[a][b][cc]);
-        }
+        lod_finish(HAS_E ? vmin : acc, lod, logtab, P.half_n);
 #pragma unroll
         for (int a = 0; a < 4; ++a)
 #pragma unroll
@@ -392,116 +350,66 @@ __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
     // stores of the unit (LOD in the accumulator registers), outside the turn
     const int kbase = (HAS_E && ARGMAX && P.tile_k0) ? P.tile_k0[tt] : 0;
     const int row0 = mt * MT + wm * 32 + g;
+    const int* cmap = colmap_s + ((ntop - 1) & 1) * TT;  // the tile's part of the column map
+    auto column = [&](int b, int cc) {  // output column of the lane's trait column (b, cc)
+      const int posl = wt * (8 * BT) + b * 8 + 2 * t + cc;
+      return out_column(P, cmap, posl, (int64_t)tt * TT + posl);
+    };
     if (PEAK) {
-      // per-trait peaks: the first maximum of each column over the warp's 32 markers, over a in registers and then
-      // over g across the lanes, compared on integer keys (this runs outside the turn, like the stores it replaces)
-      const int* cmap = colmap_s + ((ntop - 1) & 1) * TT;
+      // per-trait peaks of the warp's 32 markers (this runs outside the turn, like the stores it replaces)
+      peak_store<HAS_E>(acc, cnt, kbase, row0, g, P, 32, mt * 2 + wm, column);
+    } else {
+      const bool full_rows = (mt + 1) * MT <= P.p;  // every marker row of the tile exists
 #pragma unroll
       for (int b = 0; b < BT; ++b)
 #pragma unroll
         for (int cc = 0; cc < 2; ++cc) {
-          double lod = acc[0][b][cc];
-          int row = row0, gi = 0;
+          const OutColumn oc = out_column_ptrs(P, column(b, cc), row0, COLMAX, HAS_E);
+          if (full_rows) {
+            if (oc.L) {
 #pragma unroll
-          for (int a = 0; a < 4; ++a) {
-            const int o = (a * BT + b) * 2 + cc;
-            const int ga = HAS_E ? kbase + (int)((cnt[(o >> 2) * VM] >> ((o & 3) * 8)) & 0xFFu) : 0;
-            if (a == 0)
-              gi = ga;
-            else
-              peak_take(lod, row, gi, acc[a][b][cc], row0 + a * 8, ga, P.p);
-          }
-          peak_over_lanes(lod, row, gi, P.p, 4);
-          const int posl = wt * (8 * BT) + b * 8 + 2 * t + cc;
-          const int64_t pos = (int64_t)tt * TT + posl;
-          const int64_t col = P.col_map ? (int64_t)cmap[posl] : (pos < P.m ? pos : -1);
-          if (g == 0 && col >= 0) P.peaks[col * (P.p_pad / 32) + mt * 2 + wm] = PeakRec{lod, row, gi};
-        }
-      if (++mt == n_mt) {
-        mt = 0;
-        ++tt;
-      }
-      TCK(4)
-      continue;
-    }
-    const bool full_rows = (mt + 1) * MT <= P.p;  // every marker row of the tile exists
-    const int* cmap = colmap_s + ((ntop - 1) & 1) * TT;
+              for (int a = 0; a < 4; ++a) st_stream(oc.L + a * 8, acc[a][b][cc]);
+            }
+            if (oc.H2) {
 #pragma unroll
-    for (int b = 0; b < BT; ++b)
+              for (int a = 0; a < 4; ++a)
+                st_stream(oc.H2 + a * 8, grid_s[kbase + counter_byte(cnt, (a * BT + b) * 2 + cc)]);
+            }
+            if (oc.H2idx) {
 #pragma unroll
-      for (int cc = 0; cc < 2; ++cc) {
-        const int posl = wt * (8 * BT) + b * 8 + 2 * t + cc;
-        const int64_t pos = (int64_t)tt * TT + posl;
-        const int64_t col = P.col_map ? (int64_t)cmap[posl] : (pos < P.m ? pos : -1);
-        // output column pointers (column 0 may be split off, see ScanParams::L0)
-        double* Lc = nullptr;
-        double* Hc = nullptr;
-        double* Mc = nullptr;
-        uint8_t* Ic = nullptr;
-        if (col >= 0) {
-          if (P.L0) {
-            if (col == 0) {
-              Lc = P.L0 + row0;
-            } else {
-              if (P.L) Lc = P.L + (col - 1) * P.ldL + row0;
-              if (COLMAX) Mc = P.colmax + (col - 1);
+              for (int a = 0; a < 4; ++a)
+                oc.H2idx[a * 8] = (uint8_t)(kbase + counter_byte(cnt, (a * BT + b) * 2 + cc));
             }
           } else {
-            if (P.L) Lc = P.L + col * P.ldL + row0;
-            if (COLMAX) Mc = P.colmax + col;
-          }
-          if (HAS_E && P.H2) Hc = P.H2 + col * P.ldL + row0;
-          if (HAS_E && P.H2idx) Ic = P.H2idx + col * (int64_t)P.p + row0;
-        }
-        if (full_rows) {
-          if (Lc) {
-#pragma unroll
-            for (int a = 0; a < 4; ++a) st_stream(Lc + a * 8, acc[a][b][cc]);
-          }
-          if (HAS_E && Hc) {
 #pragma unroll
             for (int a = 0; a < 4; ++a) {
-              const int o = (a * BT + b) * 2 + cc;
-              const int cv = (int)((cnt[(o >> 2) * VM] >> ((o & 3) * 8)) & 0xFFu);
-              st_stream(Hc + a * 8, grid_s[kbase + cv]);
-            }
-          }
-          if (HAS_E && Ic) {
-#pragma unroll
-            for (int a = 0; a < 4; ++a) {
-              const int o = (a * BT + b) * 2 + cc;
-              Ic[a * 8] = (uint8_t)(kbase + (int)((cnt[(o >> 2) * VM] >> ((o & 3) * 8)) & 0xFFu));
-            }
-          }
-        } else {
-#pragma unroll
-          for (int a = 0; a < 4; ++a) {
-            if (row0 + a * 8 < P.p) {
-              if (Lc) st_stream(Lc + a * 8, acc[a][b][cc]);
-              if (HAS_E && (Hc || Ic)) {
-                const int o = (a * BT + b) * 2 + cc;
-                const int cv = (int)((cnt[(o >> 2) * VM] >> ((o & 3) * 8)) & 0xFFu);
-                if (Hc) st_stream(Hc + a * 8, grid_s[kbase + cv]);
-                if (Ic) Ic[a * 8] = (uint8_t)(kbase + cv);
+              if (row0 + a * 8 < P.p) {
+                if (oc.L) st_stream(oc.L + a * 8, acc[a][b][cc]);
+                if (oc.H2 || oc.H2idx) {
+                  const int cv = counter_byte(cnt, (a * BT + b) * 2 + cc);
+                  if (oc.H2) st_stream(oc.H2 + a * 8, grid_s[kbase + cv]);
+                  if (oc.H2idx) oc.H2idx[a * 8] = (uint8_t)(kbase + cv);
+                }
+              } else {
+                acc[a][b][cc] = 0.0;  // padded marker rows stay out of the column maximum
               }
-            } else {
-              acc[a][b][cc] = 0.0;  // padded marker rows stay out of the column maximum
             }
           }
+          if (COLMAX) {
+            // maximum on the bit patterns (LODs are >= 0, so integer order = numeric order; a NaN is the largest
+            // and propagates like Julia's maximum): integer pipe only — this runs outside the group's turn, where
+            // FP64 instructions would sit behind the other group's DMMAs
+            long long cm = max(max(__double_as_longlong(acc[0][b][cc]), __double_as_longlong(acc[1][b][cc])),
+                               max(__double_as_longlong(acc[2][b][cc]), __double_as_longlong(acc[3][b][cc])));
+            cm = max(cm, 0LL);  // -0.0 and anything negative count as 0
+            cm = max(cm, __shfl_xor_sync(0xffffffffu, cm, 4));
+            cm = max(cm, __shfl_xor_sync(0xffffffffu, cm, 8));
+            cm = max(cm, __shfl_xor_sync(0xffffffffu, cm, 16));
+            if (g == 0 && oc.colmax)
+              atomicMax(reinterpret_cast<unsigned long long*>(oc.colmax), (unsigned long long)cm);
+          }
         }
-        if (COLMAX) {
-          // maximum on the bit patterns (LODs are >= 0, so integer order = numeric order; a NaN is the largest
-          // and propagates like Julia's maximum): integer pipe only — this runs outside the group's turn, where
-          // FP64 instructions would sit behind the other group's DMMAs
-          long long cm = max(max(__double_as_longlong(acc[0][b][cc]), __double_as_longlong(acc[1][b][cc])),
-                             max(__double_as_longlong(acc[2][b][cc]), __double_as_longlong(acc[3][b][cc])));
-          cm = max(cm, 0LL);  // -0.0 and anything negative count as 0
-          cm = max(cm, __shfl_xor_sync(0xffffffffu, cm, 4));
-          cm = max(cm, __shfl_xor_sync(0xffffffffu, cm, 8));
-          cm = max(cm, __shfl_xor_sync(0xffffffffu, cm, 16));
-          if (g == 0 && Mc) atomicMax(reinterpret_cast<unsigned long long*>(Mc), (unsigned long long)cm);
-        }
-      }
+    }
     if (++mt == n_mt) {
       mt = 0;
       ++tt;
@@ -514,43 +422,32 @@ __global__ void __launch_bounds__(NTHREADS, 1) scan_kernel(const ScanParams P) {
 #endif
 }
 
-template <int NQ, bool ARGMAX, bool HAS_E, bool COLMAX, bool PEAK = false>
-void launch_one(const ScanParams& P, int sm_count, cudaStream_t stream) {
-  const SmemPlan plan = plan_smem(NQ);
-  cudaFuncSetAttribute(scan_kernel<NQ, ARGMAX, HAS_E, COLMAX, PEAK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       SMEM_LIMIT);
-  scan_kernel<NQ, ARGMAX, HAS_E, COLMAX, PEAK><<<sm_count, NTHREADS, plan.bytes, stream>>>(P);
-}
-
 template <int NQ>
 void launch_nq(const ScanParams& P, int sm_count, cudaStream_t stream) {
+  void (*kernel)(ScanParams);
   if (P.peaks) {
     if (!P.e)
-      launch_one<NQ, false, false, false, true>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, false, false, false, true>;
     else if (P.argmax_mode)
-      launch_one<NQ, true, true, false, true>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, true, true, false, true>;
     else
-      launch_one<NQ, false, true, false, true>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, false, true, false, true>;
   } else if (P.e) {
     if (P.argmax_mode)
-      launch_one<NQ, true, true, false>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, true, true, false, false>;
     else
-      launch_one<NQ, false, true, false>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, false, true, false, false>;
   } else {
     // one-element k-lists (null-grid bins, permutations): the h2 panel is not produced
     if (P.colmax)
-      launch_one<NQ, false, false, true>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, false, false, true, false>;
     else
-      launch_one<NQ, false, false, false>(P, sm_count, stream);
+      kernel = scan_kernel<NQ, false, false, false, false>;
   }
+  launch_scan_kernel(kernel, NTHREADS, plan_smem(NQ).bytes, P, sm_count, stream);
 }
 
 }  // namespace
-
-int scan_max_nq(int nk) {
-  (void)nk;
-  return 5;
-}
 
 #ifdef BLMM_SCAN_TIMING
 extern "C" __attribute__((visibility("default"))) int blmm_debug_scan_timing(long long* out, int nblocks) {
@@ -564,8 +461,7 @@ extern "C" __attribute__((visibility("default"))) int blmm_debug_scan_trace(long
 int launch_scan(const ScanParams& P, int sm_count, cudaStream_t stream) {
   // combinations the kernel variants do not cover
   if ((!P.e && (P.nk != 1 || !P.et_folded)) || (P.e && P.colmax)) return 0;
-  // peaks replace every per-marker output
-  if (P.peaks && (P.colmax || P.L || P.L0 || P.H2 || P.H2idx)) return 0;
+  if (peaks_with_panels(P)) return 0;
   // the kernel indexes its (unit, k) iterations with 32-bit integers
   if ((int64_t)P.n_tiles_t * (P.p_pad / MT) * (int64_t)(P.nk > 0 ? P.nk : 1) >= 2147483647LL) return 0;
   switch (P.nq) {

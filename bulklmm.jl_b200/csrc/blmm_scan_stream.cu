@@ -23,20 +23,24 @@
 #include <float.h>
 #include <math.h>
 
-#include "blmm_kernels.cuh"
+#include "blmm_scan_epilogue.cuh"
 
 namespace blmm {
 
 namespace {
 
-constexpr int SMEM_LIMIT = 227 * 1024;
 constexpr int GRID_MAX = 256;
 constexpr int ST_TG = 8;                  // warps along the trait dimension
 constexpr int ST_WARPS = 2 * ST_TG;       // x 2 along the marker dimension
-constexpr int BAND_DEFAULT = 8;           // trait tiles per rasterisation band (StreamParams::band overrides)
+constexpr int BAND_DEFAULT = 8;           // trait tiles per rasterisation band (ScanParams::band overrides)
 constexpr size_t ST_FIXED_SMEM = (size_t)LTAB * 16 + GRID_MAX * 8 + 128;
 
 enum { MODE_EXACT = 0, MODE_GRID = 1 };
+
+// The GRID instance scans the operands packed for scan_kernel: its tiles must be SCAN_TT traits by SCAN_MT markers.
+constexpr int GRID_NB = 2, GRID_MA = 4;
+static_assert(ST_TG * 8 * GRID_NB == SCAN_TT, "the GRID instance packs traits like scan_kernel");
+static_assert(2 * 8 * GRID_MA == SCAN_MT, "the GRID instance packs markers like scan_kernel");
 
 struct StreamPlan {
   int nstage;
@@ -47,7 +51,7 @@ struct StreamPlan {
 __host__ __device__ inline StreamPlan stream_plan(int NB, int MA) {
   StreamPlan s;
   s.stage_doubles = (size_t)(2 * 8 * MA + ST_TG * 8 * NB) * KC;
-  int ns = (int)((SMEM_LIMIT - ST_FIXED_SMEM) / (s.stage_doubles * 8));
+  int ns = (int)((SCAN_SMEM_LIMIT - ST_FIXED_SMEM) / (s.stage_doubles * 8));
   s.nstage = ns > 4 ? 4 : ns;
   s.bytes = (size_t)s.nstage * s.stage_doubles * 8 + ST_FIXED_SMEM;
   return s;
@@ -55,7 +59,7 @@ __host__ __device__ inline StreamPlan stream_plan(int NB, int MA) {
 
 // PEAK: store nothing per marker; every warp reduces its 8 * MA markers of each column to one PeakRec instead.
 template <int NB, int MA, int MODE, bool ARGMAX, bool PEAK>
-__global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const StreamParams P) {
+__global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const ScanParams P) {
   constexpr int MT = 2 * 8 * MA;        // markers per CTA tile
   constexpr int TCOLS = ST_TG * 8 * NB;  // operand columns per CTA tile
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -91,7 +95,7 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
   if (MODE == MODE_GRID && P.grid && tid < P.ngrid) grid_s[tid] = P.grid[tid];
   __syncthreads();
 
-  const int n_tt = P.n_tiles_dev ? *P.n_tiles_dev : P.n_tt;
+  const int n_tt = P.n_tiles_dev ? *P.n_tiles_dev : P.n_tiles_t;
   const int n_mt = P.p_pad / MT;
   const int nq = P.nq;
   const int nk = (MODE == MODE_GRID) ? P.nk : 1;
@@ -129,7 +133,7 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
     // partition at n = 1000 (ncu: 210 GB of DRAM reads for ~35 GB of operands).
     bulk_g2s_hint(st, P.Mop + ((((size_t)(k0 + k) * nq + q) * P.p_pad) + (size_t)mt * MT) * KC, marker_bytes, &full[s],
                   l2_evict_first_policy());
-    bulk_g2s_hint(st + MT * KC, P.Xop + (((size_t)q * P.xcol_pad) + (size_t)tt * TCOLS) * KC, trait_bytes, &full[s],
+    bulk_g2s_hint(st + MT * KC, P.Top + (((size_t)q * P.tcol_pad) + (size_t)tt * TCOLS) * KC, trait_bytes, &full[s],
                   l2_evict_last_policy());
   };
 
@@ -169,7 +173,6 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
 #pragma unroll
       for (int i = 0; i < (MA * NB * 2 + 3) / 4; ++i) cnt[i] = 0u;
     }
-    double lod[MA][(MODE == MODE_EXACT) ? 1 : NB][2];
 
     for (int kk = 0; kk < nk; ++kk) {
       double ek[NB][2], etk[NB][2];
@@ -240,7 +243,6 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
       }
 
       if (MODE == MODE_GRID) {
-        const bool first = (kk == 0);
 #pragma unroll
         for (int a = 0; a < MA; ++a)
 #pragma unroll
@@ -248,18 +250,9 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
 #pragma unroll
             for (int cc = 0; cc < 2; ++cc) {
               const double d = acc[a][b][cc];
-              const double v = fma(-(d * d), etk[b][cc], ek[b][cc]);
-              const bool better = __double_as_longlong(v) < __double_as_longlong(vmin[a][b][cc]);
-              const bool upd = first || better;
-              vmin[a][b][cc] = upd ? v : vmin[a][b][cc];
-              const int o = (a * NB + b) * 2 + cc;
-              const int sh = (o & 3) * 8;
-              if (ARGMAX) {
-                if (upd) cnt[o >> 2] = (cnt[o >> 2] & ~(0xFFu << sh)) | ((uint32_t)kk << sh);
-              } else {
-                if (better && !first) cnt[o >> 2] += (1u << sh);
-              }
+              acc[a][b][cc] = fma(-(d * d), etk[b][cc], ek[b][cc]);
             }
+        running_min_step<ARGMAX>(acc, vmin, cnt, kk);
       } else {
         // EXACT: combine the c+2 accumulators of each (marker, trait) pair
 #pragma unroll
@@ -279,26 +272,17 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
 
     // final epilogue: one logarithm per output, streaming stores
     constexpr int NBO = (MODE == MODE_EXACT) ? 1 : NB;
-    bool special = false;
-    const double c_ln = -P.half_n * 0.43429448190325182765;
-    const double c_e = -P.half_n * 0.30102999566398119521;
-#pragma unroll
-    for (int a = 0; a < MA; ++a)
-#pragma unroll
-      for (int b = 0; b < NBO; ++b)
-#pragma unroll
-        for (int cc = 0; cc < 2; ++cc) lod[a][b][cc] = fast_lod(vmin[a][b][cc], logtab, c_ln, c_e, special);
-    if (__any_sync(0xffffffffu, special)) {
-#pragma unroll
-      for (int a = 0; a < MA; ++a)
-#pragma unroll
-        for (int b = 0; b < NBO; ++b)
-#pragma unroll
-          for (int cc = 0; cc < 2; ++cc) lod[a][b][cc] = fix_lod(vmin[a][b][cc], lod[a][b][cc]);
-    }
+    double lod[MA][NBO][2];
+    lod_finish(vmin, lod, logtab, P.half_n);
     const int k0 = (MODE == MODE_GRID && P.tile_k0) ? P.tile_k0[tt] : 0;
     const int kbase = ARGMAX ? k0 : 0;
     const int i_base = mt * MT + wm * 8 * MA + g;
+    auto column = [&](int b, int cc) {  // output column of the lane's trait column (b, cc)
+      const int64_t pos = (int64_t)tt * (ST_TG * 8 * NBO) + wt * (8 * NBO) + b * 8 + 2 * t + cc;
+      return out_column(P, P.col_map, pos, pos);
+    };
+    // (peak_store and out_column_ptrs of blmm_scan_epilogue.cuh are spelled out here: as calls they change the register
+    // allocation of some instances of this kernel)
     if (PEAK) {
       // per-trait peaks: the first maximum of each column over the warp's 8 * MA markers (over a in registers, then
       // over g across the lanes); units write disjoint records, so the dynamic scheduler needs no ordering
@@ -310,20 +294,15 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
           int row = i_base, gi = 0;
 #pragma unroll
           for (int a = 0; a < MA; ++a) {
-            int ga = 0;
-            if (MODE == MODE_GRID) {
-              const int o = (a * NB + b) * 2 + cc;
-              ga = kbase + (int)((cnt[o >> 2] >> ((o & 3) * 8)) & 0xFFu);
-            }
+            const int ga = (MODE == MODE_GRID) ? kbase + counter_byte(cnt, (a * NB + b) * 2 + cc) : 0;
             if (a == 0)
               gi = ga;
             else
               peak_take(pl, row, gi, lod[a][b][cc], i_base + a * 8, ga, P.p);
           }
           peak_over_lanes(pl, row, gi, P.p, 4);
-          const int64_t pos = (int64_t)tt * (ST_TG * 8 * NBO) + wt * (8 * NBO) + b * 8 + 2 * t + cc;
-          const int64_t col = P.col_map ? (int64_t)P.col_map[pos] : (pos < P.m ? pos : -1);
-          if (g == 0 && col >= 0) P.peaks[col * (P.p_pad / (8 * MA)) + mt * 2 + wm] = PeakRec{pl, row, gi};
+          const int64_t col = column(b, cc);
+          if (g == 0 && col >= 0) P.peaks[col * peak_blocks(P.p_pad, 8 * MA) + mt * 2 + wm] = PeakRec{pl, row, gi};
         }
       continue;
     }
@@ -331,8 +310,7 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
     for (int b = 0; b < NBO; ++b)
 #pragma unroll
       for (int cc = 0; cc < 2; ++cc) {
-        const int64_t pos = (int64_t)tt * (ST_TG * 8 * NBO) + wt * (8 * NBO) + b * 8 + 2 * t + cc;
-        const int64_t col = P.col_map ? (int64_t)P.col_map[pos] : (pos < P.m ? pos : -1);
+        const int64_t col = column(b, cc);
         double* Lc = nullptr;
         double* Hc = nullptr;
         double* Mc = nullptr;
@@ -357,11 +335,7 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Str
           const double l = lod[a][b][cc];
           if (i < P.p) {
             if (Lc) st_stream(Lc + i, l);
-            if (MODE == MODE_GRID && Hc) {
-              const int o = (a * NB + b) * 2 + cc;
-              const int cv = (int)((cnt[o >> 2] >> ((o & 3) * 8)) & 0xFFu);
-              st_stream(Hc + i, grid_s[kbase + cv]);
-            }
+            if (Hc) st_stream(Hc + i, grid_s[kbase + counter_byte(cnt, (a * NB + b) * 2 + cc)]);
             cmax = fmax(cmax, l);
           }
         }
@@ -501,32 +475,29 @@ __global__ void __launch_bounds__(256) exact_columns_kernel(const double* __rest
 }
 
 template <int NB, int MA, int MODE, bool PEAK>
-void launch_stream_peak(const StreamParams& P, int sm_count, cudaStream_t stream) {
-  const StreamPlan plan = stream_plan(NB, MA);
-  if (MODE == MODE_GRID && P.argmax_mode) {
-    cudaFuncSetAttribute(scan_stream_kernel<NB, MA, MODE, true, PEAK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         SMEM_LIMIT);
-    scan_stream_kernel<NB, MA, MODE, true, PEAK><<<sm_count, 32 * ST_WARPS, plan.bytes, stream>>>(P);
-  } else {
-    cudaFuncSetAttribute(scan_stream_kernel<NB, MA, MODE, false, PEAK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         SMEM_LIMIT);
-    scan_stream_kernel<NB, MA, MODE, false, PEAK><<<sm_count, 32 * ST_WARPS, plan.bytes, stream>>>(P);
+void launch_stream_peak(const ScanParams& P, int sm_count, cudaStream_t stream) {
+  void (*kernel)(ScanParams) = scan_stream_kernel<NB, MA, MODE, false, PEAK>;
+  if constexpr (MODE == MODE_GRID) {  // (the EXACT mode has no grid)
+    if (P.argmax_mode) kernel = scan_stream_kernel<NB, MA, MODE, true, PEAK>;
   }
+  launch_scan_kernel(kernel, 32 * ST_WARPS, stream_plan(NB, MA).bytes, P, sm_count, stream);
 }
 
 template <int NB, int MA, int MODE>
-void launch_stream_one(const StreamParams& P, int sm_count, cudaStream_t stream) {
+void launch_stream_one(const ScanParams& P, int sm_count, cudaStream_t stream) {
   if (P.peaks)
     launch_stream_peak<NB, MA, MODE, true>(P, sm_count, stream);
   else
     launch_stream_peak<NB, MA, MODE, false>(P, sm_count, stream);
 }
 
+// What the K-streamed kernel does not implement: et folded into the trait operand, the grid-index panel, and peaks
+// beside per-marker outputs.
+bool stream_unsupported(const ScanParams& P) { return P.et_folded || P.H2idx || peaks_with_panels(P); }
+
 }  // namespace
 
 int stream_exact_marker_tile(int c) { return (c + 2 <= 5) ? 64 : 32; }
-int stream_grid_marker_tile() { return 64; }
-int stream_grid_trait_tile() { return ST_TG * 8 * 2; }
 
 int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* C0, int64_t m,
                          int64_t slots, int n, int n_pad, int c, double* Xop, int64_t xcol_pad, double* dyinv,
@@ -542,7 +513,8 @@ int launch_exact_columns(const double* Yr, const double* h2, const double* lambd
   return 1;
 }
 
-int launch_scan_exact(const StreamParams& P, int c, int sm_count, cudaStream_t stream) {
+int launch_scan_exact(const ScanParams& P, int c, int sm_count, cudaStream_t stream) {
+  if (stream_unsupported(P)) return 0;
   switch (c + 2) {
     case 3: launch_stream_one<3, 4, MODE_EXACT>(P, sm_count, stream); break;
     case 4: launch_stream_one<4, 4, MODE_EXACT>(P, sm_count, stream); break;
@@ -557,8 +529,9 @@ int launch_scan_exact(const StreamParams& P, int c, int sm_count, cudaStream_t s
   return 1;
 }
 
-int launch_scan_stream_grid(const StreamParams& P, int sm_count, cudaStream_t stream) {
-  launch_stream_one<2, 4, MODE_GRID>(P, sm_count, stream);
+int launch_scan_stream_grid(const ScanParams& P, int sm_count, cudaStream_t stream) {
+  if (stream_unsupported(P)) return 0;
+  launch_stream_one<GRID_NB, GRID_MA, MODE_GRID>(P, sm_count, stream);
   return 1;
 }
 

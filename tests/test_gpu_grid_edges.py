@@ -40,8 +40,8 @@ def paths(n, c, nk):
     included) and nk grid points.  Mirrors bulklmm.jl_b200/csrc/blmm_prep.cu launch_trait_stats (the
     `table_smem <= 96 * 1024` test; 'a' = table kernel with one batch, which also writes the alt-grid scalars and the
     packed trait operand, 'b' = table kernel with several batches, 'c' = generic trait_stats_kernel),
-    launch_marker_operand (`tsmem <= 56 * 1024`) and, in blmm_api.cu run_scan, `P.nq <= scan_max_nq(P.nk)` with
-    scan_max_nq = 5 in blmm_scan.cu ('resident' scan_kernel, else the K-streamed scan_stream_kernel)."""
+    launch_marker_operand (`tsmem <= 56 * 1024`) and, in blmm_api.cu run_scan, `P.nq <= SCAN_MAX_NQ` with
+    SCAN_MAX_NQ = 5 in blmm_kernels.cuh ('resident' scan_kernel, else the K-streamed scan_stream_kernel)."""
     n_pad = -(-n // 20) * 20  # KC = 20
     kb = 32 // (1 + c)
     nbatch = -(-nk // kb)
@@ -98,13 +98,13 @@ def test_case_table_covers_every_dispatch_path():
     # the mirrored thresholds are still the ones in the source: a moved threshold fails here, naming paths()
     with open(os.path.join(ROOT, "bulklmm.jl_b200", "csrc", "blmm_prep.cu")) as f:
         prep = f.read()
-    with open(os.path.join(ROOT, "bulklmm.jl_b200", "csrc", "blmm_scan.cu")) as f:
-        scan_src = f.read()
+    with open(os.path.join(ROOT, "bulklmm.jl_b200", "csrc", "blmm_kernels.cuh")) as f:
+        kernels_h = f.read()
     for needle in ("constexpr int WARPS_PER_BLOCK = 8;", "const int KB = 32 / (1 + c);",
                    "if (table_smem <= 96 * 1024)", "if (tsmem <= 56 * 1024)",
                    "(size_t)WARPS_PER_BLOCK * 2 * n_pad + (size_t)n_pad"):
         assert needle in prep, f"blmm_prep.cu no longer has `{needle}`: update paths() and the cases"
-    assert "(void)nk;\n  return 5;" in scan_src, "scan_max_nq changed: update paths()"
+    assert "constexpr int SCAN_MAX_NQ = 5;" in kernels_h, "SCAN_MAX_NQ changed: update paths()"
 
     required = {}
     for c in range(1, 9):
