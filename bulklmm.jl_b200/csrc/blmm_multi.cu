@@ -48,12 +48,10 @@ struct Worker {
   int rc = 0;
 };
 
-// grow-only device buffers of one GPU for device-resident multi-GPU calls
-enum MBuf { MB_G, MB_C, MB_U, MB_LAM, MB_W, MB_Y, MB_L, MB_H, MB_P, MB_PERM, MB_LOD, MB_MAX, MB_SCAL, MB_COUNT };
-
+// grow-only device buffers of one GPU for device-resident multi-GPU calls, one per array of a DeviceCall
 struct DevBufs {
-  void* p[MB_COUNT] = {};
-  size_t cap[MB_COUNT] = {};
+  std::vector<void*> p;
+  std::vector<size_t> cap;
 };
 
 }  // namespace
@@ -139,32 +137,75 @@ int finish(blmm_ctx* parent, int rc, int fail_rank) {
   return rc;
 }
 
-// columns [j0, j1) of GPU r when `total` columns are cut at multiples of `align`
-void shard_cols(int64_t total, int ndev, int r, int64_t align, int64_t* j0, int64_t* j1) {
-  const int64_t tiles = (total + align - 1) / align;
-  *j0 = std::min<int64_t>(total, tiles * r / ndev * align);
-  *j1 = std::min<int64_t>(total, tiles * (r + 1) / ndev * align);
+// run_all, then the parent's status and message are those of the lowest failing GPU
+int run_ranks(blmm_ctx* parent, const std::function<int(int)>& f) {
+  int fr = -1;
+  const int rc = run_all(parent->multi, f, &fr);
+  return finish(parent, rc, fr);
 }
 
-// permutation columns [s0[r], s1[r]) of every GPU: each GPU also scans the un-permuted trait as its column 0, so
-// blocks of 128 - 1 permutations fill whole 128-column tiles; the first GPUs get the tiles when there are fewer
-// tiles than GPUs (the primary always has work: it reports the un-permuted LODs)
-void shard_perms(int64_t nperms, int ndev, std::vector<int64_t>& s0, std::vector<int64_t>& s1) {
+// f(), with a Fail thrown inside reported as c's message and the returned status
+template <typename F>
+int catch_fail(blmm_ctx* c, F&& f) {
+  try {
+    return f();
+  } catch (const Fail& e) {
+    c->err = e.msg;
+    return e.code;
+  }
+}
+
+// the contiguous column block [b[r], e[r]) of every GPU r
+struct Shards {
+  std::vector<int64_t> b, e;
+  explicit Shards(int ndev) : b(ndev), e(ndev) {}
+  int64_t count(int r) const { return e[r] - b[r]; }
+};
+
+// `total` columns cut at multiples of `align`
+Shards shard_cols(int64_t total, int ndev, int64_t align) {
+  Shards s(ndev);
+  const int64_t tiles = (total + align - 1) / align;
+  for (int r = 0; r < ndev; ++r) {
+    s.b[r] = std::min<int64_t>(total, tiles * r / ndev * align);
+    s.e[r] = std::min<int64_t>(total, tiles * (r + 1) / ndev * align);
+  }
+  return s;
+}
+
+// permutation columns: each GPU also scans the un-permuted trait as its column 0, so blocks of 128 - 1 permutations
+// fill whole 128-column tiles; the first GPUs get the tiles when there are fewer tiles than GPUs (the primary always
+// has work: it reports the un-permuted LODs)
+Shards shard_perms(int64_t nperms, int ndev) {
+  Shards s(ndev);
   const int64_t tiles = (nperms + ndev + SCAN_TT - 1) / SCAN_TT;
   int64_t pos = 0;
   for (int r = 0; r < ndev; ++r) {
     const int64_t tr = tiles * (ndev - r) / ndev - tiles * (ndev - r - 1) / ndev;
     const int64_t cnt = std::min<int64_t>(tr > 0 ? tr * SCAN_TT - 1 : 0, nperms - pos);
-    s0[r] = pos;
-    s1[r] = pos + cnt;
+    s.b[r] = pos;
+    s.e[r] = pos + cnt;
     pos += cnt;
   }
+  return s;
 }
 
-template <typename T>
-T* mbuf(MultiState* M, int r, MBuf b, size_t count) {
+// the problem restricted to GPU r's block of traits
+blmm_problem trait_block(const blmm_problem* pr, const Shards& s, int r) {
+  blmm_problem sp = *pr;
+  sp.Y = pr->Y + s.b[r] * pr->n;
+  sp.m = s.count(r);
+  return sp;
+}
+
+// buffer b of GPU r, at least `bytes` long
+void* mbuf(MultiState* M, int r, size_t b, size_t bytes) {
   DevBufs& B = M->bufs[r];
-  const size_t bytes = std::max<size_t>(count * sizeof(T), 256);
+  if (B.p.size() <= b) {
+    B.p.resize(b + 1, nullptr);
+    B.cap.resize(b + 1, 0);
+  }
+  bytes = std::max<size_t>(bytes, 256);
   if (B.cap[b] < bytes) {
     if (B.p[b]) CUDA_TRY(cudaFree(B.p[b]));
     B.p[b] = nullptr;
@@ -172,7 +213,7 @@ T* mbuf(MultiState* M, int r, MBuf b, size_t count) {
     CUDA_TRY(cudaMalloc(&B.p[b], bytes));
     B.cap[b] = bytes;
   }
-  return reinterpret_cast<T*>(B.p[b]);
+  return B.p[b];
 }
 
 #define NCCL_TRY(expr)                                                                                         \
@@ -210,12 +251,148 @@ void ensure_nccl(MultiState* M) {
   M->comms = comms;
 }
 
-// One replicated input: broadcast from the primary's pointer into GPU r's buffer (in place on the primary).
-struct Bcast {
-  const void* root_ptr;
-  MBuf buf;
-  size_t bytes;
+// One array of a device-resident call: the caller's pointer on the primary GPU (NULL: the call has no such array)
+// and its element count, on every GPU (replicated inputs) or per column (scattered input, gathered outputs).
+struct Part {
+  const void* root;
+  size_t count;
 };
+
+// What a device-resident call moves between the GPUs.  The primary works on the caller's arrays; every other GPU
+// works on grow-only buffers of its own, one per array, indexed by the array's position in this description.
+struct DeviceCall {
+  std::vector<Part> replicated;  // doubles, broadcast from the primary
+  Part scattered;                // column-sharded input: every GPU receives its own columns from the primary
+  ncclDataType_t scattered_type;
+  size_t scattered_size;         // bytes per element
+  std::vector<Part> gathered;    // doubles: every GPU's column slab lands in the primary's array (count 0: no array)
+  std::vector<size_t> scratch;   // doubles of results that stay on the GPUs other than the primary
+};
+
+// one GPU's pointers to the arrays of a DeviceCall, in the order of the description (NULL where there is no array)
+struct RankPtrs {
+  std::vector<const void*> in;
+  const void* scattered = nullptr;
+  std::vector<double*> out;
+  std::vector<double*> scratch;
+};
+
+// the inputs of the model every GPU holds a copy of, in the order local_problem() reads them
+std::vector<Part> model_inputs(const blmm_problem* pr) {
+  const size_t n = (size_t)pr->n;
+  return {{pr->G, n * pr->p}, {pr->Covar, n * pr->c}, {pr->U, n * n}, {pr->lambda, n}, {pr->obs_weights, n}};
+}
+
+// the problem with GPU r's copies of the model inputs
+blmm_problem local_problem(const blmm_problem* pr, const RankPtrs& x) {
+  blmm_problem sp = *pr;
+  sp.G = (const double*)x.in[0];
+  sp.Covar = (const double*)x.in[1];
+  sp.U = (const double*)x.in[2];
+  sp.lambda = (const double*)x.in[3];
+  sp.obs_weights = (const double*)x.in[4];
+  return sp;
+}
+
+// multi-GPU device-resident calls: pointers on the primary GPU; NCCL moves the shards
+int device_checks(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o) {
+  if ((o->ld_out ? o->ld_out : pr->p) != pr->p)
+    return fail(parent, BLMM_E_INVALID, "multi-GPU device-resident calls need ld_out == p (contiguous slabs)");
+  if (pr->c < 1 || pr->c > MAXC || !pr->Y || !pr->G || !pr->Covar || !pr->U || !pr->lambda)
+    return fail(parent, BLMM_E_INVALID, "bad problem (NULL input or covariate count)");
+  return BLMM_OK;
+}
+
+// Runs a device-resident call: broadcast the replicated inputs and scatter the column blocks `s` of the sharded one,
+// call(r, pointers) on every GPU, gather the result slabs into the primary's arrays.
+int run_device(blmm_ctx* parent, const Shards& s, const DeviceCall& d,
+               const std::function<int(int, const RankPtrs&)>& call) {
+  MultiState* M = parent->multi;
+  const int nd = M->ndev;
+  int rc = catch_fail(parent, [&] {
+    ensure_nccl(M);
+    return BLMM_OK;
+  });
+  if (rc != BLMM_OK) return rc;
+  const auto gathers = [](const Part& g) { return g.root && g.count; };
+  // buffers on every GPU (a failure here must not leave the others waiting inside NCCL)
+  std::vector<RankPtrs> ptrs(nd);
+  rc = run_ranks(parent, [&](int r) -> int {
+    RankPtrs& x = ptrs[r];
+    if (r == 0) {
+      for (const Part& a : d.replicated) x.in.push_back(a.root);
+      x.scattered = d.scattered.root;
+      for (const Part& g : d.gathered) x.out.push_back((double*)g.root);
+      return BLMM_OK;
+    }
+    return catch_fail(M->sub[r], [&] {
+      const size_t cols = (size_t)s.count(r);
+      size_t b = 0;  // position in the description
+      const auto next = [&](bool used, size_t bytes) {
+        void* q = used ? mbuf(M, r, b, bytes) : nullptr;
+        ++b;
+        return q;
+      };
+      for (const Part& a : d.replicated) x.in.push_back(next(a.root, a.count * 8));
+      x.scattered = next(true, d.scattered.count * cols * d.scattered_size);
+      for (const Part& g : d.gathered) x.out.push_back((double*)next(gathers(g), g.count * cols * 8));
+      for (size_t count : d.scratch) x.scratch.push_back((double*)next(true, count * 8));
+      return BLMM_OK;
+    });
+  });
+  if (rc != BLMM_OK) return rc;
+
+  return run_ranks(parent, [&](int r) -> int {
+    blmm_ctx* c = M->sub[r];
+    return catch_fail(c, [&] {
+      const RankPtrs& x = ptrs[r];
+      cudaStream_t st = c->stream;
+      NcclApi& N = M->nccl;
+      ncclComm_t comm = M->comms[r];
+      const size_t cols = (size_t)s.count(r);
+      // broadcast / scatter
+      NCCL_TRY(N.GroupStart());
+      for (size_t k = 0; k < d.replicated.size(); ++k) {
+        if (!d.replicated[k].root) continue;
+        void* mine = const_cast<void*>(x.in[k]);
+        NCCL_TRY(N.Broadcast(mine, mine, d.replicated[k].count * 8, ncclChar, 0, comm, st));
+      }
+      const Part& sc = d.scattered;
+      if (r == 0) {
+        for (int q = 1; q < nd; ++q)
+          if (s.count(q) > 0)
+            NCCL_TRY(N.Send((const char*)sc.root + s.b[q] * sc.count * d.scattered_size, s.count(q) * sc.count,
+                            d.scattered_type, q, comm, st));
+      } else if (cols > 0) {
+        NCCL_TRY(N.Recv(const_cast<void*>(x.scattered), cols * sc.count, d.scattered_type, 0, comm, st));
+      }
+      NCCL_TRY(N.GroupEnd());
+      // compute on the local block
+      const int status = call(r, x);
+      // gather the slabs on the primary (always entered, so that no GPU waits for a failed one)
+      if (r == 0) {
+        CUDA_TRY(cudaEventRecord(M->g0, st));
+        NCCL_TRY(N.GroupStart());
+        for (int q = 1; q < nd; ++q) {
+          const size_t mq = (size_t)s.count(q);
+          if (!mq) continue;
+          for (const Part& g : d.gathered)
+            if (gathers(g))
+              NCCL_TRY(N.Recv((double*)g.root + s.b[q] * g.count, mq * g.count, ncclDouble, q, comm, st));
+        }
+        NCCL_TRY(N.GroupEnd());
+        CUDA_TRY(cudaEventRecord(M->g1, st));
+        M->gather_timed = true;
+      } else if (cols > 0) {
+        NCCL_TRY(N.GroupStart());
+        for (size_t k = 0; k < d.gathered.size(); ++k)
+          if (gathers(d.gathered[k])) NCCL_TRY(N.Send(x.out[k], cols * d.gathered[k].count, ncclDouble, 0, comm, st));
+        NCCL_TRY(N.GroupEnd());
+      }
+      return status;
+    });
+  });
+}
 
 }  // namespace
 
@@ -271,8 +448,8 @@ void multi_destroy(blmm_ctx* parent) {
     for (ncclComm_t c : M->comms) M->nccl.CommDestroy(c);
   for (int r = 0; r < (int)M->bufs.size(); ++r) {
     cudaSetDevice(M->devices[r]);
-    for (int b = 0; b < MB_COUNT; ++b)
-      if (M->bufs[r].p[b]) cudaFree(M->bufs[r].p[b]);
+    for (void* b : M->bufs[r].p)
+      if (b) cudaFree(b);
   }
   if (M->g0) cudaEventDestroy(M->g0);
   if (M->g1) cudaEventDestroy(M->g1);
@@ -286,15 +463,14 @@ blmm_ctx* multi_primary(blmm_ctx* parent) { return parent->multi->sub[0]; }
 
 int multi_sync(blmm_ctx* parent) {
   MultiState* M = parent->multi;
-  int fr = -1;
-  const int rc = run_all(M, [&](int r) { return blmm_sync(M->sub[r]); }, &fr);
+  const int rc = run_ranks(parent, [&](int r) { return blmm_sync(M->sub[r]); });
   if (rc == BLMM_OK && M->gather_timed) {
     float ms = -1.f;
     cudaSetDevice(M->devices[0]);
     if (cudaEventElapsedTime(&ms, M->g0, M->g1) == cudaSuccess) parent->gather_ms = (double)ms;
     M->gather_timed = false;
   }
-  return finish(parent, rc, fr);
+  return rc;
 }
 
 int64_t multi_launch_count(const blmm_ctx* parent) {
@@ -328,144 +504,43 @@ int multi_bulkscan(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o,
   if (!pr || !o) return fail(parent, BLMM_E_INVALID, "problem / opts is NULL");
   if (pr->n <= 0 || pr->m < 0 || pr->p <= 0) return fail(parent, BLMM_E_DIM, "Dimension mismatch.");
   if (!L_out) return fail(parent, BLMM_E_INVALID, "L_out is NULL");
-  const int64_t n = pr->n, p = pr->p, m = pr->m;
+  const int64_t n = pr->n, p = pr->p;
   const int64_t ld = o->ld_out ? o->ld_out : p;
   const bool alt = o->method == BLMM_METHOD_ALT_GRID;
-  const bool dev = o->mem_space == BLMM_MEM_DEVICE;
-  const int nd = M->ndev;
-  std::vector<int64_t> j0(nd), j1(nd);
-  for (int r = 0; r < nd; ++r) shard_cols(m, nd, r, SCAN_TT, &j0[r], &j1[r]);
-  int fr = -1;
+  const Shards s = shard_cols(pr->m, M->ndev, SCAN_TT);
 
-  if (!dev) {
+  if (o->mem_space != BLMM_MEM_DEVICE) {
     // the h2 panel's PCIe encoding is decided on the whole panel: what limits a multi-GPU host call is the host's
     // ingest rate (all GPUs feed one memory system), and one-byte indices halve the bytes that cross it
-    const int idx_hint = ((double)p * (double)m >= 1e8) ? 1 : 0;
-    const int rc = run_all(M, [&](int r) -> int {
-      if (j1[r] == j0[r]) return BLMM_OK;
+    const int idx_hint = ((double)p * (double)pr->m >= 1e8) ? 1 : 0;
+    return run_ranks(parent, [&](int r) -> int {
+      if (!s.count(r)) return BLMM_OK;
+      const int64_t j = s.b[r];
       M->sub[r]->idx_hint = idx_hint;
-      blmm_problem sp = *pr;
-      sp.Y = pr->Y + j0[r] * n;
-      sp.m = j1[r] - j0[r];
+      const blmm_problem sp = trait_block(pr, s, r);
       blmm_opts so = *o;
-      if (o->log10p_out) so.log10p_out = o->log10p_out + j0[r] * ld;
-      double* h = h2_out ? (alt ? h2_out + j0[r] * ld : h2_out + j0[r]) : nullptr;
-      return blmm_bulkscan(M->sub[r], &sp, &so, L_out + j0[r] * ld, h);
-    }, &fr);
-    return finish(parent, rc, fr);
+      if (o->log10p_out) so.log10p_out = o->log10p_out + j * ld;
+      double* h = h2_out ? (alt ? h2_out + j * ld : h2_out + j) : nullptr;
+      return blmm_bulkscan(M->sub[r], &sp, &so, L_out + j * ld, h);
+    });
   }
 
-  // device-resident: pointers on the primary GPU; NCCL moves the shards
-  if (ld != p) return fail(parent, BLMM_E_INVALID, "multi-GPU device-resident calls need ld_out == p (contiguous slabs)");
-  if (pr->c < 1 || pr->c > MAXC || !pr->Y || !pr->G || !pr->Covar || !pr->U || !pr->lambda)
-    return fail(parent, BLMM_E_INVALID, "bad problem (NULL input or covariate count)");
+  if (int e = device_checks(parent, pr, o)) return e;
   const bool pv = o->chisq_df > 0;
   if (pv && !o->log10p_out) return fail(parent, BLMM_E_INVALID, "chisq_df > 0 but log10p_out is NULL");
-  try {
-    ensure_nccl(M);
-  } catch (const Fail& f) {
-    return fail(parent, f.code, f.msg);
-  }
-  // phase A: buffers on every GPU (a failure here must not leave the others waiting inside NCCL)
-  int rc = run_all(M, [&](int r) -> int {
-    if (r == 0) return BLMM_OK;
-    try {
-      const size_t mr = (size_t)(j1[r] - j0[r]);
-      mbuf<double>(M, r, MB_G, (size_t)n * p);
-      mbuf<double>(M, r, MB_C, (size_t)n * pr->c);
-      mbuf<double>(M, r, MB_U, (size_t)n * n);
-      mbuf<double>(M, r, MB_LAM, n);
-      if (pr->obs_weights) mbuf<double>(M, r, MB_W, n);
-      mbuf<double>(M, r, MB_Y, (size_t)n * mr);
-      mbuf<double>(M, r, MB_L, (size_t)p * mr);
-      if (h2_out) mbuf<double>(M, r, MB_H, alt ? (size_t)p * mr : mr);
-      if (pv) mbuf<double>(M, r, MB_P, (size_t)p * mr);
-    } catch (const Fail& f) {
-      M->sub[r]->err = f.msg;
-      return f.code;
-    }
-    return BLMM_OK;
-  }, &fr);
-  if (rc != BLMM_OK) return finish(parent, rc, fr);
-
-  const std::vector<Bcast> bc = {{pr->G, MB_G, (size_t)n * p * 8},   {pr->Covar, MB_C, (size_t)n * pr->c * 8},
-                                 {pr->U, MB_U, (size_t)n * n * 8},   {pr->lambda, MB_LAM, (size_t)n * 8},
-                                 {pr->obs_weights, MB_W, (size_t)n * 8}};
-  rc = run_all(M, [&](int r) -> int {
-    blmm_ctx* c = M->sub[r];
-    cudaStream_t st = c->stream;
-    NcclApi& N = M->nccl;
-    ncclComm_t comm = M->comms[r];
-    int status = BLMM_OK;
-    try {
-      DevBufs& B = M->bufs[r];
-      // scatter / broadcast
-      NCCL_TRY(N.GroupStart());
-      for (const Bcast& b : bc) {
-        if (!b.root_ptr) continue;
-        void* mine = r == 0 ? const_cast<void*>(b.root_ptr) : B.p[b.buf];
-        NCCL_TRY(N.Broadcast(mine, mine, b.bytes, ncclChar, 0, comm, st));
-      }
-      if (r == 0) {
-        for (int q = 1; q < nd; ++q)
-          if (j1[q] > j0[q]) NCCL_TRY(N.Send(pr->Y + j0[q] * n, (size_t)(j1[q] - j0[q]) * n, ncclDouble, q, comm, st));
-      } else if (j1[r] > j0[r]) {
-        NCCL_TRY(N.Recv(B.p[MB_Y], (size_t)(j1[r] - j0[r]) * n, ncclDouble, 0, comm, st));
-      }
-      NCCL_TRY(N.GroupEnd());
-      // compute on the local block
-      const int64_t mr = j1[r] - j0[r];
-      double *Lr, *Hr = nullptr, *Pr = nullptr;
-      blmm_problem sp = *pr;
-      blmm_opts so = *o;
-      sp.m = mr;
-      if (r == 0) {
-        sp.Y = pr->Y;  // j0[0] == 0
-        Lr = L_out;
-        Hr = h2_out;
-        Pr = o->log10p_out;
-      } else {
-        sp.Y = (const double*)B.p[MB_Y];
-        sp.G = (const double*)B.p[MB_G];
-        sp.Covar = (const double*)B.p[MB_C];
-        sp.U = (const double*)B.p[MB_U];
-        sp.lambda = (const double*)B.p[MB_LAM];
-        if (pr->obs_weights) sp.obs_weights = (const double*)B.p[MB_W];
-        Lr = (double*)B.p[MB_L];
-        if (h2_out) Hr = (double*)B.p[MB_H];
-        if (pv) Pr = (double*)B.p[MB_P];
-      }
-      so.log10p_out = Pr;
-      so.ld_out = p;
-      if (mr > 0) status = blmm_bulkscan(c, &sp, &so, Lr, Hr);
-      // gather the slabs on the primary (always entered, so that no GPU waits for a failed one)
-      if (r == 0) {
-        CUDA_TRY(cudaEventRecord(M->g0, st));
-        NCCL_TRY(N.GroupStart());
-        for (int q = 1; q < nd; ++q) {
-          const size_t mq = (size_t)(j1[q] - j0[q]);
-          if (!mq) continue;
-          NCCL_TRY(N.Recv(L_out + j0[q] * p, mq * p, ncclDouble, q, comm, st));
-          if (h2_out) NCCL_TRY(N.Recv(alt ? h2_out + j0[q] * p : h2_out + j0[q], alt ? mq * p : mq, ncclDouble, q, comm, st));
-          if (pv) NCCL_TRY(N.Recv(o->log10p_out + j0[q] * p, mq * p, ncclDouble, q, comm, st));
-        }
-        NCCL_TRY(N.GroupEnd());
-        CUDA_TRY(cudaEventRecord(M->g1, st));
-        M->gather_timed = true;
-      } else if (mr > 0) {
-        NCCL_TRY(N.GroupStart());
-        NCCL_TRY(N.Send(Lr, (size_t)mr * p, ncclDouble, 0, comm, st));
-        if (h2_out) NCCL_TRY(N.Send(Hr, alt ? (size_t)mr * p : (size_t)mr, ncclDouble, 0, comm, st));
-        if (pv) NCCL_TRY(N.Send(Pr, (size_t)mr * p, ncclDouble, 0, comm, st));
-        NCCL_TRY(N.GroupEnd());
-      }
-    } catch (const Fail& f) {
-      c->err = f.msg;
-      return f.code;
-    }
-    return status;
-  }, &fr);
-  return finish(parent, rc, fr);
+  // gathered: L, h2 (a panel or one value per trait), -log10 p (the primary gets the caller's pointer either way)
+  const DeviceCall d{model_inputs(pr), {pr->Y, (size_t)n}, ncclDouble, sizeof(double),
+                     {{L_out, (size_t)p}, {h2_out, alt ? (size_t)p : 1}, {o->log10p_out, pv ? (size_t)p : 0}}, {}};
+  return run_device(parent, s, d, [&](int r, const RankPtrs& x) -> int {
+    if (!s.count(r)) return BLMM_OK;
+    blmm_problem sp = local_problem(pr, x);
+    sp.Y = (const double*)x.scattered;
+    sp.m = s.count(r);
+    blmm_opts so = *o;
+    so.log10p_out = x.out[2];
+    so.ld_out = p;
+    return blmm_bulkscan(M->sub[r], &sp, &so, x.out[0], x.out[1]);
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -482,16 +557,12 @@ int multi_scan_perms(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* 
   if (!lod_out) return fail(parent, BLMM_E_INVALID, "lod_out is NULL");
   const int64_t n = pr->n, p = pr->p;
   const int64_t ld = o->ld_out ? o->ld_out : p;
-  const bool dev = o->mem_space == BLMM_MEM_DEVICE;
-  const int nd = M->ndev;
-  std::vector<int64_t> s0(nd), s1(nd);
-  shard_perms(nperms, nd, s0, s1);
-  int fr = -1;
+  const Shards s = shard_perms(nperms, M->ndev);
 
-  if (!dev) {
-    const int rc = run_all(M, [&](int r) -> int {
-      const int64_t np = s1[r] - s0[r];
-      if (r > 0 && np == 0) return BLMM_OK;
+  if (o->mem_space != BLMM_MEM_DEVICE) {
+    return run_ranks(parent, [&](int r) -> int {
+      const int64_t j = s.b[r];
+      if (r > 0 && !s.count(r)) return BLMM_OK;
       double *lod = lod_out, *s2 = sigma2_out, *h2 = h2_out;
       if (r > 0) {  // the un-permuted LODs and the null fit are reported by the primary only
         M->scratch[r].resize((size_t)p + 2);
@@ -499,112 +570,33 @@ int multi_scan_perms(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* 
         s2 = lod + p;
         h2 = lod + p + 1;
       }
-      return blmm_scan_perms(M->sub[r], pr, o, perm_idx ? perm_idx + s0[r] * n : nullptr, np, lod,
-                             Lperms_out ? Lperms_out + s0[r] * ld : nullptr, maxlod_out ? maxlod_out + s0[r] : nullptr,
-                             s2, h2);
-    }, &fr);
-    return finish(parent, rc, fr);
+      return blmm_scan_perms(M->sub[r], pr, o, perm_idx ? perm_idx + j * n : nullptr, s.count(r), lod,
+                             Lperms_out ? Lperms_out + j * ld : nullptr, maxlod_out ? maxlod_out + j : nullptr, s2,
+                             h2);
+    });
   }
 
-  if (ld != p) return fail(parent, BLMM_E_INVALID, "multi-GPU device-resident calls need ld_out == p (contiguous slabs)");
-  if (pr->c < 1 || pr->c > MAXC || !pr->Y || !pr->G || !pr->Covar || !pr->U || !pr->lambda)
-    return fail(parent, BLMM_E_INVALID, "bad problem (NULL input or covariate count)");
-  try {
-    ensure_nccl(M);
-  } catch (const Fail& f) {
-    return fail(parent, f.code, f.msg);
-  }
-  int rc = run_all(M, [&](int r) -> int {
-    if (r == 0) return BLMM_OK;
-    try {
-      const size_t np = (size_t)(s1[r] - s0[r]);
-      mbuf<double>(M, r, MB_G, (size_t)n * p);
-      mbuf<double>(M, r, MB_C, (size_t)n * pr->c);
-      mbuf<double>(M, r, MB_U, (size_t)n * n);
-      mbuf<double>(M, r, MB_LAM, n);
-      if (pr->obs_weights) mbuf<double>(M, r, MB_W, n);
-      mbuf<double>(M, r, MB_Y, n);
-      mbuf<int32_t>(M, r, MB_PERM, (size_t)n * np);
-      mbuf<double>(M, r, MB_LOD, p);
-      if (Lperms_out) mbuf<double>(M, r, MB_L, (size_t)p * np);
-      if (maxlod_out) mbuf<double>(M, r, MB_MAX, np);
-      mbuf<double>(M, r, MB_SCAL, 2);
-    } catch (const Fail& f) {
-      M->sub[r]->err = f.msg;
-      return f.code;
+  if (int e = device_checks(parent, pr, o)) return e;
+  std::vector<Part> replicated = model_inputs(pr);
+  replicated.push_back({pr->Y, (size_t)n});
+  // gathered: the per-permutation maxima and L_perms; the other GPUs' un-permuted LODs and null fit (sigma2, h2) stay
+  const DeviceCall d{replicated, {perm_idx, (size_t)n}, ncclInt32, sizeof(int32_t),
+                     {{maxlod_out, 1}, {Lperms_out, (size_t)p}}, {(size_t)p, 2}};
+  return run_device(parent, s, d, [&](int r, const RankPtrs& x) -> int {
+    if (r > 0 && !s.count(r)) return BLMM_OK;
+    blmm_problem sp = local_problem(pr, x);
+    sp.Y = (const double*)x.in[5];
+    blmm_opts so = *o;
+    so.ld_out = p;
+    double *lod = lod_out, *s2 = sigma2_out, *h2 = h2_out;
+    if (r > 0) {
+      lod = x.scratch[0];
+      s2 = x.scratch[1];
+      h2 = x.scratch[1] + 1;
     }
-    return BLMM_OK;
-  }, &fr);
-  if (rc != BLMM_OK) return finish(parent, rc, fr);
-
-  const std::vector<Bcast> bc = {{pr->G, MB_G, (size_t)n * p * 8},   {pr->Covar, MB_C, (size_t)n * pr->c * 8},
-                                 {pr->U, MB_U, (size_t)n * n * 8},   {pr->lambda, MB_LAM, (size_t)n * 8},
-                                 {pr->obs_weights, MB_W, (size_t)n * 8}, {pr->Y, MB_Y, (size_t)n * 8}};
-  rc = run_all(M, [&](int r) -> int {
-    blmm_ctx* c = M->sub[r];
-    cudaStream_t st = c->stream;
-    NcclApi& N = M->nccl;
-    ncclComm_t comm = M->comms[r];
-    int status = BLMM_OK;
-    try {
-      DevBufs& B = M->bufs[r];
-      NCCL_TRY(N.GroupStart());
-      for (const Bcast& b : bc) {
-        if (!b.root_ptr) continue;
-        void* mine = r == 0 ? const_cast<void*>(b.root_ptr) : B.p[b.buf];
-        NCCL_TRY(N.Broadcast(mine, mine, b.bytes, ncclChar, 0, comm, st));
-      }
-      if (r == 0) {
-        for (int q = 1; q < nd; ++q)
-          if (s1[q] > s0[q]) NCCL_TRY(N.Send(perm_idx + s0[q] * n, (size_t)(s1[q] - s0[q]) * n, ncclInt32, q, comm, st));
-      } else if (s1[r] > s0[r]) {
-        NCCL_TRY(N.Recv(B.p[MB_PERM], (size_t)(s1[r] - s0[r]) * n, ncclInt32, 0, comm, st));
-      }
-      NCCL_TRY(N.GroupEnd());
-      const int64_t np = s1[r] - s0[r];
-      blmm_opts so = *o;
-      so.ld_out = p;
-      if (r == 0) {
-        status = blmm_scan_perms(c, pr, &so, perm_idx, np, lod_out, Lperms_out, maxlod_out, sigma2_out, h2_out);
-      } else if (np > 0) {
-        blmm_problem sp = *pr;
-        sp.Y = (const double*)B.p[MB_Y];
-        sp.G = (const double*)B.p[MB_G];
-        sp.Covar = (const double*)B.p[MB_C];
-        sp.U = (const double*)B.p[MB_U];
-        sp.lambda = (const double*)B.p[MB_LAM];
-        if (pr->obs_weights) sp.obs_weights = (const double*)B.p[MB_W];
-        double* sc = (double*)B.p[MB_SCAL];
-        status = blmm_scan_perms(c, &sp, &so, (const int32_t*)B.p[MB_PERM], np, (double*)B.p[MB_LOD],
-                                 Lperms_out ? (double*)B.p[MB_L] : nullptr, maxlod_out ? (double*)B.p[MB_MAX] : nullptr,
-                                 sc, sc + 1);
-      }
-      // NCCL gather of the per-permutation maxima (and the L_perms slabs when they are materialised)
-      if (r == 0) {
-        CUDA_TRY(cudaEventRecord(M->g0, st));
-        NCCL_TRY(N.GroupStart());
-        for (int q = 1; q < nd; ++q) {
-          const size_t nq = (size_t)(s1[q] - s0[q]);
-          if (!nq) continue;
-          if (maxlod_out) NCCL_TRY(N.Recv(maxlod_out + s0[q], nq, ncclDouble, q, comm, st));
-          if (Lperms_out) NCCL_TRY(N.Recv(Lperms_out + s0[q] * p, nq * p, ncclDouble, q, comm, st));
-        }
-        NCCL_TRY(N.GroupEnd());
-        CUDA_TRY(cudaEventRecord(M->g1, st));
-        M->gather_timed = true;
-      } else if (np > 0) {
-        NCCL_TRY(N.GroupStart());
-        if (maxlod_out) NCCL_TRY(N.Send(B.p[MB_MAX], (size_t)np, ncclDouble, 0, comm, st));
-        if (Lperms_out) NCCL_TRY(N.Send(B.p[MB_L], (size_t)np * p, ncclDouble, 0, comm, st));
-        NCCL_TRY(N.GroupEnd());
-      }
-    } catch (const Fail& f) {
-      c->err = f.msg;
-      return f.code;
-    }
-    return status;
-  }, &fr);
-  return finish(parent, rc, fr);
+    return blmm_scan_perms(M->sub[r], &sp, &so, (const int32_t*)x.scattered, s.count(r), lod, x.out[1], x.out[0], s2,
+                           h2);
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -625,18 +617,14 @@ int multi_fit_h2(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o, d
                  double* ell_out) {
   MultiState* M = parent->multi;
   if (int e = host_only(parent, pr, o)) return e;
-  int fr = -1;
-  const int rc = run_all(M, [&](int r) -> int {
-    int64_t j0, j1;
-    shard_cols(pr->m, M->ndev, r, 32, &j0, &j1);
-    if (j1 == j0) return BLMM_OK;
-    blmm_problem sp = *pr;
-    sp.Y = pr->Y + j0 * pr->n;
-    sp.m = j1 - j0;
-    return blmm_fit_h2(M->sub[r], &sp, o, h2_out ? h2_out + j0 : nullptr, sigma2_out ? sigma2_out + j0 : nullptr,
-                       ell_out ? ell_out + j0 : nullptr);
-  }, &fr);
-  return finish(parent, rc, fr);
+  const Shards s = shard_cols(pr->m, M->ndev, 32);
+  return run_ranks(parent, [&](int r) -> int {
+    if (!s.count(r)) return BLMM_OK;
+    const int64_t j = s.b[r];
+    const blmm_problem sp = trait_block(pr, s, r);
+    return blmm_fit_h2(M->sub[r], &sp, o, h2_out ? h2_out + j : nullptr, sigma2_out ? sigma2_out + j : nullptr,
+                       ell_out ? ell_out + j : nullptr);
+  });
 }
 
 int multi_scan_null(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o, double* lod_out, double* sigma2_out,
@@ -645,20 +633,16 @@ int multi_scan_null(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o
   if (int e = host_only(parent, pr, o)) return e;
   if (!lod_out) return fail(parent, BLMM_E_INVALID, "lod_out is NULL");
   const int64_t ld = o->ld_out ? o->ld_out : pr->p;
-  int fr = -1;
-  const int rc = run_all(M, [&](int r) -> int {
-    int64_t j0, j1;
-    shard_cols(pr->m, M->ndev, r, 64, &j0, &j1);
-    if (j1 == j0) return BLMM_OK;
-    blmm_problem sp = *pr;
-    sp.Y = pr->Y + j0 * pr->n;
-    sp.m = j1 - j0;
+  const Shards s = shard_cols(pr->m, M->ndev, 64);
+  return run_ranks(parent, [&](int r) -> int {
+    if (!s.count(r)) return BLMM_OK;
+    const int64_t j = s.b[r];
+    const blmm_problem sp = trait_block(pr, s, r);
     blmm_opts so = *o;
-    if (o->log10p_out) so.log10p_out = o->log10p_out + j0 * ld;
-    return blmm_scan_null(M->sub[r], &sp, &so, lod_out + j0 * ld, sigma2_out ? sigma2_out + j0 : nullptr,
-                          h2_out ? h2_out + j0 : nullptr);
-  }, &fr);
-  return finish(parent, rc, fr);
+    if (o->log10p_out) so.log10p_out = o->log10p_out + j * ld;
+    return blmm_scan_null(M->sub[r], &sp, &so, lod_out + j * ld, sigma2_out ? sigma2_out + j : nullptr,
+                          h2_out ? h2_out + j : nullptr);
+  });
 }
 
 int multi_bulkscan_peaks(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o, double* peak_lod_out,
@@ -666,37 +650,28 @@ int multi_bulkscan_peaks(blmm_ctx* parent, const blmm_problem* pr, const blmm_op
   MultiState* M = parent->multi;
   if (int e = host_only(parent, pr, o)) return e;
   if (!peak_lod_out) return fail(parent, BLMM_E_INVALID, "peak_lod_out is NULL");
-  int fr = -1;
-  const int rc = run_all(M, [&](int r) -> int {
-    int64_t j0, j1;
-    shard_cols(pr->m, M->ndev, r, SCAN_TT, &j0, &j1);
-    if (j1 == j0) return BLMM_OK;
-    blmm_problem sp = *pr;
-    sp.Y = pr->Y + j0 * pr->n;
-    sp.m = j1 - j0;
+  const Shards s = shard_cols(pr->m, M->ndev, SCAN_TT);
+  return run_ranks(parent, [&](int r) -> int {
+    if (!s.count(r)) return BLMM_OK;
+    const int64_t j = s.b[r];
+    const blmm_problem sp = trait_block(pr, s, r);
     blmm_opts so = *o;
-    if (o->log10p_out) so.log10p_out = o->log10p_out + j0;
-    return blmm_bulkscan_peaks(M->sub[r], &sp, &so, peak_lod_out + j0, peak_marker_out ? peak_marker_out + j0 : nullptr,
-                               h2_out ? h2_out + j0 : nullptr);
-  }, &fr);
-  return finish(parent, rc, fr);
+    if (o->log10p_out) so.log10p_out = o->log10p_out + j;
+    return blmm_bulkscan_peaks(M->sub[r], &sp, &so, peak_lod_out + j, peak_marker_out ? peak_marker_out + j : nullptr,
+                               h2_out ? h2_out + j : nullptr);
+  });
 }
 
 int multi_grid_loglik(blmm_ctx* parent, const blmm_problem* pr, const blmm_opts* o, double* ell_out) {
   MultiState* M = parent->multi;
   if (int e = host_only(parent, pr, o)) return e;
   if (!ell_out) return fail(parent, BLMM_E_INVALID, "ell_out is NULL");
-  int fr = -1;
-  const int rc = run_all(M, [&](int r) -> int {
-    int64_t j0, j1;
-    shard_cols(pr->m, M->ndev, r, 32, &j0, &j1);
-    if (j1 == j0) return BLMM_OK;
-    blmm_problem sp = *pr;
-    sp.Y = pr->Y + j0 * pr->n;
-    sp.m = j1 - j0;
-    return blmm_grid_loglik(M->sub[r], &sp, o, ell_out + j0 * o->ngrid);
-  }, &fr);
-  return finish(parent, rc, fr);
+  const Shards s = shard_cols(pr->m, M->ndev, 32);
+  return run_ranks(parent, [&](int r) -> int {
+    if (!s.count(r)) return BLMM_OK;
+    const blmm_problem sp = trait_block(pr, s, r);
+    return blmm_grid_loglik(M->sub[r], &sp, o, ell_out + s.b[r] * o->ngrid);
+  });
 }
 
 }  // namespace blmm
