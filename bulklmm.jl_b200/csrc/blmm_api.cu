@@ -497,7 +497,7 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   // stream does the trait rotation and then (after the weight constants) the trait statistics.
   CUDA_TRY(cudaEventRecord(ctx->fork_ev, ctx->stream));
   CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->fork_ev, 0));
-  const bool rot_in_wc = pr->n <= 128;  // small n: the covariate rotation is folded into the weight-constant blocks
+  const bool rot_in_wc = weight_consts_rot_applies(R.n);  // the covariate rotation folded into the weight constants
   if (!rot_in_wc) rotate_covariates(ctx, R, ctx->copy_stream);
   rotate_markers_aside(ctx, pr, R, ms);
   if (rot_in_wc)
@@ -509,7 +509,7 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   CUDA_TRY(cudaEventRecord(ctx->wc_ev, ctx->copy_stream));
   wait_markers(ctx, ctx->copy_stream);
   ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, nk, wc, true, Mop, ctx->d_flags,
-                                         ctx->copy_stream);
+                                         ctx->sm_count, ctx->copy_stream);
   CUDA_TRY(cudaEventRecord(ctx->join_ev, ctx->copy_stream));
   rotate_traits(ctx, pr, R, ms);
   CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ctx->wc_ev, 0));
@@ -523,8 +523,8 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   int* bin_count = bins, *bin_start = bins + 256, *bin_cursor = bins + 512, *n_tiles = bins + 768;
   CUDA_TRY(cudaMemsetAsync(bins, 0, (3 * 256 + 8) * sizeof(int), ctx->stream));
 
-  // alt-grid: the statistics kernel also writes the packed trait operand and the per-k scalars when it can
-  TraitFuse fuse{nullptr, nullptr, nullptr, 0, false};
+  // alt-grid: the trait statistics also produce the packed trait operand and the per-k scalars
+  TraitFuse fuse{};
   if (alt) {
     fuse.tcol_pad = round_up(m, SCAN_TT);
     fuse.e = ws<double>(ctx, S_E, (size_t)nk * fuse.tcol_pad);
@@ -532,8 +532,8 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
     fuse.Top = ws<double>(ctx, S_TOP, (size_t)R.n_pad * fuse.tcol_pad);
   }
   ctx->launches += launch_trait_stats(R.Y0, m, R.n, R.n_pad, R.c, nk, wc, lik_of(o), d_grid, Yr, ell, rss, best,
-                                      ellmax, h2v, alt ? nullptr : bin_count, ctx->d_flags, ctx->stream,
-                                      alt ? &fuse : nullptr);
+                                      ellmax, h2v, alt ? nullptr : bin_count, ctx->d_flags, alt ? &fuse : nullptr,
+                                      ctx->sm_count, ctx->stream);
 
   ScanParams P{};
   P.Mop = Mop;
@@ -549,10 +549,6 @@ int bulkscan_grid(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, dou
   P.ldL = ldL;
   P.peaks = parts;
   if (alt) {
-    if (!fuse.done) {
-      ctx->launches += launch_alt_scalars(ell, rss, ellmax, m, fuse.tcol_pad, nk, R.n, fuse.e, fuse.et, ctx->stream);
-      ctx->launches += launch_pack_traits(Yr, nullptr, m, fuse.tcol_pad, R.n_pad, nullptr, fuse.Top, ctx->stream);
-    }
     P.Top = fuse.Top;
     P.e = fuse.e;
     P.et = fuse.et;
@@ -617,7 +613,7 @@ int grid_loglik(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, doubl
   int* best = ws<int>(ctx, S_BEST, m);
   double* ellmax = ws<double>(ctx, S_ELLMAX, m);
   ctx->launches += launch_trait_stats(R.Y0, m, R.n, R.n_pad, R.c, nk, wc, lik_of(o), d_grid, Yr, ell, rss, best,
-                                      ellmax, nullptr, nullptr, ctx->d_flags, ctx->stream);
+                                      ellmax, nullptr, nullptr, ctx->d_flags, nullptr, ctx->sm_count, ctx->stream);
   // a zero-norm trait is only an error for the scans (colDivide!), not for wls_multivar (a device-mode call leaves
   // the flag for the next blmm_sync)
   if (!out.dev) CUDA_TRY(cudaMemsetAsync(ctx->d_flags + FLAG_ZERO_NORM, 0, sizeof(int), ctx->stream));
@@ -635,7 +631,7 @@ double* residualised_traits(blmm_ctx* ctx, const Rotated& R, const blmm_opts* o)
   int* best = ws<int>(ctx, S_BEST, R.m);
   double* ellmax = ws<double>(ctx, S_ELLMAX, R.m);
   ctx->launches += launch_trait_stats(R.Y0, R.m, R.n, R.n_pad, R.c, 0, wc0, lik_of(o), nullptr, Yr, ell, rss, best,
-                                      ellmax, nullptr, nullptr, ctx->d_flags, ctx->stream);
+                                      ellmax, nullptr, nullptr, ctx->d_flags, nullptr, ctx->sm_count, ctx->stream);
   return Yr;
 }
 
@@ -696,7 +692,8 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   WeightConsts wc0 = weight_ws(ctx, 0, R.n_pad, R.c);
   double* Mop = ws<double>(ctx, S_MOP, (size_t)R.n_pad * p_pad);
   wait_markers(ctx, ctx->stream);  // U'G was computed on the third stream meanwhile
-  ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, 1, wc0, false, Mop, ctx->d_flags, ctx->stream);
+  ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, 1, wc0, false, Mop, ctx->d_flags,
+                                         ctx->sm_count, ctx->stream);
   const int cg = R.c + 2;
   const int64_t n_tt = (m + 63) / 64;
   const int64_t slots = n_tt * 64;
@@ -801,21 +798,16 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
   // Small n: rotation of y and the covariates, residualisation, Brent, weight constants and the null residual are ONE
   // launch (null_fit_chain_kernel), with the markers rotated beside it; otherwise the same steps as separate kernels,
   // the markers forked after the trait rotation.
-  const bool fused = pr->n <= 128 && !getenv("BLMM_B200_NO_CHAIN");  // test hook: force the separate kernels
-  bool chained = false;
-  if (fused) {
+  if (null_fit_chain_applies(R.n) && !getenv("BLMM_B200_NO_CHAIN")) {  // test hook: force the separate kernels
     rotate_markers_aside(ctx, pr, R, ms);
     const double* dY = stage_in(ctx, S_Y_IN, pr->Y, (size_t)pr->n, ms);
     double* Yr1 = ws<double>(ctx, S_YR, (size_t)R.n_pad);
-    const int launched = launch_null_fit_chain(R.dU, dY, R.dC, R.lambda, R.n, R.n_pad, R.c, lik_of(o), o->optim_interval,
-                                               R.C0, Yr1, wc, h2, s2, z, zrss, ctx->d_flags, ctx->stream);
-    ctx->launches += launched;
-    chained = launched > 0;  // 0: does not apply (shared memory)
-  }
-  if (!chained) {
+    ctx->launches += launch_null_fit_chain(R.dU, dY, R.dC, R.lambda, R.n, R.n_pad, R.c, lik_of(o), o->optim_interval,
+                                           R.C0, Yr1, wc, h2, s2, z, zrss, ctx->d_flags, ctx->stream);
+  } else {
     rotate_covariates(ctx, R, ctx->stream);
     rotate_traits(ctx, pr, R, ms);
-    if (!fused) rotate_markers_aside(ctx, pr, R, ms);
+    rotate_markers_aside(ctx, pr, R, ms);
     double* Yr = residualised_traits(ctx, R, o);
     ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2,
                                    nullptr, ctx->d_flags, ctx->stream);
@@ -826,7 +818,8 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
   const int64_t p_pad = round_up(p, SCAN_MT);
   double* Mop = ws<double>(ctx, S_MOP, (size_t)R.n_pad * p_pad);
   wait_markers(ctx, ctx->stream);  // U'G was computed on the third stream meanwhile
-  ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, 1, wc, false, Mop, ctx->d_flags, ctx->stream);
+  ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, 1, wc, false, Mop, ctx->d_flags,
+                                         ctx->sm_count, ctx->stream);
 
   const int64_t ncol = nperms + 1;
   const int64_t tcol_pad = round_up(ncol, SCAN_TT);

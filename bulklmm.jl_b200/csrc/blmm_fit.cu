@@ -229,6 +229,24 @@ __device__ void brent(const FitData& d, double lo, double hi, double* xmin, doub
   *fmin_out = fx;
 }
 
+// gridbrent over [0, 1] in optim_interval pieces (src/gridbrent.jl:9-24): points = range(0, 1, length =
+// optim_interval + 1); keeps the first of equal minima
+template <int C, int UNR = 4>
+__device__ double fit_one(const FitData& d, int optim_interval) {
+  double bx = 0.0, bf = INFINITY;
+  for (int i = 0; i < optim_interval; ++i) {
+    const double lo = (double)i / (double)optim_interval;
+    const double hi = (i + 1 == optim_interval) ? 1.0 : (double)(i + 1) / (double)optim_interval;
+    double x, f;
+    brent<C, UNR>(d, lo, hi, &x, &f);
+    if (i == 0 || f < bf) {
+      bx = x;
+      bf = f;
+    }
+  }
+  return bx;
+}
+
 // Templated on the covariate count so that the common c = 1..3 cases keep their Gram matrices in a few
 // registers (a run-time switch over all eight sizes cost 200 registers per thread: 8 warps per SM).
 // BULK: many traits — occupancy hides the latency of each warp's chain (64 registers for c <= 2); otherwise (a few
@@ -262,18 +280,7 @@ __global__ void __launch_bounds__(32 * FIT_WARPS, BULK ? (C <= 2 ? 8 : (C <= 4 ?
   }
   if (j >= m) return;
   FitData d{yv, C0, lambda, n, n_pad, c, lane, lik, nullptr, false, ltab, fit_inv_denom(lik, n, C)};
-  // gridbrent: points = range(0, 1, length = optim_interval + 1); keep the first of equal minima
-  double bx = 0.0, bf = INFINITY;
-  for (int i = 0; i < optim_interval; ++i) {
-    const double lo = (double)i / (double)optim_interval;
-    const double hi = (i + 1 == optim_interval) ? 1.0 : (double)(i + 1) / (double)optim_interval;
-    double x, f;
-    brent<C, BULK ? 1 : 4>(d, lo, hi, &x, &f);
-    if (i == 0 || f < bf) {
-      bx = x;
-      bf = f;
-    }
-  }
+  const double bx = fit_one<C, BULK ? 1 : 4>(d, optim_interval);
   double s2;
   const double f = neg_loglik_c<C, BULK ? 1 : 4>(d, bx, &s2);
   if (lane == 0) {
@@ -281,23 +288,6 @@ __global__ void __launch_bounds__(32 * FIT_WARPS, BULK ? (C <= 2 ? 8 : (C <= 4 ?
     if (sigma2_out) sigma2_out[j] = s2;
     if (ell_out) ell_out[j] = -f;
   }
-}
-
-// gridbrent over [0, 1] in optim_interval pieces (src/gridbrent.jl:9-24): first of equal minima
-template <int C>
-__device__ double fit_one(const FitData& d, int optim_interval) {
-  double bx = 0.0, bf = INFINITY;
-  for (int i = 0; i < optim_interval; ++i) {
-    const double lo = (double)i / (double)optim_interval;
-    const double hi = (i + 1 == optim_interval) ? 1.0 : (double)(i + 1) / (double)optim_interval;
-    double x, f;
-    brent<C>(d, lo, hi, &x, &f);
-    if (i == 0 || f < bf) {
-      bx = x;
-      bf = f;
-    }
-  }
-  return bx;
 }
 
 // scan_alt (src/scan.jl:397-453), one warp per marker: covariates [C0 g_i] (C = c + 1 columns), the variance
@@ -349,7 +339,7 @@ __global__ void scan_alt_null_kernel(const double* __restrict__ y, int n, int n_
 //   residual z = P (sw .* y) of transform_reweight (src/transform_helpers.jl:57-92).
 // It replaces seven launches (rotate x2, weight constants x2, trait statistics, Brent, null residual) whose kernels take
 // 4-12 us each and whose launch gaps are as long again: a permutation step is 0.45 ms of scan, so they were a tenth
-// of it.  For n <= 128 (the rotation is done by one thread per output here).
+// of it.  For small n only (null_fit_chain_applies): the rotation is done by one thread per output here.
 // -----------------------------------------------------------------------------------------------
 template <int C>
 __global__ void __launch_bounds__(128, 1)
@@ -370,14 +360,9 @@ __global__ void __launch_bounds__(128, 1)
   // U'[Cov y]: one thread per output
   for (int idx = tid; idx < (C + 1) * n_pad; idx += 128) {
     const int col = idx / n_pad, a = idx % n_pad;
-    double v = 0.0;
-    if (a < n) {
-      const double* u = U + (int64_t)a * n;
-      const double* x = (col < C) ? Cov + (int64_t)col * n : y;
-      // one accumulator, k ascending: the summation order of rotate_kernel, so that this path and the separate kernels
-      // (and scan without permutations) see bit-identical rotated inputs and hence the same Brent trajectory
-      for (int b = 0; b < n; ++b) v = fma(u[b], x[b], v);
-    }
+    // rotate_elem: this path and the separate kernels (and scan without permutations) see bit-identical rotated inputs
+    // and hence the same Brent trajectory
+    const double v = (a < n) ? rotate_elem(U, (col < C) ? Cov + (int64_t)col * n : y, n, a) : 0.0;
     if (col < C) {
       c_s[idx] = v;
       C0_out[idx] = v;
@@ -388,17 +373,10 @@ __global__ void __launch_bounds__(128, 1)
   for (int l = tid; l < n_pad; l += 128) lam_s[l] = (l < n) ? lambda[l] : 0.0;
   __syncthreads();
   // unweighted basis of the covariates (slot 1 of wc: w = 1), then Yr = y0 - Q Q'y0
-  weight_consts_block(true, 0.0, lam_s, c_s, n, n_pad, C, wc.w + n_pad, wc.sw + n_pad, wc.Q + (int64_t)C * n_pad,
-                      wc.slw + 1, wc.lds + 1, flags, sh);
+  const WeightSlot ols = weight_slot(wc, 1, n_pad, C);
+  weight_consts_block(true, 0.0, lam_s, c_s, n, n_pad, C, ols, flags, sh);
   if (warp == 0) {
-    double coef[MAXC];
-    proj_coefs(y_s, wc.sw + n_pad, wc.Q + (int64_t)C * n_pad, n_pad, C, lane, coef);
-    for (int l = lane; l < n_pad; l += 32) {
-      const double v = proj_elem(y_s, wc.sw + n_pad, wc.Q + (int64_t)C * n_pad, n_pad, C, l, coef);
-      y_s[l] = v;  // each lane rewrites only the elements it read last
-      Yr_out[l] = v;
-    }
-    __syncwarp();
+    unweighted_residual(y_s, ols, n_pad, C, lane, [&](int l, double v) { Yr_out[l] = v; });
     FitData d{y_s, c_s, lam_s, n, n_pad, C, lane, lik, nullptr, false, ltab, fit_inv_denom(lik, n, C)};
     const double h2 = fit_one<C>(d, optim_interval);
     double s2;
@@ -411,57 +389,41 @@ __global__ void __launch_bounds__(128, 1)
   }
   __syncthreads();
   // transform_reweight at the fitted h2 (slot 0)
-  weight_consts_block(false, h2_s, lam_s, c_s, n, n_pad, C, wc.w, wc.sw, wc.Q, wc.slw, wc.lds, flags, sh);
+  const WeightSlot w0 = weight_slot(wc, 0, n_pad, C);
+  weight_consts_block(false, h2_s, lam_s, c_s, n, n_pad, C, w0, flags, sh);
   if (warp == 0) {
     double coef[MAXC];
-    proj_coefs(y_s, wc.sw, wc.Q, n_pad, C, lane, coef);
-    double ss = 0.0;
-    for (int l = lane; l < n_pad; l += 32) {
-      const double v = proj_elem(y_s, wc.sw, wc.Q, n_pad, C, l, coef);
-      z_out[l] = v;
-      ss = fma(v, v, ss);
-    }
-    ss = warp_sum(ss);
+    const double ss = proj_norm2(y_s, w0, n_pad, C, lane, coef, z_out);
     if (lane == 0) *zrss_out = ss;
   }
 }
 
 }  // namespace
 
+// one block rotates y and the covariates with one thread per output, each a length-n dot product: small n only (then
+// the shared memory, 2 FIT_LTAB + (2 + c) n_pad doubles, is under 20 KB for every c <= MAXC)
+bool null_fit_chain_applies(int n) { return n <= 128; }
+
 int launch_null_fit_chain(const double* U, const double* y, const double* Cov, const double* lambda, int n, int n_pad,
                           int c, LikParams lik, int optim_interval, double* C0, double* Yr, WeightConsts wc, double* h2,
                           double* sigma2, double* z, double* zrss, int* flags, cudaStream_t stream) {
   const size_t smem = ((size_t)2 * FIT_LTAB + (size_t)(2 + c) * n_pad) * sizeof(double);
-  if (n > 128 || smem > 48 * 1024) return 0;
-#define BLMM_CHAIN(CC)                                                                                              \
-  case CC:                                                                                                          \
-    null_fit_chain_kernel<CC><<<1, 128, smem, stream>>>(U, y, Cov, lambda, n, n_pad, lik, optim_interval, C0, Yr, wc, \
-                                                        h2, sigma2, z, zrss, flags);                                \
-    break;
-  switch (c) {
-    BLMM_CHAIN(1) BLMM_CHAIN(2) BLMM_CHAIN(3) BLMM_CHAIN(4) BLMM_CHAIN(5) BLMM_CHAIN(6) BLMM_CHAIN(7) BLMM_CHAIN(8)
-    default: return 0;
-  }
-#undef BLMM_CHAIN
-  return 1;
+  return dispatch_c<1, MAXC>(c, [&](auto C) {
+    null_fit_chain_kernel<C><<<1, 128, smem, stream>>>(U, y, Cov, lambda, n, n_pad, lik, optim_interval, C0, Yr, wc, h2,
+                                                       sigma2, z, zrss, flags);
+  });
 }
 
 int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_pad, int c, const double* C0,
                     const double* lambda, LikParams lik, int optim_interval, const double* h2_null, double* ell_null,
                     double* lod, double* h2_each, cudaStream_t stream) {
   const unsigned blocks = (unsigned)((p + FIT_WARPS - 1) / FIT_WARPS);
-#define BLMM_ALT(CC)                                                                                              \
-  case CC:                                                                                                        \
-    scan_alt_null_kernel<CC><<<1, 32, 0, stream>>>(y, n, n_pad, C0, lambda, lik, h2_null, ell_null);              \
-    scan_alt_kernel<CC + 1><<<blocks, 32 * FIT_WARPS, 0, stream>>>(y, G0, p, n, n_pad, C0, lambda, lik,           \
-                                                                   optim_interval, ell_null, lod, h2_each);       \
-    break;
-  switch (c) {
-    BLMM_ALT(1) BLMM_ALT(2) BLMM_ALT(3) BLMM_ALT(4) BLMM_ALT(5) BLMM_ALT(6) BLMM_ALT(7)
-    default: return 0;
-  }
-#undef BLMM_ALT
-  return 2;
+  const bool ok = dispatch_c<1, MAXC - 1>(c, [&](auto C) {
+    scan_alt_null_kernel<C><<<1, 32, 0, stream>>>(y, n, n_pad, C0, lambda, lik, h2_null, ell_null);
+    scan_alt_kernel<C + 1><<<blocks, 32 * FIT_WARPS, 0, stream>>>(y, G0, p, n, n_pad, C0, lambda, lik, optim_interval,
+                                                                  ell_null, lod, h2_each);
+  });
+  return ok ? 2 : 0;
 }
 
 int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const double* C0,
@@ -474,26 +436,17 @@ int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const do
   const int staged = smem <= 96 * 1024 ? 1 : 0;
   if (!staged) smem = tab_bytes;
   const bool bulk = blocks > 148 * 4;
-#define BLMM_FIT(CC)                                                                                          \
-  case CC:                                                                                                    \
-    if (bulk) {                                                                                               \
-      if (smem > 48 * 1024)                                                                                   \
-        cudaFuncSetAttribute(fit_h2_kernel<CC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-      fit_h2_kernel<CC, true><<<blocks, 32 * FIT_WARPS, smem, stream>>>(Yr, m, n, n_pad, c, C0, lambda, lik,  \
-                                                                        optim_interval, h2, sigma2, ell, staged); \
-    } else {                                                                                                  \
-      if (smem > 48 * 1024)                                                                                   \
-        cudaFuncSetAttribute(fit_h2_kernel<CC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-      fit_h2_kernel<CC, false><<<blocks, 32 * FIT_WARPS, smem, stream>>>(Yr, m, n, n_pad, c, C0, lambda, lik, \
-                                                                         optim_interval, h2, sigma2, ell, staged); \
-    }                                                                                                         \
-    break;
-  switch (c) {
-    BLMM_FIT(1) BLMM_FIT(2) BLMM_FIT(3) BLMM_FIT(4) BLMM_FIT(5) BLMM_FIT(6) BLMM_FIT(7) BLMM_FIT(8)
-    default: return 0;
-  }
-#undef BLMM_FIT
-  return 1;
+  auto launch = [&](auto kernel) {
+    if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    kernel<<<blocks, 32 * FIT_WARPS, smem, stream>>>(Yr, m, n, n_pad, c, C0, lambda, lik, optim_interval, h2, sigma2,
+                                                     ell, staged);
+  };
+  return dispatch_c<1, MAXC>(c, [&](auto C) {
+    if (bulk)
+      launch(fit_h2_kernel<C, true>);
+    else
+      launch(fit_h2_kernel<C, false>);
+  });
 }
 
 }  // namespace blmm

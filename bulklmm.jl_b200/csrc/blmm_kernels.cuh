@@ -8,9 +8,26 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "blmm_common.cuh"
 
 namespace blmm {
+
+// Run-time covariate count to template argument: f(std::integral_constant<int, C>{}) for the C in [LO, HI] equal to
+// c; returns false, calling nothing, when c is outside the range.
+template <int LO, int HI, class F>
+bool dispatch_c(int c, F&& f) {
+  if constexpr (LO > HI) {
+    return false;
+  } else {
+    if (c == LO) {
+      f(std::integral_constant<int, LO>{});
+      return true;
+    }
+    return dispatch_c<LO + 1, HI>(c, f);
+  }
+}
 
 // ---- preprocessing (blmm_prep.cu) -------------------------------------------------------------
 
@@ -39,8 +56,9 @@ struct WeightConsts {
 int launch_weight_consts(const double* h2_dev, int nk, const double* lambda, const double* C0, int n,
                          int n_pad, int c, WeightConsts wc, int* flags, cudaStream_t stream);
 
-// The same from the UNROTATED covariates (Cov: n x c, ld n) for n <= 128: each block rotates them by U' itself and block 0
-// also writes C0; returns 0 (nothing launched) for larger n.
+// The same from the UNROTATED covariates (Cov: n x c, ld n), for the n where weight_consts_rot_applies: each block
+// rotates them by U' itself and block 0 also writes C0.
+bool weight_consts_rot_applies(int n);
 int launch_weight_consts_rot(const double* h2_dev, int nk, const double* lambda, const double* U, const double* Cov,
                              int n, int n_pad, int c, WeightConsts wc, double* C0, int* flags, cudaStream_t stream);
 
@@ -55,20 +73,19 @@ struct LikParams {  // wls / wls_multivar scalars, src/wls.jl:72-92, 150-170
 //   rss  : [nk][m] weighted residual sum of squares (= squared norm of the residualised trait)
 //   best : [m] first arg-max over k of ell (findmax, src/bulkscan_helpers.jl:204-211)
 //   ellmax: [m] max_k ell;   h2_out (optional): grid[best];   bin_count (optional): histogram of best
-// `fuse` (optional, alt-grid): also produce what launch_alt_scalars + launch_pack_traits (identity column map)
-// would — Top[q][j][kk], e[k][j], et[k][j] for j < tcol_pad (pads: 0, 1, 0) — when the kernel in use can (the
-// table form with all grid points in one lane batch); fuse->done tells the caller whether it did.
+// `fuse` (optional, alt-grid): also the scan's trait operands for j < tcol_pad — Top[q][j][kk] = Yr (pads 0),
+// e[k][j] = exp(-2 (ell[k,j] - ellmax_j) / n) (pads 1), et = e / rss (pads 0) — in the statistics kernel itself when
+// its table form holds every grid point in one lane batch, else by two more kernels.
 struct TraitFuse {
   double* Top;
   double* e;
   double* et;
   int64_t tcol_pad;
-  bool done;
 };
 int launch_trait_stats(const double* Y0, int64_t m, int n, int n_pad, int c, int nk, WeightConsts wc,
                        LikParams lik, const double* grid_dev, double* Yr, double* ell, double* rss,
-                       int* best, double* ellmax, double* h2_out, int* bin_count, int* flags,
-                       cudaStream_t stream, TraitFuse* fuse = nullptr);
+                       int* best, double* ellmax, double* h2_out, int* bin_count, int* flags, const TraitFuse* fuse,
+                       int sm_count, cudaStream_t stream);
 
 // One warp per marker: x = P_k (sw_k .* g_i) / ||P_k (sw_k .* g_i)||  (the normalised X00 column of
 // weighted_liteqtl + computeR_LMM, src/bulkscan_helpers.jl:175-201, 47-64).
@@ -77,11 +94,7 @@ int launch_trait_stats(const double* Y0, int64_t m, int n, int n_pad, int c, int
 //   fold_sw = false: Mop = x, for trait operands that are already weighted and projected
 //                    (permutations of the re-weighted null residual, src/scan.jl:531-541; w = 1 slot).
 int launch_marker_operand(const double* G0, int64_t p, int64_t p_pad, int n, int n_pad, int c, int nk,
-                          WeightConsts wc, bool fold_sw, double* Mop, int* flags, cudaStream_t stream);
-
-// alt-grid trait scalars: e[k][j] = exp(-2 (ell[k,j] - ellmax_j) / n), et = e / rss; pads e=1, et=0.
-int launch_alt_scalars(const double* ell, const double* rss, const double* ellmax, int64_t m,
-                       int64_t tcol_pad, int nk, int n, double* e, double* et, cudaStream_t stream);
+                          WeightConsts wc, bool fold_sw, double* Mop, int* flags, int sm_count, cudaStream_t stream);
 
 // null-grid binning: lay the traits out bin by bin, each bin padded to a multiple of `tile`.
 //   tile_k0[t]  : grid index of trait tile t;  n_tiles: number of tiles in use (device scalar)
@@ -115,10 +128,11 @@ int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const do
                   const double* lambda, LikParams lik, int optim_interval, double* h2, double* sigma2,
                   double* ell, int* flags, cudaStream_t stream);
 
-// The single-trait prologue of scan with permutations in one launch (n <= 128; returns 0 when it does not apply and
-// the caller uses the separate launches): C0 = U'Cov (n_pad x c), Yr = residual of U'y on C0, h2 / sigma2 = fitlmm,
+// The single-trait prologue of scan with permutations in one launch, for the n where null_fit_chain_applies (else the
+// caller runs the separate launches): C0 = U'Cov (n_pad x c), Yr = residual of U'y on C0, h2 / sigma2 = fitlmm,
 // wc slot 0 = constants at h2 (slot 1 = the unweighted ones), z = P (sw .* Yr) with zrss = ||z||^2.
 // U: n x n (ld n), y: n, Cov: n x c (ld n) — unrotated device inputs.
+bool null_fit_chain_applies(int n);
 int launch_null_fit_chain(const double* U, const double* y, const double* Cov, const double* lambda, int n, int n_pad,
                           int c, LikParams lik, int optim_interval, double* C0, double* Yr, WeightConsts wc, double* h2,
                           double* sigma2, double* z, double* zrss, int* flags, cudaStream_t stream);
@@ -189,7 +203,9 @@ constexpr int SCAN_MAX_NQ = 5;  // largest number of K-chunks for which launch_s
 int launch_scan(const ScanParams& P, int sm_count, cudaStream_t stream);
 int launch_scan_stream_grid(const ScanParams& P, int sm_count, cudaStream_t stream);
 
-int stream_exact_marker_tile(int c);  // marker tile of the EXACT kernel for c covariates
+// marker atoms (8 markers each, per warp) of the EXACT kernel for c covariates: its c + 2 operand kinds take registers
+constexpr int exact_marker_atoms(int c) { return c + 2 <= 5 ? 4 : 2; }
+constexpr int stream_exact_marker_tile(int c) { return 2 * 8 * exact_marker_atoms(c); }  // markers per CTA tile
 // z_j, q_j1..q_jc, w_j columns and 1/dy_j of every trait at its own h2 (slots = n_tt*64 >= m)
 int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* C0, int64_t m,
                          int64_t slots, int n, int n_pad, int c, double* Xop, int64_t xcol_pad, double* dyinv,

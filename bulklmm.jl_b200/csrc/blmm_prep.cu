@@ -16,6 +16,29 @@ namespace {
 
 constexpr int WARPS_PER_BLOCK = 8;
 
+// Lane batches of the table kernels: KB grid points of (1 + c) kinds each per batch of 32 lane slots.
+__host__ __device__ inline int table_kb(int c) {
+  const int KB = 32 / (1 + c);
+  return KB;
+}
+__host__ __device__ inline int table_batches(int c, int nk) { return (nk + table_kb(c) - 1) / table_kb(c); }
+
+// Dynamic shared memory of the table kernels (the tables and two staged vectors per warp), or 0 when it is over the
+// limit and the generic kernel runs instead (BXD-size grid scans: 30 KB and 51 KB).
+size_t trait_table_smem(int n_pad, int c, int nk) {
+  const size_t table_smem =
+      ((size_t)table_batches(c, nk) * n_pad * 32 + (size_t)WARPS_PER_BLOCK * 2 * n_pad) * sizeof(double);
+  if (table_smem <= 96 * 1024) return table_smem;
+  return 0;
+}
+size_t marker_table_smem(int n_pad, int c, int nk) {  // + the transposed table and the store offsets
+  const int nbatch = table_batches(c, nk);
+  const size_t tsmem =
+      ((size_t)2 * nbatch * n_pad * 32 + (size_t)WARPS_PER_BLOCK * 2 * n_pad + (size_t)n_pad) * sizeof(double);
+  if (tsmem <= 56 * 1024) return tsmem;
+  return 0;
+}
+
 // -----------------------------------------------------------------------------------------------
 // FP64 SIMT GEMM tile (64 x 64 outputs, K step 16, 256 threads, 4 x 4 per thread) used by the two
 // setup products: rotation (A = U', B = X, both K-contiguous) and kinship ((G-1/2)(G-1/2)').
@@ -160,13 +183,12 @@ __global__ void __launch_bounds__(128) weight_consts_kernel(const double* __rest
   __shared__ WcShared sh;
   const int k = blockIdx.x;
   const bool ols = (k == nk);
-  weight_consts_block(ols, ols ? 0.0 : h2_dev[k], lambda, C0, n, n_pad, c, wc.w + (int64_t)k * n_pad,
-                      wc.sw + (int64_t)k * n_pad, wc.Q + (int64_t)k * c * n_pad, wc.slw + k, wc.lds + k, flags, sh);
+  weight_consts_block(ols, ols ? 0.0 : h2_dev[k], lambda, C0, n, n_pad, c, weight_slot(wc, k, n_pad, c), flags, sh);
 }
 
-// The same with the rotation of the covariates folded in (n <= 128): every block rotates the c covariate columns itself
-// (one thread per output, k ascending: rotate_kernel's summation order, so C0 is bit-identical) instead of waiting for
-// a separate launch; the covariate rotation sat at the head of the marker-side critical path of every grid scan.
+// The same with the rotation of the covariates folded in (weight_consts_rot_applies): every block rotates the c
+// covariate columns itself (rotate_elem: C0 is bit-identical) instead of waiting for a separate launch; the covariate
+// rotation sat at the head of the marker-side critical path of every grid scan.
 __global__ void __launch_bounds__(128) weight_consts_rot_kernel(const double* __restrict__ h2_dev, int nk,
                                                                 const double* __restrict__ lambda,
                                                                 const double* __restrict__ U,
@@ -177,20 +199,14 @@ __global__ void __launch_bounds__(128) weight_consts_rot_kernel(const double* __
   __shared__ WcShared sh;
   for (int idx = threadIdx.x; idx < c * n_pad; idx += 128) {
     const int col = idx / n_pad, a = idx % n_pad;
-    double v = 0.0;
-    if (a < n) {
-      const double* u = U + (int64_t)a * n;
-      const double* x = Cov + (int64_t)col * n;
-      for (int b = 0; b < n; ++b) v = fma(u[b], x[b], v);
-    }
+    const double v = (a < n) ? rotate_elem(U, Cov + (int64_t)col * n, n, a) : 0.0;
     c_s[idx] = v;
     if (blockIdx.x == 0) C0_out[idx] = v;
   }
   __syncthreads();
   const int k = blockIdx.x;
   const bool ols = (k == nk);
-  weight_consts_block(ols, ols ? 0.0 : h2_dev[k], lambda, c_s, n, n_pad, c, wc.w + (int64_t)k * n_pad,
-                      wc.sw + (int64_t)k * n_pad, wc.Q + (int64_t)k * c * n_pad, wc.slw + k, wc.lds + k, flags, sh);
+  weight_consts_block(ols, ols ? 0.0 : h2_dev[k], lambda, c_s, n, n_pad, c, weight_slot(wc, k, n_pad, c), flags, sh);
 }
 
 // ell of wls / wls_multivar (src/wls.jl:72-92) from the weighted rss
@@ -207,6 +223,11 @@ __device__ __forceinline__ double null_loglik(double rss, double slw, double lds
   return ll;
 }
 
+// alt-grid weight of grid point k in the single-logarithm scan: e = exp(-2 (ell_k - max_k ell) / n)
+__device__ __forceinline__ double alt_e(double ll, double llmax, int n) {
+  return exp(-(ll - llmax) * (2.0 / (double)n));
+}
+
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK)
     trait_stats_kernel(const double* __restrict__ Y0, int64_t m, int n, int n_pad, int c, int nk, WeightConsts wc,
                        LikParams lik, const double* __restrict__ grid_dev, double* __restrict__ Yr,
@@ -219,31 +240,14 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK)
   double* yb = smem + (int64_t)wid * n_pad;
   for (int l = lane; l < n_pad; l += 32) yb[l] = Y0[j * n_pad + l];
   __syncwarp();
-  double coef[MAXC];
-  {
-    // unweighted residual on the covariates (slot nk: w = 1)
-    const double* sw1 = wc.sw + (int64_t)nk * n_pad;
-    const double* Qo = wc.Q + (int64_t)nk * c * n_pad;
-    proj_coefs(yb, sw1, Qo, n_pad, c, lane, coef);
-    for (int l = lane; l < n_pad; l += 32) {
-      const double y = proj_elem(yb, sw1, Qo, n_pad, c, l, coef);
-      yb[l] = y;
-      Yr[j * n_pad + l] = y;
-    }
-    __syncwarp();
-  }
+  // unweighted residual on the covariates (slot nk: w = 1)
+  unweighted_residual(yb, weight_slot(wc, nk, n_pad, c), n_pad, c, lane,
+                      [&](int l, double y) { Yr[j * n_pad + l] = y; });
   double bestv = -INFINITY;
   int bestk = 0;
   for (int k = 0; k < nk; ++k) {
-    const double* sw = wc.sw + (int64_t)k * n_pad;
-    const double* Q = wc.Q + (int64_t)k * c * n_pad;
-    proj_coefs(yb, sw, Q, n_pad, c, lane, coef);
-    double s = 0.0;
-    for (int l = lane; l < n_pad; l += 32) {
-      const double z = proj_elem(yb, sw, Q, n_pad, c, l, coef);
-      s = fma(z, z, s);
-    }
-    const double rss = warp_sum(s);
+    double coef[MAXC];
+    const double rss = proj_norm2(yb, weight_slot(wc, k, n_pad, c), n_pad, c, lane, coef);
     const double ll = null_loglik(rss, wc.slw[k], wc.lds[k], n, c, lik, nullptr);
     if (lane == 0) {
       ell[(int64_t)k + j * nk] = ll;
@@ -263,12 +267,13 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK)
   }
 }
 
-// Table form of trait_stats_kernel for problems whose weight tables fit in shared memory (every BXD-size
-// grid scan).  Lane v of a warp owns one (kind a, grid point k) pair: a = 0 accumulates sum_l w_k[l] y_l^2,
+// Table form of trait_stats_kernel for problems whose weight tables fit in shared memory (trait_table_smem; every
+// BXD-size grid scan).  Lane v of a warp owns one (kind a, grid point k) pair: a = 0 accumulates sum_l w_k[l] y_l^2,
 // a >= 1 accumulates t_ka = sum_l Q_ka[l] sw_k[l] y_l, in ONE pass over the trait with no cross-lane
 // reduction; then rss_k = s_k - sum_a t_ka^2 (Gram form on the trait already residualised without weights, so
 // nothing large cancels), and lane k evaluates the log-likelihood of grid point k.  The block's table
 // T[batch][l][32] (lane-contiguous: conflict-free) is built once and reused for every trait of the block.
+// With fuse.Top (a single batch), also the alt-grid operands: Top, e and et for j < tcol_pad.
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
     trait_stats_table_kernel(const double* __restrict__ Y0, int64_t m, int n, int n_pad, int c, int nk, WeightConsts wc,
                              LikParams lik, const double* __restrict__ grid_dev, double* __restrict__ Yr,
@@ -277,27 +282,16 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
                              TraitFuse fuse) {
   extern __shared__ double smem[];
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int KB = 32 / (1 + c);  // grid points per batch of 32 lane slots
-  const int nbatch = (nk + KB - 1) / KB;
+  const int KB = table_kb(c);
+  const int nbatch = table_batches(c, nk);
   double* T = smem;                                   // [nbatch][n_pad][32]
   double* ybase = smem + (size_t)nbatch * n_pad * 32;  // [WARPS_PER_BLOCK][2][n_pad]: residual and its square
-  for (int idx = threadIdx.x; idx < nbatch * n_pad * 32; idx += blockDim.x) {
-    const int v = idx & 31, l = (idx >> 5) % n_pad, bt = (idx >> 5) / n_pad;
-    const int a = v / KB, k = bt * KB + v % KB;
-    double val = 0.0;
-    if (a <= c && k < nk && l < n) {
-      const double sw = wc.sw[(int64_t)k * n_pad + l];
-      val = (a == 0) ? wc.w[(int64_t)k * n_pad + l] : wc.Q[((int64_t)k * c + (a - 1)) * n_pad + l] * sw;
-    }
-    T[idx] = val;
-  }
-  __syncthreads();
+  build_weight_table(wc, n, n_pad, c, nk, KB, nbatch, T, nullptr);
   const int a_lane = lane / KB, kk_lane = lane % KB;
   double* yb = ybase + (int64_t)wid * 2 * n_pad;
   double* yb2 = yb + n_pad;
   const double* src = (a_lane == 0) ? yb2 : yb;  // this lane's kind: a = 0 sums w y^2, a >= 1 sums (Q sw) y
-  const double* sw1 = wc.sw + (int64_t)nk * n_pad;
-  const double* Qo = wc.Q + (int64_t)nk * c * n_pad;
+  const WeightSlot ols = weight_slot(wc, nk, n_pad, c);  // slot nk: w = 1
   const int64_t jend = fuse.Top ? fuse.tcol_pad : m;
   for (int64_t j = (int64_t)blockIdx.x * WARPS_PER_BLOCK + wid; j < jend; j += (int64_t)gridDim.x * WARPS_PER_BLOCK) {
     if (j >= m) {
@@ -311,34 +305,16 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
     }
     for (int l = lane; l < n_pad; l += 32) yb[l] = Y0[j * n_pad + l];
     __syncwarp();
-    double coef[MAXC];
-    proj_coefs(yb, sw1, Qo, n_pad, c, lane, coef);  // unweighted residual on the covariates (slot nk: w = 1)
-    for (int l = lane; l < n_pad; l += 32) {
-      const double y = proj_elem(yb, sw1, Qo, n_pad, c, l, coef);  // reads only this lane's element of yb
-      yb[l] = y;
+    unweighted_residual(yb, ols, n_pad, c, lane, [&](int l, double y) {
       yb2[l] = y * y;
       Yr[j * n_pad + l] = y;
       if (fuse.Top) fuse.Top[((int64_t)(l / KC) * fuse.tcol_pad + j) * KC + (l % KC)] = y;
-    }
-    __syncwarp();
+    });
     double bestv = -INFINITY;
     int bestk = 0x7fffffff;
     double ll_mine = 0.0, rss_mine = 1.0;  // lane k's values (single batch), for the fused alt-grid scalars
     for (int bt = 0; bt < nbatch; ++bt) {
-      const double* Tb = T + (size_t)bt * n_pad * 32 + lane;
-      double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
-      int l = 0;
-      for (; l + 4 <= n; l += 4) {
-        s0 = fma(Tb[(l + 0) * 32], src[l + 0], s0);
-        s1 = fma(Tb[(l + 1) * 32], src[l + 1], s1);
-        s2 = fma(Tb[(l + 2) * 32], src[l + 2], s2);
-        s3 = fma(Tb[(l + 3) * 32], src[l + 3], s3);
-      }
-      for (; l < n; ++l) s0 = fma(Tb[l * 32], src[l], s0);
-      const double sv = (s0 + s1) + (s2 + s3);
-      double rss = sv;
-      const double t2 = sv * sv;
-      for (int a = 1; a <= c; ++a) rss -= __shfl_sync(0xffffffffu, t2, (a * KB + kk_lane) & 31);
+      const double rss = table_pass(T + (size_t)bt * n_pad * 32, src, n, c, KB, kk_lane, lane).red;
       const int k = bt * KB + kk_lane;
       const bool valid = (a_lane == 0) && (k < nk);
       const int kc = valid ? k : 0;
@@ -366,9 +342,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
       }
     }
     if (fuse.Top && lane < nk) {
-      // alt-grid scalars (launch_alt_scalars): e = exp(-2 (ell_k - max_k ell) / n), et = e / rss_k; one batch, so
-      // lane k still holds its own ell and rss
-      const double ev = exp(-(ll_mine - bestv) * (2.0 / (double)n));
+      // alt-grid scalars (as alt_scalars_kernel); one batch, so lane k still holds its own ell and rss
+      const double ev = alt_e(ll_mine, bestv, n);
       fuse.e[(int64_t)lane * fuse.tcol_pad + j] = ev;
       fuse.et[(int64_t)lane * fuse.tcol_pad + j] = ev / rss_mine;
     }
@@ -390,41 +365,32 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK)
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t i = (int64_t)blockIdx.x * WARPS_PER_BLOCK + wid;
   if (i >= p_pad) return;
-  const int nq = n_pad / KC;
   if (i >= p) {
-    for (int k = 0; k < nk; ++k)
-      for (int l = lane; l < n_pad; l += 32)
-        Mop[(((int64_t)k * nq + l / KC) * p_pad + i) * KC + (l % KC)] = 0.0;
+    zero_marker_column(Mop, i, p_pad, n_pad, nk, lane);
     return;
   }
+  const int nq = n_pad / KC;
   double* gb = smem + (int64_t)wid * n_pad;
   for (int l = lane; l < n_pad; l += 32) gb[l] = G0[i * n_pad + l];
   __syncwarp();
-  double coef[MAXC];
   for (int k = 0; k < nk; ++k) {
-    const double* sw = wc.sw + (int64_t)k * n_pad;
-    const double* Q = wc.Q + (int64_t)k * c * n_pad;
-    proj_coefs(gb, sw, Q, n_pad, c, lane, coef);
-    double s = 0.0;
-    for (int l = lane; l < n_pad; l += 32) {
-      const double z = proj_elem(gb, sw, Q, n_pad, c, l, coef);
-      s = fma(z, z, s);
-    }
-    const double nrm = sqrt(warp_sum(s));
+    const WeightSlot s = weight_slot(wc, k, n_pad, c);
+    double coef[MAXC];
+    const double nrm = sqrt(proj_norm2(gb, s, n_pad, c, lane, coef));
     if (lane == 0 && !(nrm > DBL_EPSILON)) atomicExch(&flags[FLAG_ZERO_NORM], 1);
     const double inv = 1.0 / nrm;
     for (int l = lane; l < n_pad; l += 32) {
-      const double z = proj_elem(gb, sw, Q, n_pad, c, l, coef);
-      Mop[(((int64_t)k * nq + l / KC) * p_pad + i) * KC + (l % KC)] = (fold_sw ? sw[l] * z : z) * inv;
+      const double z = proj_elem(gb, s.sw, s.Q, n_pad, c, l, coef);
+      Mop[(((int64_t)k * nq + l / KC) * p_pad + i) * KC + (l % KC)] = (fold_sw ? s.sw[l] * z : z) * inv;
     }
   }
 }
 
 // Table form of marker_operand_kernel for the weight-folded operand of the grid scans (fold_sw), when the
-// per-block tables fit in shared memory.  As in trait_stats_table_kernel lane v owns one (kind a, grid point k) pair
-// and gets s_k = sum_l w_k g_l^2 and t_ka = sum_l Q_ka sw_k g_l in one pass without cross-lane reductions
-// (||P_k(sw_k g)||^2 = s_k - sum_a t_ka^2; g is first residualised without weights on the covariates, which P_k
-// annihilates anyway, so nothing large cancels).  The second pass writes sw_k P_k(sw_k g) / ||.|| =
+// per-block tables fit in shared memory (marker_table_smem).  As in trait_stats_table_kernel lane v owns one (kind a,
+// grid point k) pair and gets s_k = sum_l w_k g_l^2 and t_ka = sum_l Q_ka sw_k g_l in one pass without cross-lane
+// reductions (||P_k(sw_k g)||^2 = s_k - sum_a t_ka^2; g is first residualised without weights on the covariates, which
+// P_k annihilates anyway, so nothing large cancels).  The second pass writes sw_k P_k(sw_k g) / ||.|| =
 // (w_k g - sum_a (Q_ka sw_k) t_ka) / ||.|| from the same table entries, read through a transposed copy so that
 // lanes walking along l do not collide on one bank.
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
@@ -432,8 +398,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
                                 WeightConsts wc, double* __restrict__ Mop, int* flags) {
   extern __shared__ double smem[];
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int KB = 32 / (1 + c);
-  const int nbatch = (nk + KB - 1) / KB;
+  const int KB = table_kb(c);
+  const int nbatch = table_batches(c, nk);
   const int nq = n_pad / KC;
   double* T = smem;                                       // [nbatch][n_pad][32]  (lane-contiguous)
   double* Tt = T + (size_t)nbatch * n_pad * 32;           // [nbatch][32][n_pad]  (l-contiguous)
@@ -441,56 +407,24 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
   // [n_pad] offset of element l inside one k-slab for marker 0: (l / KC) p_pad KC + l % KC (marker i adds i KC)
   int64_t* off_s = reinterpret_cast<int64_t*>(gbase + (size_t)WARPS_PER_BLOCK * 2 * n_pad);
   for (int l = threadIdx.x; l < n_pad; l += blockDim.x) off_s[l] = (int64_t)(l / KC) * p_pad * KC + (l % KC);
-  for (int idx = threadIdx.x; idx < nbatch * n_pad * 32; idx += blockDim.x) {
-    const int v = idx & 31, l = (idx >> 5) % n_pad, bt = (idx >> 5) / n_pad;
-    const int a = v / KB, k = bt * KB + v % KB;
-    double val = 0.0;
-    if (a <= c && k < nk && l < n) {
-      const double sw = wc.sw[(int64_t)k * n_pad + l];
-      val = (a == 0) ? wc.w[(int64_t)k * n_pad + l] : wc.Q[((int64_t)k * c + (a - 1)) * n_pad + l] * sw;
-    }
-    T[idx] = val;
-    Tt[((size_t)bt * 32 + v) * n_pad + l] = val;
-  }
-  __syncthreads();
+  build_weight_table(wc, n, n_pad, c, nk, KB, nbatch, T, Tt);
   const int a_lane = lane / KB, kk_lane = lane % KB;
   double* gb = gbase + (int64_t)wid * 2 * n_pad;
   double* gb2 = gb + n_pad;
   const double* src = (a_lane == 0) ? gb2 : gb;
-  const double* sw1 = wc.sw + (int64_t)nk * n_pad;
-  const double* Qo = wc.Q + (int64_t)nk * c * n_pad;
+  const WeightSlot ols = weight_slot(wc, nk, n_pad, c);  // slot nk: w = 1
   for (int64_t i = (int64_t)blockIdx.x * WARPS_PER_BLOCK + wid; i < p_pad; i += (int64_t)gridDim.x * WARPS_PER_BLOCK) {
     if (i >= p) {
-      for (int k = 0; k < nk; ++k)
-        for (int l = lane; l < n_pad; l += 32) Mop[(((int64_t)k * nq + l / KC) * p_pad + i) * KC + (l % KC)] = 0.0;
+      zero_marker_column(Mop, i, p_pad, n_pad, nk, lane);
       continue;
     }
     for (int l = lane; l < n_pad; l += 32) gb[l] = G0[i * n_pad + l];
     __syncwarp();
-    double coef[MAXC];
-    proj_coefs(gb, sw1, Qo, n_pad, c, lane, coef);
-    for (int l = lane; l < n_pad; l += 32) {
-      const double gv = proj_elem(gb, sw1, Qo, n_pad, c, l, coef);
-      gb[l] = gv;
-      gb2[l] = gv * gv;
-    }
-    __syncwarp();
+    unweighted_residual(gb, ols, n_pad, c, lane, [&](int l, double g) { gb2[l] = g * g; });
     for (int bt = 0; bt < nbatch; ++bt) {
-      const double* Tb = T + (size_t)bt * n_pad * 32 + lane;
-      double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
-      int l = 0;
-      for (; l + 4 <= n; l += 4) {
-        s0 = fma(Tb[(l + 0) * 32], src[l + 0], s0);
-        s1 = fma(Tb[(l + 1) * 32], src[l + 1], s1);
-        s2 = fma(Tb[(l + 2) * 32], src[l + 2], s2);
-        s3 = fma(Tb[(l + 3) * 32], src[l + 3], s3);
-      }
-      for (; l < n; ++l) s0 = fma(Tb[l * 32], src[l], s0);
-      const double sv = (s0 + s1) + (s2 + s3);  // lane (a, kk): a = 0 -> sum w g^2, a >= 1 -> t_a
-      double n2 = sv;
-      const double t2 = sv * sv;
-      for (int a = 1; a <= c; ++a) n2 -= __shfl_sync(0xffffffffu, t2, (a * KB + kk_lane) & 31);
-      const double nrm = sqrt(n2);
+      const TablePass tp = table_pass(T + (size_t)bt * n_pad * 32, src, n, c, KB, kk_lane, lane);
+      const double sv = tp.sv;  // lane (a, kk): a = 0 -> sum w g^2, a >= 1 -> t_a
+      const double nrm = sqrt(tp.red);
       const bool valid0 = (a_lane == 0) && (bt * KB + kk_lane < nk);
       if (valid0 && !(nrm > DBL_EPSILON)) atomicExch(&flags[FLAG_ZERO_NORM], 1);
       const double inv_mine = 1.0 / nrm;  // meaningful in lanes (0, kk)
@@ -520,9 +454,10 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 4)
   }
 }
 
+// alt-grid trait scalars: e[k][j] = alt_e(ell[k,j], ellmax_j), et = e / rss; pads e = 1, et = 0.
 __global__ void alt_scalars_kernel(const double* __restrict__ ell, const double* __restrict__ rss,
-                                   const double* __restrict__ ellmax, int64_t m, int64_t tcol_pad, int nk,
-                                   double inv_half_n, double* __restrict__ e, double* __restrict__ et) {
+                                   const double* __restrict__ ellmax, int64_t m, int64_t tcol_pad, int nk, int n,
+                                   double* __restrict__ e, double* __restrict__ et) {
   const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= tcol_pad) return;
   if (j >= m) {
@@ -534,7 +469,7 @@ __global__ void alt_scalars_kernel(const double* __restrict__ ell, const double*
   }
   const double emax = ellmax[j];
   for (int k = 0; k < nk; ++k) {
-    const double ev = exp(-(ell[(int64_t)k + j * nk] - emax) * inv_half_n);
+    const double ev = alt_e(ell[(int64_t)k + j * nk], emax, n);
     e[(int64_t)k * tcol_pad + j] = ev;
     et[(int64_t)k * tcol_pad + j] = ev / rss[(int64_t)k * m + j];
   }
@@ -616,17 +551,9 @@ __global__ void pack_perms_kernel(const double* __restrict__ z, const double* __
 __global__ void __launch_bounds__(32) null_residual_kernel(const double* __restrict__ Yr, int n, int n_pad, int c,
                                                            WeightConsts wc, double* __restrict__ z,
                                                            double* __restrict__ rss) {
-  const int lane = threadIdx.x;
   double coef[MAXC];
-  proj_coefs(Yr, wc.sw, wc.Q, n_pad, c, lane, coef);
-  double s = 0.0;
-  for (int l = lane; l < n_pad; l += 32) {
-    const double v = proj_elem(Yr, wc.sw, wc.Q, n_pad, c, l, coef);
-    z[l] = v;
-    s = fma(v, v, s);
-  }
-  s = warp_sum(s);
-  if (lane == 0) *rss = s;
+  const double s = proj_norm2(Yr, weight_slot(wc, 0, n_pad, c), n_pad, c, threadIdx.x, coef, z);
+  if (threadIdx.x == 0) *rss = s;
 }
 
 // -----------------------------------------------------------------------------------------------
@@ -755,72 +682,62 @@ int launch_weight_consts(const double* h2_dev, int nk, const double* lambda, con
   return 1;
 }
 
+// one thread per rotated covariate element, each a length-n dot product: worth folding in for small n only
+bool weight_consts_rot_applies(int n) { return n <= 128; }
+
 int launch_weight_consts_rot(const double* h2_dev, int nk, const double* lambda, const double* U, const double* Cov,
                              int n, int n_pad, int c, WeightConsts wc, double* C0, int* flags, cudaStream_t stream) {
-  if (n > 128) return 0;
   weight_consts_rot_kernel<<<nk + 1, 128, (size_t)c * n_pad * sizeof(double), stream>>>(h2_dev, nk, lambda, U, Cov, n,
                                                                                          n_pad, c, wc, C0, flags);
   return 1;
 }
 
+namespace {
+// Blocks of a table kernel over `cols` warp columns: one resident wave (4 blocks per SM by shared memory); fewer,
+// longer-lived blocks were measured slower, the kernels being bound by per-column latency, not by building the tables.
+// Raises the kernel's dynamic shared-memory limit when smem needs more than the default 48 KB.
+template <class Kernel>
+unsigned table_wave(Kernel* kernel, size_t smem, int64_t cols, int sm_count) {
+  if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  return (unsigned)std::min<int64_t>((cols + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, (int64_t)sm_count * 4);
+}
+}  // namespace
+
 int launch_trait_stats(const double* Y0, int64_t m, int n, int n_pad, int c, int nk, WeightConsts wc,
                        LikParams lik, const double* grid_dev, double* Yr, double* ell, double* rss,
-                       int* best, double* ellmax, double* h2_out, int* bin_count, int* flags,
-                       cudaStream_t stream, TraitFuse* fuse) {
-  if (fuse) fuse->done = false;
-  // table form when the block's weight table fits in shared memory (BXD-size grid scans: 20 KB)
-  const int KB = 32 / (1 + c);
-  const int nbatch = (nk + KB - 1) / KB;
-  const size_t table_smem = ((size_t)nbatch * n_pad * 32 + (size_t)WARPS_PER_BLOCK * 2 * n_pad) * sizeof(double);
-  if (table_smem <= 96 * 1024) {
-    if (table_smem > 48 * 1024)
-      cudaFuncSetAttribute(trait_stats_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)table_smem);
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    TraitFuse f{nullptr, nullptr, nullptr, 0, false};
-    if (fuse && nbatch == 1 && fuse->Top && fuse->e && fuse->et) {
-      f = *fuse;
-      fuse->done = true;
-    }
-    const int64_t cols = f.Top ? f.tcol_pad : m;
-    const int64_t want = (cols + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-    const unsigned blocks = (unsigned)std::min<int64_t>(want, (int64_t)sms * 4);  // one resident wave
-    trait_stats_table_kernel<<<blocks, 32 * WARPS_PER_BLOCK, table_smem, stream>>>(
-        Y0, m, n, n_pad, c, nk, wc, lik, grid_dev, Yr, ell, rss, best, ellmax, h2_out, bin_count, flags, f);
-    return 1;
+                       int* best, double* ellmax, double* h2_out, int* bin_count, int* flags, const TraitFuse* fuse,
+                       int sm_count, cudaStream_t stream) {
+  const size_t table_smem = trait_table_smem(n_pad, c, nk);
+  bool fused = false;
+  if (table_smem) {
+    // with one lane batch, lane k holds grid point k's ell and rss at the end: the alt-grid operands come for free
+    const TraitFuse f = (fuse && table_batches(c, nk) == 1) ? *fuse : TraitFuse{};
+    fused = f.Top != nullptr;
+    const int64_t cols = fused ? f.tcol_pad : m;
+    trait_stats_table_kernel<<<table_wave(trait_stats_table_kernel, table_smem, cols, sm_count), 32 * WARPS_PER_BLOCK,
+                               table_smem, stream>>>(Y0, m, n, n_pad, c, nk, wc, lik, grid_dev, Yr, ell, rss, best,
+                                                     ellmax, h2_out, bin_count, flags, f);
+  } else {
+    const size_t smem = (size_t)WARPS_PER_BLOCK * n_pad * sizeof(double);
+    if (smem > 48 * 1024)
+      cudaFuncSetAttribute(trait_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const unsigned blocks = (unsigned)((m + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
+    trait_stats_kernel<<<blocks, 32 * WARPS_PER_BLOCK, smem, stream>>>(Y0, m, n, n_pad, c, nk, wc, lik, grid_dev, Yr,
+                                                                        ell, rss, best, ellmax, h2_out, bin_count,
+                                                                        flags);
   }
-  const size_t smem = (size_t)WARPS_PER_BLOCK * n_pad * sizeof(double);
-  if (smem > 48 * 1024)
-    cudaFuncSetAttribute(trait_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  const unsigned blocks = (unsigned)((m + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
-  trait_stats_kernel<<<blocks, 32 * WARPS_PER_BLOCK, smem, stream>>>(Y0, m, n, n_pad, c, nk, wc, lik, grid_dev, Yr,
-                                                                      ell, rss, best, ellmax, h2_out, bin_count,
-                                                                      flags);
-  return 1;
+  if (!fuse || fused) return 1;
+  alt_scalars_kernel<<<(unsigned)((fuse->tcol_pad + 255) / 256), 256, 0, stream>>>(ell, rss, ellmax, m, fuse->tcol_pad,
+                                                                                   nk, n, fuse->e, fuse->et);
+  return 2 + launch_pack_traits(Yr, nullptr, m, fuse->tcol_pad, n_pad, nullptr, fuse->Top, stream);
 }
 
 int launch_marker_operand(const double* G0, int64_t p, int64_t p_pad, int n, int n_pad, int c, int nk,
-                          WeightConsts wc, bool fold_sw, double* Mop, int* flags, cudaStream_t stream) {
-  if (fold_sw) {
-    // table form when the block's tables fit in shared memory (BXD-size grid scans: 50 KB)
-    const int KB = 32 / (1 + c);
-    const int nbatch = (nk + KB - 1) / KB;
-    const size_t tsmem = ((size_t)2 * nbatch * n_pad * 32 + (size_t)WARPS_PER_BLOCK * 2 * n_pad + (size_t)n_pad) * sizeof(double);
-    if (tsmem <= 56 * 1024) {
-      if (tsmem > 48 * 1024)
-        cudaFuncSetAttribute(marker_operand_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsmem);
-      int dev = 0, sms = 148;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      // one resident wave (4 blocks per SM by shared memory); fewer, longer-lived blocks were measured slower —
-      // the kernel is bound by per-marker latency, not by building the tables
-      const int64_t want = (p_pad + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-      const unsigned blocks = (unsigned)std::min<int64_t>(want, (int64_t)sms * 4);
-      marker_operand_table_kernel<<<blocks, 32 * WARPS_PER_BLOCK, tsmem, stream>>>(G0, p, p_pad, n, n_pad, c, nk, wc, Mop,
-                                                                                    flags);
-      return 1;
-    }
+                          WeightConsts wc, bool fold_sw, double* Mop, int* flags, int sm_count, cudaStream_t stream) {
+  if (const size_t tsmem = fold_sw ? marker_table_smem(n_pad, c, nk) : 0) {
+    marker_operand_table_kernel<<<table_wave(marker_operand_table_kernel, tsmem, p_pad, sm_count), 32 * WARPS_PER_BLOCK,
+                                  tsmem, stream>>>(G0, p, p_pad, n, n_pad, c, nk, wc, Mop, flags);
+    return 1;
   }
   const size_t smem = (size_t)WARPS_PER_BLOCK * n_pad * sizeof(double);
   if (smem > 48 * 1024)
@@ -828,13 +745,6 @@ int launch_marker_operand(const double* G0, int64_t p, int64_t p_pad, int n, int
   const unsigned blocks = (unsigned)((p_pad + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
   marker_operand_kernel<<<blocks, 32 * WARPS_PER_BLOCK, smem, stream>>>(G0, p, p_pad, n, n_pad, c, nk, wc,
                                                                          fold_sw ? 1 : 0, Mop, flags);
-  return 1;
-}
-
-int launch_alt_scalars(const double* ell, const double* rss, const double* ellmax, int64_t m,
-                       int64_t tcol_pad, int nk, int n, double* e, double* et, cudaStream_t stream) {
-  alt_scalars_kernel<<<(unsigned)((tcol_pad + 255) / 256), 256, 0, stream>>>(ell, rss, ellmax, m, tcol_pad, nk,
-                                                                              2.0 / (double)n, e, et);
   return 1;
 }
 

@@ -497,36 +497,21 @@ bool stream_unsupported(const ScanParams& P) { return P.et_folded || P.H2idx || 
 
 }  // namespace
 
-int stream_exact_marker_tile(int c) { return (c + 2 <= 5) ? 64 : 32; }
-
 int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* C0, int64_t m,
                          int64_t slots, int n, int n_pad, int c, double* Xop, int64_t xcol_pad, double* dyinv,
                          int* flags, cudaStream_t stream) {
   const unsigned blocks = (unsigned)((slots + 7) / 8);
-#define BLMM_EXCOL(C) \
-  case C: exact_columns_kernel<C><<<blocks, 256, 0, stream>>>(Yr, h2, lambda, C0, m, slots, n, n_pad, Xop, xcol_pad, dyinv, flags); break;
-  switch (c) {
-    BLMM_EXCOL(1) BLMM_EXCOL(2) BLMM_EXCOL(3) BLMM_EXCOL(4) BLMM_EXCOL(5) BLMM_EXCOL(6) BLMM_EXCOL(7) BLMM_EXCOL(8)
-    default: return 0;
-  }
-#undef BLMM_EXCOL
-  return 1;
+  return dispatch_c<1, MAXC>(c, [&](auto C) {
+    exact_columns_kernel<C><<<blocks, 256, 0, stream>>>(Yr, h2, lambda, C0, m, slots, n, n_pad, Xop, xcol_pad, dyinv,
+                                                        flags);
+  });
 }
 
 int launch_scan_exact(const ScanParams& P, int c, int sm_count, cudaStream_t stream) {
   if (stream_unsupported(P)) return 0;
-  switch (c + 2) {
-    case 3: launch_stream_one<3, 4, MODE_EXACT>(P, sm_count, stream); break;
-    case 4: launch_stream_one<4, 4, MODE_EXACT>(P, sm_count, stream); break;
-    case 5: launch_stream_one<5, 4, MODE_EXACT>(P, sm_count, stream); break;
-    case 6: launch_stream_one<6, 2, MODE_EXACT>(P, sm_count, stream); break;
-    case 7: launch_stream_one<7, 2, MODE_EXACT>(P, sm_count, stream); break;
-    case 8: launch_stream_one<8, 2, MODE_EXACT>(P, sm_count, stream); break;
-    case 9: launch_stream_one<9, 2, MODE_EXACT>(P, sm_count, stream); break;
-    case 10: launch_stream_one<10, 2, MODE_EXACT>(P, sm_count, stream); break;
-    default: return 0;
-  }
-  return 1;
+  return dispatch_c<1, MAXC>(c, [&](auto C) {
+    launch_stream_one<C + 2, exact_marker_atoms(C), MODE_EXACT>(P, sm_count, stream);  // NB = the c + 2 column kinds
+  });
 }
 
 int launch_scan_stream_grid(const ScanParams& P, int sm_count, cudaStream_t stream) {
