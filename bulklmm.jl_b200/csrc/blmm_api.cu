@@ -650,8 +650,9 @@ int fit_h2(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* h2
   rotate_covariates(ctx, R, ctx->stream);
   rotate_traits(ctx, pr, R, ms);
   double* Yr = residualised_traits(ctx, R, o);
-  ctx->launches += launch_fit_h2(Yr, m, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2, el,
-                                 ctx->d_flags, ctx->stream);
+  const WeightConsts ols = weight_ws(ctx, 0, R.n_pad, R.c);  // the w = 1 constants residualised_traits left
+  ctx->launches += launch_fit_h2(Yr, m, R.n, R.n_pad, R.c, ols.Q, ols.lds, R.lambda, lik_of(o), o->optim_interval, h2,
+                                 s2, el, ctx->d_flags, ctx->stream);
   out.deliver();
   return BLMM_OK;
 }
@@ -684,12 +685,12 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   rotate_traits(ctx, pr, R, ms);
   rotate_markers_aside(ctx, pr, R, ms);
   double* Yr = residualised_traits(ctx, R, o);  // also leaves the w = 1 constants in weight slot 0
-  ctx->launches += launch_fit_h2(Yr, m, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2,
-                                 nullptr, ctx->d_flags, ctx->stream);
+  WeightConsts wc0 = weight_ws(ctx, 0, R.n_pad, R.c);
+  ctx->launches += launch_fit_h2(Yr, m, R.n, R.n_pad, R.c, wc0.Q, wc0.lds, R.lambda, lik_of(o), o->optim_interval, h2,
+                                 s2, nullptr, ctx->d_flags, ctx->stream);
   // markers residualised (unweighted) on the covariates and normalised: r^2 is invariant to both
   const int mt = stream_exact_marker_tile(R.c);
   const int64_t p_pad = round_up(p, mt);
-  WeightConsts wc0 = weight_ws(ctx, 0, R.n_pad, R.c);
   double* Mop = ws<double>(ctx, S_MOP, (size_t)R.n_pad * p_pad);
   wait_markers(ctx, ctx->stream);  // U'G was computed on the third stream meanwhile
   ctx->launches += launch_marker_operand(R.G0, p, p_pad, R.n, R.n_pad, R.c, 1, wc0, false, Mop, ctx->d_flags,
@@ -700,7 +701,7 @@ int bulkscan_exact(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, do
   const int64_t xcol_pad = slots * cg;
   double* Xop = ws<double>(ctx, S_XOP, (size_t)R.n_pad * xcol_pad);
   double* dyinv = ws<double>(ctx, S_DYINV, slots);
-  ctx->launches += launch_exact_columns(Yr, h2, R.lambda, R.C0, m, slots, R.n, R.n_pad, R.c, Xop, xcol_pad, dyinv,
+  ctx->launches += launch_exact_columns(Yr, h2, R.lambda, wc0.Q, m, slots, R.n, R.n_pad, R.c, Xop, xcol_pad, dyinv,
                                         ctx->d_flags, ctx->stream);
   ScanParams P{};
   P.Mop = Mop;
@@ -758,11 +759,12 @@ int scan_alt(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, double* 
   rotate_traits(ctx, pr, R, o->mem_space);
   rotate_markers_aside(ctx, pr, R, o->mem_space);
   double* Yr = residualised_traits(ctx, R, o);
+  const WeightConsts ols = weight_ws(ctx, 0, R.n_pad, R.c);  // the w = 1 constants residualised_traits left
   double* misc = ws<double>(ctx, S_MISC, 8);  // [0] h2_null, [1] sigma2, [2] ell_null
-  ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, misc, misc + 1,
-                                 nullptr, ctx->d_flags, ctx->stream);
+  ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, ols.Q, ols.lds, R.lambda, lik_of(o), o->optim_interval, misc,
+                                 misc + 1, nullptr, ctx->d_flags, ctx->stream);
   wait_markers(ctx, ctx->stream);  // U'G was computed on the third stream meanwhile
-  const int launched = launch_scan_alt(Yr, R.G0, p, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval,
+  const int launched = launch_scan_alt(Yr, R.G0, p, R.n, R.n_pad, R.c, ols.Q, ols.lds, R.lambda, lik_of(o), o->optim_interval,
                                        misc, misc + 2, dlod, dh2, ctx->stream);
   if (!launched) throw Fail{BLMM_E_INVALID, "unsupported covariate count"};
   ctx->launches += launched;
@@ -809,8 +811,9 @@ int scan_perms(blmm_ctx* ctx, const blmm_problem* pr, const blmm_opts* o, const 
     rotate_traits(ctx, pr, R, ms);
     rotate_markers_aside(ctx, pr, R, ms);
     double* Yr = residualised_traits(ctx, R, o);
-    ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, R.C0, R.lambda, lik_of(o), o->optim_interval, h2, s2,
-                                   nullptr, ctx->d_flags, ctx->stream);
+    const WeightConsts ols = weight_ws(ctx, 0, R.n_pad, R.c);  // read by the fit before slot 0 is reused below
+    ctx->launches += launch_fit_h2(Yr, 1, R.n, R.n_pad, R.c, ols.Q, ols.lds, R.lambda, lik_of(o), o->optim_interval, h2,
+                                   s2, nullptr, ctx->d_flags, ctx->stream);
     // transform_reweight at the fitted h2 (weight slot 0)
     ctx->launches += launch_weight_consts(h2, 1, R.lambda, R.C0, R.n, R.n_pad, R.c, wc, ctx->d_flags, ctx->stream);
     ctx->launches += launch_null_residual(Yr, R.n, R.n_pad, R.c, wc, z, zrss, ctx->stream);

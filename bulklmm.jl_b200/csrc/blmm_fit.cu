@@ -5,6 +5,7 @@
 // butterfly reduction is symmetric), so the Brent control flow is warp-uniform.
 #include <float.h>
 #include <math.h>
+#include <stdlib.h>
 
 #include "blmm_kernels.cuh"
 #include "blmm_prep_dev.cuh"
@@ -51,7 +52,8 @@ __device__ __forceinline__ double fit_ln(double v, const double2* __restrict__ t
 
 struct FitData {
   const double* y;       // trait (residualised on C0, padded), length n_pad
-  const double* C0;      // [c][n_pad]
+  const double* Qc;      // [c][n_pad] orthonormal basis of the covariates: C0 = Qc R (the w = 1 weight slot)
+  double ld_r;           // log det(C0'C0) = log det(R'R): REML's log det(C0'WC0) = log det(Qc'WQc) + ld_r
   const double* lambda;  // [n]
   int n, n_pad, c, lane;
   LikParams lik;
@@ -67,7 +69,10 @@ __device__ __forceinline__ double fit_inv_denom(const LikParams& lik, int n, int
 }
 
 // -ell(h2) and sigma2.  The covariate projection uses the Gram form S = C'WC, t = C'Wy,
-// rss = y'Wy - t'S^-1 t, log det S = 2 log|det R|, evaluated in one pass over the n weights.
+// rss = y'Wy - t'S^-1 t, log det S = 2 log|det R|, evaluated in one pass over the n weights.  C is the orthonormal
+// basis Qc (and, for scan_alt, the marker column), not C0: the projection is the same, but the Gram matrix of C0 would
+// be conditioned as kappa(C0)^2 (1e10 for two near-collinear covariates, ell then off by ~1e-8 relative), that of Qc
+// only by the spread of the weights.
 template <int C, int UNR = 4>
 __device__ double neg_loglik_c(const FitData& d, double h2, double* sigma2_out) {
   constexpr int NT = C * (C + 1) / 2;
@@ -100,7 +105,7 @@ __device__ double neg_loglik_c(const FitData& d, double h2, double* sigma2_out) 
     yy = fma(wy, y, yy);
     double cv[C];
 #pragma unroll
-    for (int a = 0; a < C; ++a) cv[a] = (a == C - 1 && d.xcol) ? d.xcol[l] : d.C0[(int64_t)a * d.n_pad + l];
+    for (int a = 0; a < C; ++a) cv[a] = (a == C - 1 && d.xcol) ? d.xcol[l] : d.Qc[(int64_t)a * d.n_pad + l];
     int idx = 0;
 #pragma unroll
     for (int a = 0; a < C; ++a) {
@@ -163,7 +168,7 @@ __device__ double neg_loglik_c(const FitData& d, double h2, double* sigma2_out) 
   // (rss + ab) / sigma2 is `denom` up to the rounding of the division that made sigma2; the reference evaluates the
   // quotient (src/wls.jl:84), so it is evaluated here too
   double ll = -0.5 * (((double)d.n + b) * log_s2 - slw + (rss + ab) * fast_rcp(sigma2));
-  if (d.lik.reml) ll += 0.5 * ((double)C * log_s2 - lds);
+  if (d.lik.reml) ll += 0.5 * ((double)C * log_s2 - (lds + d.ld_r));
   if (sigma2_out) *sigma2_out = sigma2;
   return -ll;
 }
@@ -253,8 +258,8 @@ __device__ double fit_one(const FitData& d, int optim_interval) {
 // traits: the null fit of scan / permutations) nothing hides it and the registers are better spent on no spills.
 template <int C, bool BULK>
 __global__ void __launch_bounds__(32 * FIT_WARPS, BULK ? (C <= 2 ? 8 : (C <= 4 ? 4 : 2)) : 1)
-    fit_h2_kernel(const double* __restrict__ Yr, int64_t m, int n, int n_pad, int c, const double* __restrict__ C0,
-                  const double* __restrict__ lambda, LikParams lik, int optim_interval, double* __restrict__ h2_out,
+    fit_h2_kernel(const double* __restrict__ Yr, int64_t m, int n, int n_pad, int c, const double* __restrict__ Qc,
+                  const double* __restrict__ ld_r, const double* __restrict__ lambda, LikParams lik, int optim_interval, double* __restrict__ h2_out,
                   double* __restrict__ sigma2_out, double* __restrict__ ell_out, int staged) {
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t j = (int64_t)blockIdx.x * FIT_WARPS + wid;
@@ -271,15 +276,15 @@ __global__ void __launch_bounds__(32 * FIT_WARPS, BULK ? (C <= 2 ? 8 : (C <= 4 ?
     double* c_s = lam_s + n_pad;
     double* y_s = c_s + (int64_t)C * n_pad + (int64_t)wid * n_pad;
     for (int l = threadIdx.x; l < n_pad; l += blockDim.x) lam_s[l] = (l < n) ? lambda[l] : 0.0;
-    for (int l = threadIdx.x; l < C * n_pad; l += blockDim.x) c_s[l] = C0[l];
+    for (int l = threadIdx.x; l < C * n_pad; l += blockDim.x) c_s[l] = Qc[l];
     for (int l = lane; l < n_pad; l += 32) y_s[l] = yv[l];
     __syncthreads();
     lambda = lam_s;
-    C0 = c_s;
+    Qc = c_s;
     yv = y_s;
   }
   if (j >= m) return;
-  FitData d{yv, C0, lambda, n, n_pad, c, lane, lik, nullptr, false, ltab, fit_inv_denom(lik, n, C)};
+  FitData d{yv, Qc, *ld_r, lambda, n, n_pad, c, lane, lik, nullptr, false, ltab, fit_inv_denom(lik, n, C)};
   const double bx = fit_one<C, BULK ? 1 : 4>(d, optim_interval);
   double s2;
   const double f = neg_loglik_c<C, BULK ? 1 : 4>(d, bx, &s2);
@@ -297,7 +302,7 @@ __global__ void __launch_bounds__(32 * FIT_WARPS, BULK ? (C <= 2 ? 8 : (C <= 4 ?
 template <int C>
 __global__ void __launch_bounds__(32 * FIT_WARPS, C <= 2 ? 8 : (C <= 4 ? 4 : 2))
     scan_alt_kernel(const double* __restrict__ y, const double* __restrict__ G0, int64_t p, int n, int n_pad,
-                    const double* __restrict__ C0, const double* __restrict__ lambda, LikParams lik,
+                    const double* __restrict__ Qc, const double* __restrict__ ld_r, const double* __restrict__ lambda, LikParams lik,
                     int optim_interval, const double* __restrict__ ell_null, double* __restrict__ lod,
                     double* __restrict__ h2_each) {
   __shared__ double2 ltab[FIT_LTAB];
@@ -306,7 +311,7 @@ __global__ void __launch_bounds__(32 * FIT_WARPS, C <= 2 ? 8 : (C <= 4 ? 4 : 2))
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t i = (int64_t)blockIdx.x * FIT_WARPS + wid;
   if (i >= p) return;
-  FitData d{y, C0, lambda, n, n_pad, C, lane, lik, G0 + i * n_pad, false, ltab, fit_inv_denom(lik, n, C)};
+  FitData d{y, Qc, *ld_r, lambda, n, n_pad, C, lane, lik, G0 + i * n_pad, false, ltab, fit_inv_denom(lik, n, C)};
   const double h2 = fit_one<C>(d, optim_interval);
   d.sqrt_weights = true;
   d.lik.reml = 0;
@@ -320,14 +325,14 @@ __global__ void __launch_bounds__(32 * FIT_WARPS, C <= 2 ? 8 : (C <= 4 ? 4 : 2))
 
 // ell_null of scan_alt: wls(y0, X0_covar, sqrt(w(h2_null)), prior).ell, one warp
 template <int C>
-__global__ void scan_alt_null_kernel(const double* __restrict__ y, int n, int n_pad, const double* __restrict__ C0,
+__global__ void scan_alt_null_kernel(const double* __restrict__ y, int n, int n_pad, const double* __restrict__ Qc,
                                      const double* __restrict__ lambda, LikParams lik,
                                      const double* __restrict__ h2_null, double* __restrict__ ell_null) {
   __shared__ double2 ltab[FIT_LTAB];
   fit_build_ln_table(ltab, threadIdx.x, blockDim.x);
   __syncthreads();
   lik.reml = 0;
-  FitData d{y, C0, lambda, n, n_pad, C, (int)(threadIdx.x & 31), lik, nullptr, true, ltab, fit_inv_denom(lik, n, C)};
+  FitData d{y, Qc, 0.0, lambda, n, n_pad, C, (int)(threadIdx.x & 31), lik, nullptr, true, ltab, fit_inv_denom(lik, n, C)};
   const double e = -neg_loglik_c<C>(d, h2_null[0], nullptr);
   if (threadIdx.x == 0) ell_null[0] = e;
 }
@@ -353,6 +358,7 @@ __global__ void __launch_bounds__(128, 1)
   double* lam_s = cs + 2 * FIT_LTAB;               // [n_pad]
   double* c_s = lam_s + n_pad;                     // [C][n_pad]  rotated covariates
   double* y_s = c_s + (int64_t)C * n_pad;          // [n_pad]     rotated, then residualised trait
+  double* q_s = y_s + n_pad;                       // [C][n_pad]  orthonormal basis of the rotated covariates
   __shared__ WcShared sh;
   __shared__ double h2_s;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -375,9 +381,11 @@ __global__ void __launch_bounds__(128, 1)
   // unweighted basis of the covariates (slot 1 of wc: w = 1), then Yr = y0 - Q Q'y0
   const WeightSlot ols = weight_slot(wc, 1, n_pad, C);
   weight_consts_block(true, 0.0, lam_s, c_s, n, n_pad, C, ols, flags, sh);
+  for (int l = tid; l < C * n_pad; l += 128) q_s[l] = ols.Q[l];
+  __syncthreads();
   if (warp == 0) {
     unweighted_residual(y_s, ols, n_pad, C, lane, [&](int l, double v) { Yr_out[l] = v; });
-    FitData d{y_s, c_s, lam_s, n, n_pad, C, lane, lik, nullptr, false, ltab, fit_inv_denom(lik, n, C)};
+    FitData d{y_s, q_s, *ols.lds, lam_s, n, n_pad, C, lane, lik, nullptr, false, ltab, fit_inv_denom(lik, n, C)};
     const double h2 = fit_one<C>(d, optim_interval);
     double s2;
     neg_loglik_c<C>(d, h2, &s2);
@@ -401,32 +409,33 @@ __global__ void __launch_bounds__(128, 1)
 }  // namespace
 
 // one block rotates y and the covariates with one thread per output, each a length-n dot product: small n only (then
-// the shared memory, 2 FIT_LTAB + (2 + c) n_pad doubles, is under 20 KB for every c <= MAXC)
+// the shared memory, 2 FIT_LTAB + (2 + 2 c) n_pad doubles, is under 30 KB for every c <= MAXC)
 bool null_fit_chain_applies(int n) { return n <= 128; }
 
 int launch_null_fit_chain(const double* U, const double* y, const double* Cov, const double* lambda, int n, int n_pad,
                           int c, LikParams lik, int optim_interval, double* C0, double* Yr, WeightConsts wc, double* h2,
                           double* sigma2, double* z, double* zrss, int* flags, cudaStream_t stream) {
-  const size_t smem = ((size_t)2 * FIT_LTAB + (size_t)(2 + c) * n_pad) * sizeof(double);
+  const size_t smem = ((size_t)2 * FIT_LTAB + (size_t)(2 + 2 * c) * n_pad) * sizeof(double);
   return dispatch_c<1, MAXC>(c, [&](auto C) {
     null_fit_chain_kernel<C><<<1, 128, smem, stream>>>(U, y, Cov, lambda, n, n_pad, lik, optim_interval, C0, Yr, wc, h2,
                                                        sigma2, z, zrss, flags);
   });
 }
 
-int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_pad, int c, const double* C0,
-                    const double* lambda, LikParams lik, int optim_interval, const double* h2_null, double* ell_null,
+int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_pad, int c, const double* Qc,
+                    const double* ld_r, const double* lambda, LikParams lik, int optim_interval, const double* h2_null, double* ell_null,
                     double* lod, double* h2_each, cudaStream_t stream) {
   const unsigned blocks = (unsigned)((p + FIT_WARPS - 1) / FIT_WARPS);
   const bool ok = dispatch_c<1, MAXC - 1>(c, [&](auto C) {
-    scan_alt_null_kernel<C><<<1, 32, 0, stream>>>(y, n, n_pad, C0, lambda, lik, h2_null, ell_null);
-    scan_alt_kernel<C + 1><<<blocks, 32 * FIT_WARPS, 0, stream>>>(y, G0, p, n, n_pad, C0, lambda, lik, optim_interval,
+    scan_alt_null_kernel<C><<<1, 32, 0, stream>>>(y, n, n_pad, Qc, lambda, lik, h2_null, ell_null);
+    scan_alt_kernel<C + 1><<<blocks, 32 * FIT_WARPS, 0, stream>>>(y, G0, p, n, n_pad, Qc, ld_r, lambda, lik,
+                                                                  optim_interval,
                                                                   ell_null, lod, h2_each);
   });
   return ok ? 2 : 0;
 }
 
-int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const double* C0,
+int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const double* Qc, const double* ld_r,
                   const double* lambda, LikParams lik, int optim_interval, double* h2, double* sigma2,
                   double* ell, int* flags, cudaStream_t stream) {
   (void)flags;
@@ -434,12 +443,13 @@ int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const do
   const size_t tab_bytes = (size_t)FIT_LTAB * sizeof(double2);
   size_t smem = tab_bytes + (size_t)(1 + c + FIT_WARPS) * n_pad * sizeof(double);
   const int staged = smem <= 96 * 1024 ? 1 : 0;
-  if (!staged) smem = tab_bytes;
+  const int stage = staged && !getenv("BLMM_B200_FIT_UNSTAGED");  // test hook: force the unstaged kernel
+  if (!stage) smem = tab_bytes;
   const bool bulk = blocks > 148 * 4;
   auto launch = [&](auto kernel) {
     if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kernel<<<blocks, 32 * FIT_WARPS, smem, stream>>>(Yr, m, n, n_pad, c, C0, lambda, lik, optim_interval, h2, sigma2,
-                                                     ell, staged);
+    kernel<<<blocks, 32 * FIT_WARPS, smem, stream>>>(Yr, m, n, n_pad, c, Qc, ld_r, lambda, lik, optim_interval, h2, sigma2,
+                                                     ell, stage);
   };
   return dispatch_c<1, MAXC>(c, [&](auto C) {
     if (bulk)

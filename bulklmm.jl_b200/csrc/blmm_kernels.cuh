@@ -124,7 +124,9 @@ int launch_null_residual(const double* Yr, int n, int n_pad, int c, WeightConsts
 // ---- heritability fit (blmm_fit.cu) -----------------------------------------------------------
 // fitlmm per trait: gridbrent over [0,1] in optim_interval pieces (src/lmm.jl:56-86,
 // src/gridbrent.jl:9-24, Optim.jl Brent).  One warp per trait.  Outputs length m (nullable).
-int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const double* C0,
+// Qc, ld_r: the w = 1 weight slot's orthonormal covariate basis (C0 = Qc R) and log det(C0'C0) = log det(R'R) (device
+// scalar), which turns REML's log det(Qc'WQc) into log det(C0'WC0).
+int launch_fit_h2(const double* Yr, int64_t m, int n, int n_pad, int c, const double* Qc, const double* ld_r,
                   const double* lambda, LikParams lik, int optim_interval, double* h2, double* sigma2,
                   double* ell, int* flags, cudaStream_t stream);
 
@@ -139,9 +141,9 @@ int launch_null_fit_chain(const double* U, const double* y, const double* Cov, c
 
 // scan_alt (src/scan.jl:397-453) for ONE trait y (residualised, padded): per-marker Brent with covariates
 // [C0 g_i] (c + 1 <= MAXC columns), lod_i = (ell_alt_i - ell_null) / ln 10, h2_each[i] (nullable).
-// h2_null: device scalar from launch_fit_h2; ell_null: device scalar workspace.
-int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_pad, int c, const double* C0,
-                    const double* lambda, LikParams lik, int optim_interval, const double* h2_null, double* ell_null,
+// h2_null: device scalar from launch_fit_h2; ell_null: device scalar workspace; Qc, ld_r as for launch_fit_h2.
+int launch_scan_alt(const double* y, const double* G0, int64_t p, int n, int n_pad, int c, const double* Qc,
+                    const double* ld_r, const double* lambda, LikParams lik, int optim_interval, const double* h2_null, double* ell_null,
                     double* lod, double* h2_each, cudaStream_t stream);
 
 // ---- the scans (blmm_scan.cu, blmm_scan_stream.cu) -----------------------------------------------
@@ -206,8 +208,9 @@ int launch_scan_stream_grid(const ScanParams& P, int sm_count, cudaStream_t stre
 // marker atoms (8 markers each, per warp) of the EXACT kernel for c covariates: its c + 2 operand kinds take registers
 constexpr int exact_marker_atoms(int c) { return c + 2 <= 5 ? 4 : 2; }
 constexpr int stream_exact_marker_tile(int c) { return 2 * 8 * exact_marker_atoms(c); }  // markers per CTA tile
-// z_j, q_j1..q_jc, w_j columns and 1/dy_j of every trait at its own h2 (slots = n_tt*64 >= m)
-int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* C0, int64_t m,
+// z_j, q_j1..q_jc, w_j columns and 1/dy_j of every trait at its own h2 (slots = n_tt*64 >= m); Qc: the unweighted
+// orthonormal covariate basis (the w = 1 weight slot)
+int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* Qc, int64_t m,
                          int64_t slots, int n, int n_pad, int c, double* Xop, int64_t xcol_pad, double* dyinv,
                          int* flags, cudaStream_t stream);
 int launch_scan_exact(const ScanParams& P, int c, int sm_count, cudaStream_t stream);

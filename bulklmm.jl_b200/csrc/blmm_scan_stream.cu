@@ -15,7 +15,8 @@
 // marker operand cannot carry them; instead trait j contributes c+2 columns against the
 // un-weighted rotated markers g_i (SURVEY appendix A5):
 //     num = g'z_j,  t_a = g'q_ja (a = 1..c),  s = (g o g)'w_j,   r^2 = num^2 / ((s - sum t_a^2) dy_j)
-// with W_j = diag(w_j), C0'W_jC0 = LL', Q_j = W_j C0 L^-T, z_j = W_j y_j - Q_j (Q_j'y_j), dy_j = y_j'z_j.
+// with W_j = diag(w_j), Qc'W_jQc = LL' (Qc: orthonormal basis of C0), Q_j = W_j Qc L^-T, z_j = W_j y_j - Q_j (Q_j'y_j),
+// dy_j = y_j'z_j.
 // g o g is squared in registers from the marker fragment.  A warp owns 8 traits x (c+2) column
 // kinds x 8*MA markers, so all accumulators of one (marker, trait) pair sit in one thread.
 //
@@ -353,11 +354,14 @@ __global__ void __launch_bounds__(32 * ST_WARPS, 1) scan_stream_kernel(const Sca
 // Per-trait columns of the EXACT mode.  One warp per trait slot j < n_tt*64 (slots >= m are
 // zero-filled).  Column kind a of trait j lands at packed column ((j/8)*(C+2) + a)*8 + j%8:
 // a = 0: z_j,  a = 1..C: q_ja,  a = C+1: w_j.
+// Qc is the orthonormal basis of the covariates (CholQR^2 with w = 1, weight_consts_block: C0 = Qc R).  The weighted
+// Gram matrix S = Qc'WQc is then conditioned by the spread of the weights alone: built from C0 itself it would carry
+// kappa(C0)^2 (1e10 for two near-collinear covariates) into the basis q and the LODs.
 // -----------------------------------------------------------------------------------------------
 template <int C>
 __global__ void __launch_bounds__(256) exact_columns_kernel(const double* __restrict__ Yr, const double* __restrict__ h2,
                                                             const double* __restrict__ lambda,
-                                                            const double* __restrict__ C0, int64_t m, int64_t slots,
+                                                            const double* __restrict__ Qc, int64_t m, int64_t slots,
                                                             int n, int n_pad, double* __restrict__ Xop,
                                                             int64_t xcol_pad, double* __restrict__ dyinv, int* flags) {
   constexpr int CG = C + 2;
@@ -388,7 +392,7 @@ __global__ void __launch_bounds__(256) exact_columns_kernel(const double* __rest
     const double wy = w * y[l];
     double cv[C];
 #pragma unroll
-    for (int a = 0; a < C; ++a) cv[a] = C0[(int64_t)a * n_pad + l];
+    for (int a = 0; a < C; ++a) cv[a] = Qc[(int64_t)a * n_pad + l];
     int idx = 0;
 #pragma unroll
     for (int a = 0; a < C; ++a) {
@@ -455,7 +459,7 @@ __global__ void __launch_bounds__(256) exact_columns_kernel(const double* __rest
       for (int a = 0; a < C; ++a) {
         double sv = 0.0;
 #pragma unroll
-        for (int b = 0; b <= a; ++b) sv = fma(Li[a * (a + 1) / 2 + b], C0[(int64_t)b * n_pad + l], sv);
+        for (int b = 0; b <= a; ++b) sv = fma(Li[a * (a + 1) / 2 + b], Qc[(int64_t)b * n_pad + l], sv);
         qa[a] = w * sv;
         z = fma(-qa[a], u[a], z);
       }
@@ -497,12 +501,12 @@ bool stream_unsupported(const ScanParams& P) { return P.et_folded || P.H2idx || 
 
 }  // namespace
 
-int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* C0, int64_t m,
+int launch_exact_columns(const double* Yr, const double* h2, const double* lambda, const double* Qc, int64_t m,
                          int64_t slots, int n, int n_pad, int c, double* Xop, int64_t xcol_pad, double* dyinv,
                          int* flags, cudaStream_t stream) {
   const unsigned blocks = (unsigned)((slots + 7) / 8);
   return dispatch_c<1, MAXC>(c, [&](auto C) {
-    exact_columns_kernel<C><<<blocks, 256, 0, stream>>>(Yr, h2, lambda, C0, m, slots, n, n_pad, Xop, xcol_pad, dyinv,
+    exact_columns_kernel<C><<<blocks, 256, 0, stream>>>(Yr, h2, lambda, Qc, m, slots, n, n_pad, Xop, xcol_pad, dyinv,
                                                         flags);
   });
 }
